@@ -2,7 +2,7 @@
 """bench.py -- k-mers indexed/s and queried/s of the B200 k-mer position index (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3k32|c3|c2]
-                    [--scaling strong|weak]
+                    [--scaling strong|weak] [--dump-outputs DIR]
 
 A step = one pass of the hot path over one synthetic sequence.  The default workload is BASELINE.json's target
 configuration, `c3k32`: ONE 250 Mbp synthetic chromosome with N gaps, k=32, make.kmer.hash + kmer.pos(2|8)
@@ -19,6 +19,8 @@ configuration, `c3k32`: ONE 250 Mbp synthetic chromosome with N gaps, k=32, make
         The sharded index is checked against committed digests of the reference's output (`parity_checked`).
 --impl reference times the reference's own C (oracle/_ref, single-threaded like the reference) on the host cores for
 the same metric on a bounded prefix of the same sequence.
+--dump-outputs DIR (N=1) writes the pos and count matrices of the last timed step to DIR/pos.npy and DIR/count.npy,
+each a fixed, seeded sample of 2^20 rows (see dump_rows), so that two builds can be compared output for output.
 Prints ONE JSON line on rank 0.
 """
 from __future__ import annotations
@@ -238,6 +240,23 @@ def timed(torch, fn, n):
     return a.elapsed_time(b) / n
 
 
+DUMP_ROWS = 1 << 20     # rows sampled from each output: 24 MB of .npy files for pos + count
+
+
+def dump_rows(n: int) -> np.ndarray:
+    """The rows of an n-row output that --dump-outputs keeps: all of them, or DUMP_ROWS distinct ones in ascending order,
+    the same for every run with the same n."""
+    return np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+
+
+def dump_outputs(torch, out_dir: str, outputs: dict) -> None:
+    """Writes `name.npy`: the rows `dump_rows` picks from each device array, as float64 (it holds every int32 exactly)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        rows = torch.from_numpy(dump_rows(a.shape[0])).to(a.device)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a[rows].cpu().numpy().astype(np.float64))
+
+
 def index_leg(kh, torch, seq_dev, k, steps, warm):
     """build + kmer.pos(2|8), everything resident in HBM: (ms per step, N, U)."""
     ix = kh.make_kmer_hash(seq_dev, k)
@@ -362,6 +381,8 @@ def bench_single(args, kh, torch, w, k, L, steps, warm, hbm_peak, peak_src, dev)
     launches = kh.launch_count() - l0
     prof = kh.profile(enable=False)
     kh.profile(reset=True)
+    if args.dump_outputs:
+        dump_outputs(torch, args.dump_outputs, {"pos": pos_dev, "count": cnt_dev})
 
     for _ in range(warm):
         step_e2e()
@@ -407,12 +428,16 @@ def bench_single(args, kh, torch, w, k, L, steps, warm, hbm_peak, peak_src, dev)
     # ---- CPU baseline beside it (rank 0, bounded sample) --------------------------------------------------------
     cpu = None
     if not args.no_cpu:
-        sample = min(L, args.cpu_sample)
-        n_cpu, tb, te, pr = cpu_reference(k, np.ascontiguousarray(np.asarray(seq_pin)[:sample]))
-        cpu = {"value": n_cpu / (tb + te), "unit": "k-mers/s", "cores": 1, "kind": "reference",
-               "sample": f"first {sample} bases of the same sequence; reference seq_to_hash {tb:.2f}s + kmer_positions(2|8) loop {te:.2f}s, "
-                         f"gcc -O2, 1 thread (the reference path is single-threaded); host has {os.cpu_count()} cores",
-               "build_only_value": n_cpu / tb}
+        from oracle import Reference
+        if not Reference.available():
+            print("bench.py: cpu_baseline not measured: the reference engine (oracle/_ref) is not built", file=sys.stderr)
+        else:
+            sample = min(L, args.cpu_sample)
+            n_cpu, tb, te, pr = cpu_reference(k, np.ascontiguousarray(np.asarray(seq_pin)[:sample]))
+            cpu = {"value": n_cpu / (tb + te), "unit": "k-mers/s", "cores": 1, "kind": "reference",
+                   "sample": f"first {sample} bases of the same sequence; reference seq_to_hash {tb:.2f}s + kmer_positions(2|8) loop {te:.2f}s, "
+                             f"gcc -O2, 1 thread (the reference path is single-threaded); host has {os.cpu_count()} cores",
+                   "build_only_value": n_cpu / tb}
 
     # ---- secondary workloads: the other BASELINE configs of this path, value only ---------------------------------
     secondary = {}
@@ -473,7 +498,13 @@ def main():
     ap.add_argument("--no-pageable", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--cpu-sample", type=int, default=60_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="N=1: write the last timed step's outputs to DIR/pos.npy "
+                    "and DIR/count.npy (the same seeded sample of 2^20 rows in every run)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs needs --impl ours --gpus 1")
     if args.impl == "reference":
         run_reference(args)
     else:

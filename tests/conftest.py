@@ -24,7 +24,7 @@ def oracle():
 def reference():
     from oracle import Reference
     if not Reference.available():
-        pytest.skip("oracle/_ref/libkmer_ref.so not built and /root/reference absent")
+        pytest.skip("reference engine oracle/_ref/libkmer_ref.so not built (make -C oracle REF=<kmer_hasheR checkout>)")
     return Reference()
 
 
