@@ -2372,10 +2372,13 @@ __global__ void count_merge_kernel(const uint32_t *__restrict__ mstart, const ui
   }
 }
 // rows (i, count of source s) for s = 0..source_n-1: what kmer.pos(ptr, 2) returns for a count table (the reference's
-// kmer_positions walks v.a[0..v.n), src/kmer_hash.c:1108-1112, and v holds the counters)
-__global__ void count_rows_kernel(const int32_t *__restrict__ counts, uint64_t cells, int source_n, int2 *__restrict__ out) {
-  for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < cells; c += (uint64_t)gridDim.x * blockDim.x)
-    out[c] = make_int2((int)(c / source_n + 1), counts[c]);
+// kmer_positions walks v.a[0..v.n), src/kmer_hash.c:1108-1112, and v holds the counters).  Writes cells
+// [first, first + rows) to out[0, rows): a chunk starts at any cell, not only at a multiple of source_n.
+__global__ void count_rows_kernel(const int32_t *__restrict__ counts, uint64_t first, uint64_t rows, int source_n, int2 *__restrict__ out) {
+  for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < rows; c += (uint64_t)gridDim.x * blockDim.x) {
+    const uint64_t cell = first + c;
+    out[c] = make_int2((int)(cell / source_n + 1), counts[cell]);
+  }
 }
 // spectrum[min(count, max_count)] += 1 over the k-mers (count_spectrum, src/kmer_tree.c:85-99); source < 0: summed over sources
 __global__ void spectrum_counts_kernel(const int32_t *__restrict__ counts, uint64_t U, int source_n, int source, uint32_t max_count,
@@ -2527,8 +2530,7 @@ extern "C" int kmg_count_positions(const kmg_counter *c, int32_t *out) {
   const int sn = c->source_n, sms = g_ctx.sms;
   return stream_rows(cells, 8, out, CHUNK_BYTES / 8, [=](uint64_t first, uint64_t rows, void *dst, uint64_t *, cudaStream_t s) -> int {
     const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(rows, 256), (uint64_t)sms * 16);
-    // chunks start at a multiple of source_n only if rows do; index from the absolute cell
-    LAUNCH("count_rows", s, count_rows_kernel<<<grid, 256, 0, s>>>(counts, first + rows, sn, (int2 *)dst - first));
+    LAUNCH("count_rows", s, count_rows_kernel<<<grid, 256, 0, s>>>(counts, first, rows, sn, (int2 *)dst));
     return KMG_OK;
   });
 }

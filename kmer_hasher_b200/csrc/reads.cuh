@@ -225,8 +225,8 @@ __global__ void pack_kernel(const uint8_t *__restrict__ text, uint64_t n, const 
           if (is_seq && hdr_before[line] == 0) { out->bad = 1; is_seq = false; }
           base = is_seq ? seq_before[line] + hdr_before[line] - 1 : 0;
         }
-      } else if (is_seq && c != '\r') {
-        seq[base + (p - start)] = c;
+      } else if (is_seq && !(c == '\r' && (p + 1 == n || text[p + 1] == '\n'))) {
+        seq[base + (p - start)] = c;                                    // as line_bounds: only a line's final '\r' is dropped
       }
     }
   }

@@ -51,6 +51,9 @@ def _records():
             ("scaf_2", "has\ttabs", random_dna(70_001, 5, p_n=0.002, p_lower=0.3)),
             ("quirk", "", np.concatenate([random_dna(500, 6), np.frombuffer(b"N", np.uint8), random_dna(21, 7)])),   # last run exactly k
             ("tail", "", random_dna(3_333, 8))]
+    # a '\r' inside a sequence line is sequence (only a line's final '\r' is a line end): here never the last byte of a
+    # line at the widths written (60, 80, one line), once the first byte of a 60-wide line
+    recs[-1][2][[100, 120, 241]] = ord("\r")
     return recs
 
 
