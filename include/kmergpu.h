@@ -242,6 +242,24 @@ int kmg_count_spectrum(const kmg_counter *c, int source /* < 0: summed over sour
 int kmg_index_spectrum(const kmg_index *idx, uint32_t max_count, double *spec /* max_count+1 */);
 int kmg_count_free(kmg_counter *c);
 
+/* ---- seq.kmer.depth: per-window k-mer counts along a sequence (additive; the reference has it only for its suffix-hash
+ * counter, seq_kmer_depth_sh) ------------------------------------------------------------------------------------------
+ * For every window start r = 0 .. nwin-1 of q, nwin = max(0, qlen - k + 1) with k = the handle's own k, row r of `out` is
+ * the count of the window's k-mer: source_n int32 per row for a count table (the k-mer's row of the count matrix), one
+ * for a position index (the length of its position list).  Row r is the window at 1-based start r+1 (= i - k + 1 of
+ * seq.kmer.pos).  A k-mer absent from the table gives 0; a window the window rule does not emit (an N/n inside, or the
+ * end-of-string rule; exactly the windows make.kmer.hash skips) gives INT32_MIN = R's NA_integer_ in every column.
+ * KMG_STRAND_BOTH: count(key) + count(rc(key)), rc = the reverse complement in code space (the k 2-bit codes reversed,
+ * each complemented as code ^ 2: A<->T, C<->G); a palindrome (rc(key) == key, even k only) counts once; sums saturate at
+ * INT32_MAX; validity is the forward window's.  For ACGT/acgt bytes rc(key) is the key of the same window in
+ * kmg_query_begin_rc's string; for other non-N bytes it is not (that routine complements bytes IUPAC-style, R -> Y, this
+ * complements the code the byte was given).  `q` and `out` may be host (pageable or pinned) or device memory.  The first
+ * call on a count table builds its key table (cached; kmg_count_add drops it). */
+#define KMG_STRAND_FORWARD 0
+#define KMG_STRAND_BOTH 1
+int kmg_count_depth(const kmg_counter *c, const char *q, int64_t qlen, int strands, int32_t *out /* nwin * source_n */);
+int kmg_index_depth(const kmg_index *idx, const char *q, int64_t qlen, int strands, int32_t *out /* nwin */);
+
 /* ---- FASTA / FASTQ ingestion (SURVEY.md 8f rank 4) ---------------------------------------------------------
  * Replaces, for the index path, what the reference does with klib's kseq.h over zlib (src/kseq.h; read loop
  * src/kmer_reader.c:41-77): the host inflates the file, the DEVICE finds and classifies the lines and packs the records'

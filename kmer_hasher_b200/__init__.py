@@ -21,8 +21,8 @@ from . import _lib
 from ._lib import KmgError, check
 
 __all__ = ["KmerHash", "KmerCounts", "SequenceFile", "make_kmer_hash_file", "count_kmers_file", "make_kmer_hash", "kmer_pos", "seq_kmer_pos", "kmer_pairs", "count_kmers", "kmer_spectrum",
-           "pinned_empty", "KmgError",
-           "OPT_KMER", "OPT_POS", "OPT_PAIRS", "OPT_COUNT"]
+           "seq_kmer_depth", "pinned_empty", "KmgError",
+           "OPT_KMER", "OPT_POS", "OPT_PAIRS", "OPT_COUNT", "NA_INTEGER"]
 
 # opt.flag bits, src/kmer_hash.c:17 (pos_opt_flags) in the reference
 OPT_KMER, OPT_POS, OPT_PAIRS, OPT_COUNT = 1, 2, 4, 8
@@ -30,6 +30,7 @@ ORDER_GROUPED, ORDER_SORTED = 0, 1      # include/kmergpu.h
 KMER_HASH_TAG = "kmer_hash_250930"      # src/kmer_hash.c:22
 MAX_K = 32                              # src/kmer_util.h:12
 INT_MAX = 2**31 - 1
+NA_INTEGER = -2**31                     # R's NA_integer_: seq_kmer_depth's value for a window that is not a k-mer
 
 _L = _lib.load()                        # loud failure when libkmergpu.so is absent
 
@@ -504,6 +505,41 @@ def seq_kmer_pos(ex_ptr, seq, k, *, allow_k32: bool = False, out: np.ndarray | N
         _L.kmg_query_free(st)
     del keep
     return a[:M.value]
+
+
+def seq_kmer_depth(ptr, seq, *, both_strands: bool = False, out=None):
+    """seq.kmer.depth (additive; the R closure is in INTEGRATION.md): for every k-mer window of `seq`, how often its k-mer
+    was counted.  `ptr` is a count table (count_kmers: one column per source) or a position index (make_kmer_hash: one
+    column, the length of the k-mer's position list); k is the handle's own.
+
+    Returns an (nwin, source_n) int32 array, nwin = len(seq) - k + 1, row r = the window at 1-based start r + 1.  An absent
+    k-mer gives 0; a window make.kmer.hash would skip (an N/n in it, or the end-of-string rule) gives NA_INTEGER in every
+    column.  `both_strands=True` adds the count of the reverse complement (code space: A<->T, C<->G; a palindrome counts
+    once; saturating at 2^31 - 1).  `seq` is a str, bytes, uint8 numpy array or uint8 torch tensor (host or device);
+    `out` may supply the result array (numpy, pinned or a torch device tensor) of at least nwin * source_n int32."""
+    ix = _extract(ptr)
+    if isinstance(seq, (list, tuple)):
+        if len(seq) != 1:
+            raise ValueError("seq_r should be a single sequence")
+        seq = seq[0]
+    counts = isinstance(ix, KmerCounts)
+    cols = ix.source_n if counts else 1
+    p, n, keep = _seq_buffer(seq)
+    if n <= ix.k:
+        raise ValueError("the sequence should be longer than k")
+    nwin = n - ix.k + 1
+    if nwin * cols > INT_MAX:
+        raise OverflowError(f"{nwin * cols} values exceed an R matrix extent")
+    if out is None:
+        out = np.empty((nwin, cols), np.int32)
+    else:
+        size = out.nbytes if isinstance(out, np.ndarray) else out.numel() * out.element_size()
+        if size < 4 * nwin * cols:
+            raise ValueError(f"out holds {size} bytes; the depth needs {4 * nwin * cols}")
+    depth = _L.kmg_count_depth if counts else _L.kmg_index_depth
+    check(depth(ix._handle(), p, n, int(bool(both_strands)), _out_ptr(out)))
+    del keep
+    return out
 
 
 def kmer_pairs(ptr_a, ptr_b, *, out: np.ndarray | None = None) -> np.ndarray:

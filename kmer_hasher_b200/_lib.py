@@ -86,6 +86,8 @@ SIGNATURES = {
     "kmg_count_spectrum": (C.c_int, [vp, C.c_int, C.c_uint32, C.POINTER(C.c_double)]),
     "kmg_index_spectrum": (C.c_int, [vp, C.c_uint32, C.POINTER(C.c_double)]),
     "kmg_count_free": (C.c_int, [vp]),
+    "kmg_count_depth": (C.c_int, [vp, vp, C.c_int64, C.c_int, vp]),
+    "kmg_index_depth": (C.c_int, [vp, vp, C.c_int64, C.c_int, vp]),
     "kmg_reads_open": (C.c_int, [C.c_char_p, C.POINTER(vp)]),
     "kmg_reads_from_memory": (C.c_int, [vp, C.c_int64, C.POINTER(vp)]),
     "kmg_reads_count": (C.c_int, [vp, u64p, u64p]),

@@ -1399,7 +1399,7 @@ static int ensure_hash(kmg_index *ix) {
   while (cap < 2 * ix->U) cap <<= 1;                          // load <= 0.5
   TRY(dalloc(&slots, cap, s));
   CU(cudaMemsetAsync(slots, 0, cap * sizeof(uint4), s));
-  LAUNCH("hash_insert", s, hash_insert_kernel<<<grid, 256, 0, s>>>(ix->ukeys, ix->ustart, ix->U, KeyHash{slots, cap / BUCKET_SLOTS, 0}, false));
+  LAUNCH("hash_insert", s, hash_insert_kernel<<<grid, 256, 0, s>>>(ix->ukeys, IndexPayload{ix->ustart}, ix->U, KeyHash{slots, cap / BUCKET_SLOTS, 0}, false));
   CU(cudaStreamSynchronize(s));
   ix->hash = slots; ix->hash_nb = cap / BUCKET_SLOTS; ix->hash_hbits = 0;
   prof_bytes("hash_insert", 12.0 * ix->U + 16.0 * ix->U);
@@ -2347,6 +2347,10 @@ struct kmg_counter {
   uint64_t U = 0, new_total = 0;     // distinct k-mers; sum over calls of the k-mers that were new (khash_ptr.kmer_count)
   uint64_t *keys = nullptr;          // [U] ascending 2-bit keys
   int32_t *counts = nullptr;         // [U][source_n]
+  // made on the first depth call, dropped whenever keys / counts are replaced
+  std::mutex mu;
+  uint4 *hash = nullptr;             // key table (probe.cuh), slots {key, row u, count (source_n == 1) or 1}
+  uint64_t hash_nb = 0;
 };
 
 __global__ void count_first_kernel(const uint32_t *__restrict__ ustart, uint64_t U, int source_n, int source, int32_t *__restrict__ counts) {
@@ -2418,6 +2422,7 @@ extern "C" int kmg_count_free(kmg_counter *c) {
   if (mine) cudaStreamSynchronize(g_ctx.stream()); else cudaDeviceSynchronize();
   g_arena[c->device & 63].put(c->keys, nullptr, true);
   g_arena[c->device & 63].put(c->counts, nullptr, true);
+  g_arena[c->device & 63].put(c->hash, nullptr, true);
   cudaGetLastError();
   if (prev >= 0) cudaSetDevice(prev);
   delete c;
@@ -2439,6 +2444,11 @@ extern "C" int kmg_count_add(kmg_counter *c, const char *seq, int64_t len, int s
   TRY(kmg_build_ordered(seq, len, c->k, KMG_ORDER_SORTED, &b));
   if (b->U == 0) { kmg_free(b); return KMG_OK; }
   cudaStream_t s = g_ctx.stream();
+  {                                                          // the key table describes the arrays about to be replaced
+    std::lock_guard<std::mutex> g(c->mu);
+    dfree(c->hash, s);
+    c->hash_nb = 0;
+  }
   const int sn = c->source_n;
   const unsigned grid_of_b = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(b->U, 256), (uint64_t)g_ctx.sms * 16);
   uint64_t *cat_keys = nullptr;
@@ -2579,6 +2589,96 @@ extern "C" int kmg_index_spectrum(const kmg_index *ix, uint32_t max_count, doubl
   if (rc == KMG_OK) rc = spectrum_out(d, max_count, spec, s);
   dfree(d, s);
   return rc;
+}
+
+// ------------------------------------------------------------------------------------------------
+// seq.kmer.depth: for every window of a query, the count of its k-mer in a count table or a position index
+// ------------------------------------------------------------------------------------------------
+// Key table of a count table: the probe's CAS build (hbits = 0, power-of-two buckets, load <= 0.5).  The keys are in
+// ascending raw-key order, not in an order the streamed build of a grouped index could use.
+static int ensure_count_hash(kmg_counter *c) {
+  std::lock_guard<std::mutex> g(c->mu);
+  if (c->hash || c->U == 0) return KMG_OK;
+  cudaStream_t s = g_ctx.stream();
+  uint64_t cap = 4 * BUCKET_SLOTS;
+  while (cap < 2 * c->U) cap <<= 1;
+  uint4 *slots = nullptr;
+  TRY(dalloc(&slots, cap, s));
+  auto body = [&]() -> int {
+    CU(cudaMemsetAsync(slots, 0, cap * sizeof(uint4), s));
+    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(c->U, 256), (uint64_t)g_ctx.sms * 32);
+    LAUNCH("count_hash_insert", s, hash_insert_kernel<<<grid, 256, 0, s>>>(c->keys, CountPayload{c->counts, c->source_n}, c->U,
+                                                                         KeyHash{slots, cap / BUCKET_SLOTS, 0}, false));
+    CU(cudaStreamSynchronize(s));
+    return KMG_OK;
+  };
+  const int rc = body();
+  if (rc != KMG_OK) { dfree(slots, s); return rc; }
+  c->hash = slots; c->hash_nb = cap / BUCKET_SLOTS;
+  prof_bytes("count_hash_insert", 12.0 * c->U + 16.0 * c->U);
+  return KMG_OK;
+}
+
+constexpr int DEPTH_THREADS = 256, DEPTH_ITEMS = 8, DEPTH_TILE = DEPTH_THREADS * DEPTH_ITEMS;
+
+// Argument checks shared by both entries; *nwin = max(0, qlen - k + 1)
+static int depth_args(const char *q, int64_t qlen, int k, int strands, const int32_t *out, int64_t *nwin) {
+  if (qlen < 0 || (qlen > 0 && !q)) return fail(KMG_ERR_ARG, "bad query pointer/length");
+  if (qlen + 1 > (int64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "query longer than int coordinates");
+  if (strands != KMG_STRAND_FORWARD && strands != KMG_STRAND_BOTH) return fail(KMG_ERR_ARG, "strands must be KMG_STRAND_FORWARD or KMG_STRAND_BOTH");
+  *nwin = qlen - k + 1 > 0 ? qlen - k + 1 : 0;
+  if (*nwin > 0 && !out) return fail(KMG_ERR_ARG, "out is NULL");
+  return KMG_OK;
+}
+
+// kt.nb == 0: empty table.  cols > 1: `cols` columns gathered from the count matrix, else one column from the slot.
+static int depth_run(const char *qseq, int64_t qlen, int64_t nwin, int k, bool both, KeyHash kt, const int32_t *counts, int cols,
+                     int32_t *out) {
+  cudaStream_t s = g_ctx.stream();
+  DevSeq ds;
+  TRY(upload_seq(qseq, qlen, s, &ds));
+  SeqView sv;
+  sv.base = ds.base; sv.nstarts = nwin; sv.avail = qlen; sv.s0 = 0; sv.L = qlen; sv.k = k;
+  const size_t row_bytes = 4 * (size_t)cols;
+  const bool multi = cols > 1;                           // not counts != nullptr: an empty table has no matrix
+  const int rc = stream_rows((uint64_t)nwin, row_bytes, out, CHUNK_BYTES / row_bytes, [=](uint64_t first, uint64_t rows, void *dst, uint64_t *, cudaStream_t st) -> int {
+    const unsigned grid = (unsigned)ceil_div<uint64_t>(first % 16 + rows, DEPTH_TILE);
+    const int64_t f = (int64_t)first, n = (int64_t)rows;
+    int32_t *o = (int32_t *)dst;
+#define KMG_DEPTH(B, M) LAUNCH("depth_lookup", st, (depth_lookup_kernel<DEPTH_THREADS, DEPTH_ITEMS, B, M><<<grid, DEPTH_THREADS, 0, st>>>(sv, f, n, kt, counts, cols, o)))
+    if (both) { if (multi) KMG_DEPTH(true, true); else KMG_DEPTH(true, false); }
+    else { if (multi) KMG_DEPTH(false, true); else KMG_DEPTH(false, false); }
+#undef KMG_DEPTH
+    return KMG_OK;
+  });
+  dfree(ds.buf, s);
+  // one 128-byte line of HBM per table request (tools/micro/gups.cu); with several columns one more per request for the
+  // row gather; counted for every window, so a query whose windows miss or are invalid is charged the same
+  const double lines = (both ? 2.0 : 1.0) * (multi ? 2.0 : 1.0) * (double)nwin;
+  prof_bytes("depth_lookup", (double)qlen + 128.0 * lines + (double)row_bytes * (double)nwin);
+  return rc;
+}
+
+extern "C" int kmg_count_depth(const kmg_counter *cc, const char *q, int64_t qlen, int strands, int32_t *out) {
+  TRY(use_counter(cc));
+  int64_t nwin = 0;
+  TRY(depth_args(q, qlen, cc->k, strands, out, &nwin));
+  if (nwin == 0) return KMG_OK;
+  kmg_counter *c = const_cast<kmg_counter *>(cc);
+  TRY(ensure_count_hash(c));
+  const KeyHash kt{c->hash, c->hash_nb, 0};
+  return depth_run(q, qlen, nwin, c->k, strands == KMG_STRAND_BOTH, kt, c->counts, c->source_n, out);
+}
+
+extern "C" int kmg_index_depth(const kmg_index *cix, const char *q, int64_t qlen, int strands, int32_t *out) {
+  TRY(use_index(cix));
+  int64_t nwin = 0;
+  TRY(depth_args(q, qlen, cix->k, strands, out, &nwin));
+  if (nwin == 0) return KMG_OK;
+  kmg_index *ix = const_cast<kmg_index *>(cix);
+  TRY(ensure_hash(ix));
+  const KeyHash kt{ix->hash, ix->hash ? ix->hash_nb : 0, ix->hash_hbits};
+  return depth_run(q, qlen, nwin, ix->k, strands == KMG_STRAND_BOTH, kt, nullptr, 1, out);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -77,10 +77,24 @@ __device__ __forceinline__ void cas_insert(const KeyHash &kh, uint64_t key, uint
   }
 }
 
-// Distinct keys only: one 128-bit CAS claims a slot and fills it (a stored slot is never all-zero: count >= 1).
+// Slot payloads {z, w} (w != 0: the slot is taken).  Position index: {first position slot, list length}.
+struct IndexPayload {
+  const uint32_t *ustart;
+  __device__ __forceinline__ uint2 operator()(uint64_t u) const { const uint32_t s = ustart[u]; return make_uint2(s, ustart[u + 1] - s); }
+};
+// Count table (U x source_n matrix): {row u, count} with one column (a k-mer in the table was counted, so count >= 1),
+// {row u, 1} with several (the lookup then gathers the row).
+struct CountPayload {
+  const int32_t *counts;
+  int source_n;
+  __device__ __forceinline__ uint2 operator()(uint64_t u) const { return make_uint2((uint32_t)u, source_n == 1 ? (uint32_t)counts[u] : 1u); }
+};
+
+// Distinct keys only: one 128-bit CAS claims a slot and fills it (a stored slot is never all-zero: w >= 1).
 // overflow_only (tables written by hash_stream_kernel): insert only a bucket's third and later k-mers, found by the same
 // test as there (the two k-mers before it share its home bucket).
-__global__ void hash_insert_kernel(const uint64_t *__restrict__ ukeys, const uint32_t *__restrict__ ustart, uint64_t U, KeyHash kh,
+template <class Payload>
+__global__ void hash_insert_kernel(const uint64_t *__restrict__ ukeys, const Payload pay, uint64_t U, KeyHash kh,
                                    const bool overflow_only) {
   for (uint64_t u = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; u < U; u += (uint64_t)gridDim.x * blockDim.x) {
     const uint64_t key = ukeys[u];
@@ -89,8 +103,8 @@ __global__ void hash_insert_kernel(const uint64_t *__restrict__ ukeys, const uin
       if (u < 2) continue;
       if (kh.bucket(ukeys[u - 1]) != b || kh.bucket(ukeys[u - 2]) != b) continue;
     }
-    const uint32_t start = ustart[u];
-    cas_insert(kh, key, start, ustart[u + 1] - start, b, overflow_only);
+    const uint2 p = pay(u);
+    cas_insert(kh, key, p.x, p.y, b, overflow_only);
   }
 }
 
@@ -246,6 +260,90 @@ probe_lookup_kernel(const SeqView sv, const uint64_t *__restrict__ keys_in, int6
 #pragma unroll
       for (int j = 0; j < BATCH; ++j)
         if (q0 + t0 + i0 + j < total) found[q0 + t0 + i0 + j] = r[j];
+    }
+  }
+}
+
+// ---- seq.kmer.depth: per-window counts of the query's k-mers ------------------------------------------------
+// Reverse complement of a k-mer key in code space: the k 2-bit codes reversed and each complemented as code ^ 2
+// (A0 <-> T2, C1 <-> G3).  Complement all codes, reverse the 64 bits (which also swaps the two bits of every code), swap
+// them back, drop the 64 - 2k bits that were above the key.
+__device__ __forceinline__ uint64_t revcomp_key(uint64_t key, int k) {
+  uint64_t x = __brevll(key ^ 0xAAAAAAAAAAAAAAAAull);
+  x = ((x >> 1) & 0x5555555555555555ull) | ((x & 0x5555555555555555ull) << 1);
+  return x >> (64 - 2 * k);
+}
+
+// Windows [first, first + rows) of the query into out[0, rows * cols): row r = window first + r, cols = source_n with
+// MULTI (the k-mer's row of the count matrix, gathered through the slot's row number) else 1 (the slot's count field:
+// a position list's length or a one-column count).  A window the window rule drops gets INT32_MIN (R's NA_integer_) in
+// every column, an absent k-mer 0.  BOTH: count(key) + count(revcomp(key)), a palindrome once, saturated at INT32_MAX.
+// A chunk may start at any window; tile_pack needs 16-aligned tile starts, so tiles start at `first` rounded down to
+// 16 and windows in front of the chunk are encoded (the keys roll through them) but neither looked up nor written.
+// The lookup is probe_lookup_kernel's: BATCH sectors in flight per thread (twice as many with BOTH), then resolve.
+// nb == 0: an empty table, nothing is looked up.  Blocks per SM: the most whose register share holds the variant
+// without spills (ptxas: 62 registers forward / one column, ~70 forward / gathered, ~120 both strands).
+template <int THREADS, int ITEMS, bool BOTH, bool MULTI>
+__global__ void __launch_bounds__(THREADS, BOTH ? 2 : (MULTI ? 3 : 4))
+depth_lookup_kernel(const SeqView sv, int64_t first, int64_t rows, const KeyHash kh, const int32_t *__restrict__ counts,
+                    const int source_n, int32_t *__restrict__ out) {
+  constexpr int TILE = THREADS * ITEMS, BATCH = 4;
+  static_assert(ITEMS % BATCH == 0, "items in batches");
+  __shared__ TileCodes<TILE> tc;
+  const int64_t q0 = (first & ~int64_t(15)) + (int64_t)blockIdx.x * TILE, end = first + rows;
+  if (q0 >= end) return;
+  const int t0 = threadIdx.x * ITEMS;
+  const bool special = tile_pack<TILE, THREADS>(sv, q0, tc);
+  const bool have = kh.nb != 0;
+  const int cols = MULTI ? source_n : 1;
+  const uint64_t kmask = key_mask(sv.k);
+  uint64_t key = 0;
+#pragma unroll
+  for (int i0 = 0; i0 < ITEMS; i0 += BATCH) {
+    uint4 s0[BATCH], s1[BATCH], c0[BATCH], c1[BATCH];
+    uint64_t kk[BATCH], home[BATCH], rk[BATCH], rhome[BATCH];
+    bool ok[BATCH], in[BATCH], pal[BATCH];
+#pragma unroll
+    for (int j = 0; j < BATCH; ++j) {
+      const int i = i0 + j;
+      if (i == 0) key = tile_key<TILE>(tc, t0, sv.k);
+      else {                                              // roll in the base at tile position t0 + i + k - 1
+        const int p = t0 + i + sv.k - 1;
+        key = ((key << 2) | ((tc.codes[p >> 4] >> (30 - 2 * (p & 15))) & 3u)) & kmask;
+      }
+      const int64_t q = q0 + t0 + i;
+      in[j] = q >= first && q < end;
+      ok[j] = in[j] && tile_valid<TILE>(sv, tc, q0, t0 + i, special);
+      kk[j] = key;
+      home[j] = kh.bucket(key);
+      if (ok[j] && have) ld_stream_sector(kh.slots + home[j] * BUCKET_SLOTS, s0[j], s1[j]);
+      if constexpr (BOTH) {
+        rk[j] = revcomp_key(key, sv.k);
+        pal[j] = rk[j] == key;
+        rhome[j] = kh.bucket(rk[j]);
+        if (ok[j] && have && !pal[j]) ld_stream_sector(kh.slots + rhome[j] * BUCKET_SLOTS, c0[j], c1[j]);
+      }
+    }
+    uint2 f[BATCH], r[BATCH];
+#pragma unroll
+    for (int j = 0; j < BATCH; ++j) {
+      f[j] = ok[j] && have ? resolve_key(kh, kk[j], home[j], s0[j], s1[j]) : make_uint2(0u, 0u);
+      r[j] = make_uint2(0u, 0u);
+      if constexpr (BOTH) if (ok[j] && have && !pal[j]) r[j] = resolve_key(kh, rk[j], rhome[j], c0[j], c1[j]);
+    }
+    int32_t *dst = out + (q0 + t0 + i0 - first) * cols;   // row of window j: dst + j * cols (only rows of the chunk are touched)
+    for (int s = 0; s < cols; ++s) {
+      int32_t v[BATCH];
+#pragma unroll
+      for (int j = 0; j < BATCH; ++j) {
+        uint64_t c = (uint64_t)f[j].y + r[j].y;
+        if constexpr (MULTI) c = (f[j].y ? (uint32_t)__ldg(counts + (uint64_t)f[j].x * cols + s) : 0u) +
+                                 (uint64_t)(r[j].y ? (uint32_t)__ldg(counts + (uint64_t)r[j].x * cols + s) : 0u);
+        v[j] = ok[j] ? (int32_t)(c < (uint64_t)INT32_MAX ? c : (uint64_t)INT32_MAX) : INT32_MIN;
+      }
+#pragma unroll
+      for (int j = 0; j < BATCH; ++j)
+        if (in[j]) dst[j * cols + s] = v[j];
     }
   }
 }

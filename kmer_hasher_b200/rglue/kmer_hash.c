@@ -11,6 +11,7 @@
  *   sequence_kmer_positions(ptr, seq, k)    replaces src/kmer_hash.c:1151-1172
  *   kmer_pair_pos(ptr.a, ptr.b)             replaces src/kmer_hash.c:1174-1203 (which crashes: test.R:330-331)
  *   count_kmers(ptr, params, seq)           replaces src/kmer_hash.c:548-591 (count.kmers: per-source counts)
+ *   sequence_kmer_depth(ptr, seq, strands)  additive: per-window counts of a sequence's k-mers (seq.kmer.depth)
  *   R_init_kmer_hash                        replaces src/kmer_hash.c:1221-1224
  *
  * Differences a user can observe: k-mers come out in the order of a mix of their 2-bit key (ascending key
@@ -406,6 +407,33 @@ SEXP count_kmers_file(SEXP hash_ptr_r, SEXP params_r, SEXP file_r) {
   return ptr_r;
 }
 
+/* seq.kmer.depth(ptr, seq, both.strands) -> t(.Call("sequence_kmer_depth", ptr, as.character(seq), as.integer(both.strands)))
+ * (additive; INTEGRATION.md): for every k-mer window of seq, the count of its k-mer in a count table (source_n rows, one
+ * per source) or a position index (one row: the length of the position list).  Returns a source_n x nwin matrix, nwin =
+ * length(seq) - k + 1 with the handle's k; NA for a window make.kmer.hash would skip (the library writes INT32_MIN, which
+ * is NA_integer_). */
+SEXP sequence_kmer_depth(SEXP ptr_r, SEXP seq_r, SEXP strands_r) {
+  if (TYPEOF(seq_r) != STRSXP || length(seq_r) != 1) error("seq_r should be a single sequence");
+  if (TYPEOF(strands_r) != INTSXP || length(strands_r) != 1 || (INTEGER(strands_r)[0] != 0 && INTEGER(strands_r)[0] != 1))
+    error("both.strands should be TRUE or FALSE");
+  kmer_handle *h = handle_or_error(ptr_r);
+  const int strands = INTEGER(strands_r)[0] ? KMG_STRAND_BOTH : KMG_STRAND_FORWARD;
+  int sn = 1;
+  if (h->counter && kmg_count_sizes(h->counter, NULL, &sn, NULL, NULL) != KMG_OK) error("seq.kmer.depth failed: %s", kmg_last_error());
+  SEXP s = STRING_ELT(seq_r, 0);
+  const int len = length(s);
+  if (len <= h->k) error("the sequence should be longer than k");
+  const uint64_t nwin = (uint64_t)(len - h->k + 1);
+  if (nwin * (uint64_t)sn > (uint64_t)INT_MAX)
+    error("seq.kmer.depth would return %llu values, more than an R matrix can hold (2^31-1)", (unsigned long long)(nwin * (uint64_t)sn));
+  SEXP m = PROTECT(allocMatrix(INTSXP, sn, (int)nwin));
+  const int rc = h->counter ? kmg_count_depth(h->counter, CHAR(s), (int64_t)len, strands, INTEGER(m))
+                            : kmg_index_depth(h->index, CHAR(s), (int64_t)len, strands, INTEGER(m));
+  UNPROTECT(1);
+  if (rc != KMG_OK) error("seq.kmer.depth failed: %s", kmg_last_error());
+  return m;
+}
+
 static const R_CallMethodDef call_methods[] = {
     {"make_kmer_h_index", (DL_FUNC)&make_kmer_h_index, 3},
     {"kmer_positions", (DL_FUNC)&kmer_positions, 2},
@@ -414,6 +442,7 @@ static const R_CallMethodDef call_methods[] = {
     {"count_kmers", (DL_FUNC)&count_kmers, 3},
     {"make_kmer_h_index_file", (DL_FUNC)&make_kmer_h_index_file, 4},
     {"count_kmers_file", (DL_FUNC)&count_kmers_file, 3},
+    {"sequence_kmer_depth", (DL_FUNC)&sequence_kmer_depth, 3},
     {NULL, NULL, 0}};
 
 void R_init_kmer_hash(DllInfo *info) { R_registerRoutines(info, NULL, call_methods, NULL, NULL); }
