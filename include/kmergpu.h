@@ -141,6 +141,25 @@ int kmg_join_emit(kmg_join *st, int32_t *out /* 2M */);
 int kmg_join_emit_chunk(kmg_join *st, uint64_t first, uint64_t n, int32_t *out /* 2n */);
 int kmg_join_free(kmg_join *st);
 
+/* ---- dot plots: seq.kmer.pos / kmer.pairs rows counted into an image on the device (additive) -----------------------
+ * What a dot plot draws is the 2-D histogram of those rows, which needs nx*ny counts instead of M rows: no 2^31-1 row
+ * limit and no transfer of the rows.  kmg_query_dotplot bins the rows kmg_query_begin (rc = 0) or kmg_query_begin_rc
+ * (rc = 1) + kmg_query_emit give for (idx, q, qlen, k), x = i (1-based END of the query window; with rc = 1 a coordinate
+ * of the reverse-complemented string), y = j (1-based start in the index).  kmg_join_dotplot bins the rows of
+ * kmg_join_begin + kmg_join_emit, x = position in a, y = position in b (same device).
+ * max_count: 0 = no limit; else a k-mer with more than max_count positions in the index (in a join: in either index)
+ * adds no rows -- how dot plots suppress repeats.
+ * Windows are half-open, 0 <= x0 < x1 <= 2^31 (y alike): a row counts iff x0 <= x < x1 and y0 <= y < y1, into bin
+ * bx = floor((x - x0) * nx / (x1 - x0)), by likewise (exact integer arithmetic).  out: nx*ny doubles, column-major,
+ * out[bx + by*nx] (an R matrix with nx rows); every cell is written (exact below 2^53), nothing else is touched; device,
+ * pinned or pageable memory.  An empty index, query or intersection gives an all-zero image.
+ * KMG_ERR_ARG: NULL handle or out, nx or ny < 1, an empty or out-of-range window, rc not 0/1; KMG_ERR_RANGE: nx*ny >
+ * INT32_MAX, or the query length check of kmg_query_begin; KMG_ERR_K as there. */
+int kmg_query_dotplot(const kmg_index *idx, const char *q, int64_t qlen, int k, int rc, int64_t x0, int64_t x1, int nx,
+                      int64_t y0, int64_t y1, int ny, uint32_t max_count, double *out /* nx*ny */);
+int kmg_join_dotplot(const kmg_index *a, const kmg_index *b, int64_t x0, int64_t x1, int nx, int64_t y0, int64_t y1, int ny,
+                     uint32_t max_count, double *out /* nx*ny */);
+
 /* ---- sharded build (one process per GPU; the exchange itself is the host's NCCL all-to-all) ----
  * A rank holds bytes [g0,g1) of a global sequence of length L in device memory at d_seq (d_seq[0]
  * is byte g0) and owns the window starts [s0,s1), g0 <= max(s0-1,0), g1 >= min(L, s1+k-1).

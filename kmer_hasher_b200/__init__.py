@@ -21,7 +21,7 @@ from . import _lib
 from ._lib import KmgError, check
 
 __all__ = ["KmerHash", "KmerCounts", "SequenceFile", "make_kmer_hash_file", "count_kmers_file", "make_kmer_hash", "kmer_pos", "seq_kmer_pos", "kmer_pairs", "count_kmers", "kmer_spectrum",
-           "seq_kmer_depth", "pinned_empty", "KmgError",
+           "seq_kmer_depth", "seq_kmer_dotplot", "kmer_pairs_dotplot", "pinned_empty", "KmgError",
            "OPT_KMER", "OPT_POS", "OPT_PAIRS", "OPT_COUNT", "NA_INTEGER"]
 
 # opt.flag bits, src/kmer_hash.c:17 (pos_opt_flags) in the reference
@@ -561,6 +561,68 @@ def kmer_pairs(ptr_a, ptr_b, *, out: np.ndarray | None = None) -> np.ndarray:
     finally:
         _L.kmg_join_free(st)
     return r[:M.value]
+
+
+def _dotplot_args(bins, ranges, max_count, out):
+    """(nx, ny, (x0, x1), (y0, y1), max_count, out) checked; `out` allocated column-major when None."""
+    nx, ny = (int(b) for b in bins)
+    if nx < 1 or ny < 1:
+        raise ValueError("bins must be positive")
+    if nx * ny > INT_MAX:
+        raise OverflowError(f"a dot plot of {nx} x {ny} bins has more than 2^31 - 1 cells")
+    win = []
+    for name, r in zip(("x", "y"), ranges):
+        lo, hi = (int(v) for v in r)
+        if not 0 <= lo < hi <= 2**31:
+            raise ValueError(f"{name} range [{lo}, {hi}) must satisfy 0 <= start < end <= 2^31")
+        win.append((lo, hi))
+    max_count = int(max_count)
+    if not 0 <= max_count < 2**32:
+        raise ValueError("max_count must be 0 (no limit) or a positive 32-bit count")
+    if out is None:
+        out = np.empty((nx, ny), np.float64, order="F")
+    else:
+        size = out.nbytes if isinstance(out, np.ndarray) else out.numel() * out.element_size()
+        if size < 8 * nx * ny:
+            raise ValueError(f"out holds {size} bytes; the image needs {8 * nx * ny}")
+    return nx, ny, win[0], win[1], max_count, out
+
+
+def seq_kmer_dotplot(ptr, seq, k, *, y_range, bins=(1000, 1000), x_range=None, reverse_complement=False, max_count=0,
+                     allow_k32=False, out=None):
+    """seq.kmer.dotplot (additive; the R closure is in INTEGRATION.md): the rows seq_kmer_pos(ptr, seq, k,
+    reverse_complement=...) would return, counted on the device into an nx x ny image -- x = i (1-based END of the query
+    window, of the reverse-complemented string with reverse_complement=True), y = j (1-based start in the index).
+
+    x_range = (x0, x1) and y_range = (y0, y1) are half-open windows (0 <= start < end <= 2^31; x_range defaults to
+    (1, len(seq) + 1), the index's length is not recorded so y_range is required); a row counts into bin
+    (floor((x - x0) * nx / (x1 - x0)), floor((y - y0) * ny / (y1 - y0))) if it lies in both windows.  max_count > 0 drops
+    the k-mers with more positions in the index.  Returns a float64 (nx, ny) array in column-major order (the bytes of the
+    R matrix); `out` may supply it (numpy, pinned or a torch device tensor of at least nx * ny float64)."""
+    ix = _extract_index(ptr)
+    if isinstance(seq, (list, tuple)):
+        if len(seq) != 1:
+            raise ValueError("seq_r should be a single sequence")
+        seq = seq[0]
+    k = int(k)
+    p, n, keep = _seq_buffer(seq)
+    if n <= k or k > (32 if allow_k32 else 31):
+        raise ValueError("the sequence should be longer than k and k should not be longer than 31")
+    nx, ny, (x0, x1), (y0, y1), mc, out = _dotplot_args(bins, (x_range if x_range is not None else (1, n + 1), y_range),
+                                                        max_count, out)
+    check(_L.kmg_query_dotplot(ix._handle(), p, n, k, int(bool(reverse_complement)), x0, x1, nx, y0, y1, ny, mc, _out_ptr(out)))
+    del keep
+    return out
+
+
+def kmer_pairs_dotplot(ptr_a, ptr_b, *, a_range, b_range, bins=(1000, 1000), max_count=0, out=None):
+    """kmer.pairs.dotplot (additive; INTEGRATION.md): the rows kmer_pairs(ptr_a, ptr_b) would return, counted on the device
+    into an nx x ny image, x = position in ptr_a over the half-open a_range, y = position in ptr_b over b_range; binning,
+    max_count (here: more positions in either index), result and `out` as in seq_kmer_dotplot."""
+    a, b = _extract_index(ptr_a), _extract_index(ptr_b)
+    nx, ny, (x0, x1), (y0, y1), mc, out = _dotplot_args(bins, (a_range, b_range), max_count, out)
+    check(_L.kmg_join_dotplot(a._handle(), b._handle(), x0, x1, nx, y0, y1, ny, mc, _out_ptr(out)))
+    return out
 
 
 def profile(enable: bool | None = None, reset: bool = False) -> dict:

@@ -45,6 +45,9 @@ SIGNATURES = {
     "kmg_join_emit": (C.c_int, [vp, vp]),
     "kmg_join_emit_chunk": (C.c_int, [vp, C.c_uint64, C.c_uint64, vp]),
     "kmg_join_free": (C.c_int, [vp]),
+    "kmg_query_dotplot": (C.c_int, [vp, vp, C.c_int64, C.c_int, C.c_int, C.c_int64, C.c_int64, C.c_int,
+                                    C.c_int64, C.c_int64, C.c_int, C.c_uint32, vp]),
+    "kmg_join_dotplot": (C.c_int, [vp, vp, C.c_int64, C.c_int64, C.c_int, C.c_int64, C.c_int64, C.c_int, C.c_uint32, vp]),
     "kmg_shard_sample": (C.c_int, [vp, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int, vp]),
     "kmg_shard_partition": (C.c_int, [vp, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int,
                                       u64p, C.c_int, vp, vp, u64p]),

@@ -1407,7 +1407,8 @@ static int ensure_hash(kmg_index *ix) {
 }
 
 static int query_common(const kmg_index *cix, bool from_seq, const SeqView &sv, const uint64_t *d_keys,
-                        const int32_t *d_i, int64_t n, kmg_query **out, uint64_t *M, const uint64_t *d_n = nullptr, bool mixed = false) {
+                        const int32_t *d_i, int64_t n, kmg_query **out, uint64_t *M, const uint64_t *d_n = nullptr, bool mixed = false,
+                        uint32_t max_count = UINT32_MAX) {
   kmg_index *ix = const_cast<kmg_index *>(cix);
   cudaStream_t s = g_ctx.stream();
   kmg_query *q = new (std::nothrow) kmg_query();
@@ -1438,11 +1439,11 @@ static int query_common(const kmg_index *cix, bool from_seq, const SeqView &sv, 
     if (from_seq) {
       LAUNCH("probe_lookup", s, probe_lookup_kernel<PROBE_THREADS, PROBE_ITEMS, true><<<ltiles, PROBE_THREADS, 0, s>>>(sv, nullptr, 0, nullptr, kt, found));
       LAUNCH("probe_compact", s, probe_compact_kernel<PROBE_THREADS, COMPACT_ITEMS, true><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
-                                     found, sv.s0 + sv.k, nullptr, total, nullptr, q->hit_i, q->hit_start, q->row_off, qs, status, ticket));
+                                     found, sv.s0 + sv.k, nullptr, total, nullptr, q->hit_i, q->hit_start, q->row_off, qs, status, ticket, max_count));
     } else {
       LAUNCH("probe_lookup_rec", s, probe_lookup_kernel<PROBE_THREADS, PROBE_ITEMS, false><<<ltiles, PROBE_THREADS, 0, s>>>(sv, d_keys, n, d_n, kt, found, mixed));
       LAUNCH("probe_compact", s, probe_compact_kernel<PROBE_THREADS, COMPACT_ITEMS, false><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
-                                     found, 0, d_i, n, d_n, q->hit_i, q->hit_start, q->row_off, qs, status, ticket));
+                                     found, 0, d_i, n, d_n, q->hit_i, q->hit_start, q->row_off, qs, status, ticket, max_count));
     }
     QueryStats h;
     CU(cudaMemcpyAsync(&h, qs, sizeof h, cudaMemcpyDeviceToHost, s));
@@ -1461,7 +1462,8 @@ static int query_common(const kmg_index *cix, bool from_seq, const SeqView &sv, 
   return KMG_OK;
 }
 
-extern "C" int kmg_query_begin(const kmg_index *ix, const char *qseq, int64_t qlen, int k, kmg_query **st, uint64_t *M) {
+// seq.kmer.pos of q (rc: of reverseComplement(q), taken on the device); k-mers with more than max_count positions give no rows
+static int query_seq(const kmg_index *ix, const char *qseq, int64_t qlen, int k, bool rc, uint32_t max_count, kmg_query **st, uint64_t *M) {
   if (!st) return fail(KMG_ERR_ARG, "st is NULL");
   *st = nullptr;
   if (k < 1 || k > KMG_MAX_K) return fail(KMG_ERR_K, "k must be in [1,32]");
@@ -1469,44 +1471,39 @@ extern "C" int kmg_query_begin(const kmg_index *ix, const char *qseq, int64_t ql
   if (qlen + 1 > (int64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "query longer than int coordinates");
   TRY(use_index(ix));
   cudaStream_t s = g_ctx.stream();
-  DevSeq ds;
-  TRY(upload_seq(qseq, qlen, s, &ds));
-  SeqView sv;
-  sv.base = ds.base; sv.nstarts = qlen - k + 1 > 0 ? qlen - k + 1 : 0; sv.avail = qlen; sv.s0 = 0; sv.L = qlen; sv.k = k;
-  int rc = query_common(ix, true, sv, nullptr, nullptr, 0, st, M);
-  dfree(ds.buf, s);
-  return rc;
+  DevSeq fwd, rev;
+  auto body = [&]() -> int {
+    TRY(upload_seq(qseq, qlen, s, &fwd));
+    const uint8_t *base = fwd.base;
+    if (rc) {
+      const size_t cap = 16 + (size_t)((qlen + 15) / 16) * 16 + 16;
+      TRY(dalloc(&rev.buf, cap, s));
+      rev.base = rev.buf + 16; rev.len = qlen;
+      CU(cudaMemsetAsync(rev.buf, 0, 16, s));
+      CU(cudaMemsetAsync(rev.buf + cap - 32, 0, 32, s));
+      if (qlen > 0) {
+        const unsigned grid = (unsigned)std::min<int64_t>(ceil_div<int64_t>(qlen, 256), (int64_t)g_ctx.sms * 16);
+        LAUNCH("revcomp", s, revcomp_kernel<<<grid, 256, 0, s>>>(fwd.base, qlen, rev.base));
+        prof_bytes("revcomp", 2.0 * qlen);
+      }
+      base = rev.base;
+    }
+    SeqView sv;
+    sv.base = base; sv.nstarts = qlen - k + 1 > 0 ? qlen - k + 1 : 0; sv.avail = qlen; sv.s0 = 0; sv.L = qlen; sv.k = k;
+    return query_common(ix, true, sv, nullptr, nullptr, 0, st, M, nullptr, false, max_count);
+  };
+  const int rv = body();
+  dfree(fwd.buf, s); dfree(rev.buf, s);              // on every path
+  return rv;
+}
+
+extern "C" int kmg_query_begin(const kmg_index *ix, const char *qseq, int64_t qlen, int k, kmg_query **st, uint64_t *M) {
+  return query_seq(ix, qseq, qlen, k, false, UINT32_MAX, st, M);
 }
 
 // seq.kmer.pos(idx, reverseComplement(q), k) with the reverse complement taken on the device
 extern "C" int kmg_query_begin_rc(const kmg_index *ix, const char *qseq, int64_t qlen, int k, kmg_query **st, uint64_t *M) {
-  if (!st) return fail(KMG_ERR_ARG, "st is NULL");
-  *st = nullptr;
-  if (k < 1 || k > KMG_MAX_K) return fail(KMG_ERR_K, "k must be in [1,32]");
-  if (qlen < 0 || (qlen > 0 && !qseq)) return fail(KMG_ERR_ARG, "bad query pointer/length");
-  if (qlen + 1 > (int64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "query longer than int coordinates");
-  TRY(use_index(ix));
-  cudaStream_t s = g_ctx.stream();
-  DevSeq fwd, rc;
-  auto body = [&]() -> int {
-    TRY(upload_seq(qseq, qlen, s, &fwd));
-    const size_t cap = 16 + (size_t)((qlen + 15) / 16) * 16 + 16;
-    TRY(dalloc(&rc.buf, cap, s));
-    rc.base = rc.buf + 16; rc.len = qlen;
-    CU(cudaMemsetAsync(rc.buf, 0, 16, s));
-    CU(cudaMemsetAsync(rc.buf + cap - 32, 0, 32, s));
-    if (qlen > 0) {
-      const unsigned grid = (unsigned)std::min<int64_t>(ceil_div<int64_t>(qlen, 256), (int64_t)g_ctx.sms * 16);
-      LAUNCH("revcomp", s, revcomp_kernel<<<grid, 256, 0, s>>>(fwd.base, qlen, rc.base));
-      prof_bytes("revcomp", 2.0 * qlen);
-    }
-    SeqView sv;
-    sv.base = rc.base; sv.nstarts = qlen - k + 1 > 0 ? qlen - k + 1 : 0; sv.avail = qlen; sv.s0 = 0; sv.L = qlen; sv.k = k;
-    return query_common(ix, true, sv, nullptr, nullptr, 0, st, M);
-  };
-  const int rv = body();
-  dfree(fwd.buf, s); dfree(rc.buf, s);               // on every path
-  return rv;
+  return query_seq(ix, qseq, qlen, k, true, UINT32_MAX, st, M);
 }
 
 extern "C" int kmg_query_records(const kmg_index *ix, const uint64_t *d_keys, const int32_t *d_i, int64_t n, kmg_query **st, uint64_t *M) {
@@ -1584,7 +1581,7 @@ extern "C" int kmg_join_free(kmg_join *j) {
   return KMG_OK;
 }
 
-extern "C" int kmg_join_begin(const kmg_index *a, const kmg_index *cb, kmg_join **out, uint64_t *M) {
+static int join_begin(const kmg_index *a, const kmg_index *cb, uint32_t max_count, kmg_join **out, uint64_t *M) {
   if (!out) return fail(KMG_ERR_ARG, "st is NULL");
   *out = nullptr;
   if (!a || !cb) return fail(KMG_ERR_ARG, "index is NULL");
@@ -1621,7 +1618,7 @@ extern "C" int kmg_join_begin(const kmg_index *a, const kmg_index *cb, kmg_join 
     LAUNCH("probe_lookup_rec", s, probe_lookup_kernel<PROBE_THREADS, PROBE_ITEMS, false><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
                                       sv, a->ukeys, (int64_t)U, nullptr, kt, found));
     LAUNCH("join_compact", s, join_compact_kernel<PROBE_THREADS, PROBE_ITEMS><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
-                                  found, a->ustart, U, j->hit_astart, j->hit_bstart, j->hit_cb, j->row_off, qs, status, ticket));
+                                  found, a->ustart, U, j->hit_astart, j->hit_bstart, j->hit_cb, j->row_off, qs, status, ticket, max_count));
     QueryStats h;
     CU(cudaMemcpyAsync(&h, qs, sizeof h, cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
@@ -1636,6 +1633,10 @@ extern "C" int kmg_join_begin(const kmg_index *a, const kmg_index *cb, kmg_join 
   *out = j;
   if (M) *M = j->M;
   return KMG_OK;
+}
+
+extern "C" int kmg_join_begin(const kmg_index *a, const kmg_index *b, kmg_join **out, uint64_t *M) {
+  return join_begin(a, b, UINT32_MAX, out, M);
 }
 
 extern "C" int kmg_join_emit_chunk(kmg_join *j, uint64_t first, uint64_t n, int32_t *out) {
@@ -1659,6 +1660,89 @@ extern "C" int kmg_join_emit_chunk(kmg_join *j, uint64_t first, uint64_t n, int3
 extern "C" int kmg_join_emit(kmg_join *j, int32_t *out) {
   if (!j) return fail(KMG_ERR_ARG, "join is NULL");
   return kmg_join_emit_chunk(j, 0, j->M, out);
+}
+
+// ------------------------------------------------------------------------------------------------
+// dot plots: the 2-D histogram of a probe's or a join's rows, counted on the device
+// ------------------------------------------------------------------------------------------------
+// Rows are walked in slices of DOT_SLICE_ROWS, so the block-start scratch stays 4 MB however many rows there are.
+constexpr uint64_t DOT_SLICE_ROWS = uint64_t(1) << 30;
+
+static DotAxis dot_axis(int64_t lo, int64_t hi, int n) {
+  const uint64_t range = (uint64_t)(hi - lo);
+  return DotAxis{(uint64_t)lo, range, ~uint64_t(0) / range, (uint32_t)n};
+}
+
+static int dotplot_args(int64_t x0, int64_t x1, int nx, int64_t y0, int64_t y1, int ny, const double *out) {
+  if (!out) return fail(KMG_ERR_ARG, "out is NULL");
+  if (nx < 1 || ny < 1) return fail(KMG_ERR_ARG, "bin counts must be at least 1 (nx = %d, ny = %d)", nx, ny);
+  const int64_t top = int64_t(1) << 31;
+  if (x0 < 0 || x1 <= x0 || x1 > top) return fail(KMG_ERR_ARG, "x window [%lld, %lld) is not inside [0, 2^31]", (long long)x0, (long long)x1);
+  if (y0 < 0 || y1 <= y0 || y1 > top) return fail(KMG_ERR_ARG, "y window [%lld, %lld) is not inside [0, 2^31]", (long long)y0, (long long)y1);
+  if ((int64_t)nx * ny > (int64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "an image of %d x %d bins exceeds 2^31 - 1 cells", nx, ny);
+  return KMG_OK;
+}
+
+// The rows [0, M) of `rows` (hits' row offsets row_off[0, H)) binned into an nx x ny image, written to out as doubles.
+template <class Rows>
+static int dotplot_run(const Rows &rows, const uint64_t *row_off, uint64_t H, uint64_t M, double row_bytes, DotAxis ax, DotAxis ay,
+                       double *out) {
+  cudaStream_t s = g_ctx.stream();
+  const uint64_t cells = (uint64_t)ax.n * ay.n;
+  unsigned long long *img = nullptr;
+  uint64_t *blk = nullptr;
+  TRY(dalloc(&img, cells, s));
+  auto body = [&]() -> int {
+    CU(cudaMemsetAsync(img, 0, cells * sizeof(unsigned long long), s));
+    if (M) TRY(dalloc(&blk, (size_t)ceil_div<uint64_t>(std::min(M, DOT_SLICE_ROWS), EMIT_TILE), s));
+    for (uint64_t first = 0; first < M; first += DOT_SLICE_ROWS) {
+      const uint64_t n = std::min(DOT_SLICE_ROWS, M - first);
+      TRY(block_starts(row_off, H, first, n, s, blk));
+      LAUNCH("dotplot_bin", s, dotplot_bin_kernel<EMIT_THREADS, Rows><<<(unsigned)ceil_div<uint64_t>(n, EMIT_TILE), EMIT_THREADS, 0, s>>>(
+                                   rows, row_off, H, first, n, blk, ax, ay, img));
+    }
+    const int sms = g_ctx.sms;
+    const unsigned long long *im = img;
+    return stream_rows(cells, 8, out, CHUNK_BYTES / 8, [=](uint64_t f, uint64_t n, void *dst, uint64_t *, cudaStream_t st) -> int {
+      const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(n, 256), (uint64_t)sms * 16);
+      LAUNCH("dotplot_finish", st, dotplot_finish_kernel<<<grid, 256, 0, st>>>(im + f, n, (double *)dst));
+      return KMG_OK;
+    });
+  };
+  const int rc = body();
+  cudaStreamSynchronize(s);
+  dfree(blk, s); dfree(img, s);
+  if (rc != KMG_OK) return rc;
+  prof_bytes("dotplot_bin", row_bytes * (double)M + 8.0 * (double)cells);
+  prof_bytes("dotplot_finish", 16.0 * (double)cells);
+  return KMG_OK;
+}
+
+extern "C" int kmg_query_dotplot(const kmg_index *ix, const char *q, int64_t qlen, int k, int rc, int64_t x0, int64_t x1, int nx,
+                                 int64_t y0, int64_t y1, int ny, uint32_t max_count, double *out) {
+  if (!ix) return fail(KMG_ERR_ARG, "index is NULL");
+  if (rc != 0 && rc != 1) return fail(KMG_ERR_ARG, "rc must be 0 or 1");
+  TRY(dotplot_args(x0, x1, nx, y0, y1, ny, out));
+  kmg_query *st = nullptr;
+  uint64_t M = 0;
+  TRY(query_seq(ix, q, qlen, k, rc == 1, max_count ? max_count : UINT32_MAX, &st, &M));
+  const ProbeRows rows{st->hit_i, st->hit_start, ix->pos};
+  const int rv = dotplot_run(rows, st->row_off, st->H, M, 4.0, dot_axis(x0, x1, nx), dot_axis(y0, y1, ny), out);
+  kmg_query_free(st);
+  return rv;
+}
+
+extern "C" int kmg_join_dotplot(const kmg_index *a, const kmg_index *b, int64_t x0, int64_t x1, int nx, int64_t y0, int64_t y1, int ny,
+                                uint32_t max_count, double *out) {
+  if (!a || !b) return fail(KMG_ERR_ARG, "index is NULL");
+  TRY(dotplot_args(x0, x1, nx, y0, y1, ny, out));
+  kmg_join *j = nullptr;
+  uint64_t M = 0;
+  TRY(join_begin(a, b, max_count ? max_count : UINT32_MAX, &j, &M));
+  const JoinRows rows{j->hit_astart, j->hit_bstart, j->hit_cb, a->pos, b->pos};
+  const int rv = dotplot_run(rows, j->row_off, j->H, M, 8.0, dot_axis(x0, x1, nx), dot_axis(y0, y1, ny), out);
+  kmg_join_free(j);
+  return rv;
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -351,11 +351,12 @@ depth_lookup_kernel(const SeqView sv, int64_t first, int64_t rows, const KeyHash
 // ---- pass 2: ordered compaction of the hits + chained 64-bit scan of their row counts --------------------
 //   coordinate i of a hit: FROM_SEQ: 1-based END of the window (src/kmer_pos.c:127,132: `i` is one past the
 //   window); else the record's own i.
+//   max_count: a window whose k-mer has more positions is a miss (dot plots drop repeats); UINT32_MAX = no limit.
 template <int THREADS, int ITEMS, bool FROM_SEQ>
 __global__ void __launch_bounds__(THREADS)
 probe_compact_kernel(const uint2 *__restrict__ found, int64_t coord0, const int32_t *__restrict__ i_in, int64_t n_in,
                      const uint64_t *__restrict__ n_dev, int32_t *__restrict__ hit_i, uint32_t *__restrict__ hit_start,
-                     uint64_t *__restrict__ row_off, QueryStats *qs, Pair64 *status, uint32_t *ticket) {
+                     uint64_t *__restrict__ row_off, QueryStats *qs, Pair64 *status, uint32_t *ticket, const uint32_t max_count) {
   constexpr int TILE = THREADS * ITEMS, WARPS = THREADS / 32;
   static_assert(ITEMS % 2 == 0, "pairs of windows are read as one 16-byte word");
   static_assert(TILE <= 4096, "rows inside a tile: at most TILE * (2^32 - 1) < 2^48");
@@ -383,6 +384,8 @@ probe_compact_kernel(const uint2 *__restrict__ found, int64_t coord0, const int3
 #pragma unroll
     for (int i = 0; i < ITEMS; ++i) f[i] = t0 + i < total ? found[t0 + i] : make_uint2(0u, 0u);
   }
+#pragma unroll
+  for (int i = 0; i < ITEMS; ++i) if (f[i].y > max_count) f[i].y = 0;
   uint32_t hmine = 0;
   uint64_t rmine = 0;
 #pragma unroll
@@ -484,11 +487,12 @@ __global__ void revcomp_kernel(const uint8_t *__restrict__ in, int64_t L, uint8_
 // kmer_pair_pos (src/kmer_hash.c:1174-1203): for every k-mer of `a` that `b` also holds, rows (a_pos, b_pos),
 // a position outer, b position inner.  a's distinct keys are looked up in b's key table (probe_lookup_kernel,
 // record source); this kernel compacts the shared ones in a's order and scans their row counts ca * cb.
+// max_count: a k-mer with more positions in either index is not shared (UINT32_MAX = no limit).
 template <int THREADS, int ITEMS>
 __global__ void __launch_bounds__(THREADS)
 join_compact_kernel(const uint2 *__restrict__ found, const uint32_t *__restrict__ ustart_a, uint64_t U,
                     uint32_t *__restrict__ hit_astart, uint32_t *__restrict__ hit_bstart, uint32_t *__restrict__ hit_cb,
-                    uint64_t *__restrict__ row_off, QueryStats *qs, Pair64 *status, uint32_t *ticket) {
+                    uint64_t *__restrict__ row_off, QueryStats *qs, Pair64 *status, uint32_t *ticket, const uint32_t max_count) {
   constexpr int TILE = THREADS * ITEMS, WARPS = THREADS / 32;
   __shared__ uint32_t s_tile, s_wh[WARPS];
   __shared__ uint64_t s_wr[WARPS], s_bh, s_br;
@@ -508,6 +512,7 @@ join_compact_kernel(const uint2 *__restrict__ found, const uint32_t *__restrict_
 #pragma unroll
   for (int i = 0; i < ITEMS; ++i) {
     f[i] = t0 + i < U ? found[t0 + i] : make_uint2(0u, 0u);
+    if (f[i].y > max_count || as[i + 1] - as[i] > max_count) f[i].y = 0;
     rows[i] = f[i].y ? (uint64_t)(as[i + 1] - as[i]) * f[i].y : 0;
     hmine += f[i].y != 0;
     rmine += rows[i];
@@ -569,6 +574,94 @@ join_emit_kernel(const uint32_t *__restrict__ hit_astart, const uint32_t *__rest
     const uint64_t ia = within / cb;                       // a position outer, b position inner (src/kmer_hash.c:1190-1195)
     out[b0 + s] = make_int2((int)pos_a[hit_astart[h] + ia], (int)pos_b[hit_bstart[h] + (within - ia * cb)]);
   }
+}
+
+// ---- dot plots: the rows of a probe or a join counted into an nx x ny image -----------------------------------------
+// One axis of the image: a coordinate v is in the window iff 0 <= v - lo < range, and goes to bin floor((v - lo) * n / range).
+// (v - lo) * n < 2^31 * 2^31, so the quotient is exact from the host's inv = floor((2^64 - 1) / range): umulhi(p, inv) is
+// the quotient or one less (inv > 2^64 / range - 1 and p < 2^62), and one compare corrects it.
+struct DotAxis {
+  uint64_t lo, range, inv;
+  uint32_t n;
+};
+constexpr uint32_t DOT_NONE = 0xFFFFFFFFu;
+
+__device__ __forceinline__ uint32_t dot_bin(const DotAxis &a, uint32_t v) {
+  const uint64_t d = (uint64_t)v - a.lo;                  // wraps to >= 2^63 below the window
+  if (d >= a.range) return DOT_NONE;
+  const uint64_t p = d * a.n;
+  uint64_t q = __umul64hi(p, a.inv);
+  if ((q + 1) * a.range <= p) ++q;
+  return (uint32_t)q;
+}
+
+// Row sources: (x, y) of the within-th row of hit h.  A probe pairs the hit's query coordinate with the within-th position
+// of its k-mer (probe_emit_kernel); a join takes a's positions outer and b's inner (join_emit_kernel), with a 32-bit
+// division whenever the row number within the hit fits 32 bits.
+struct ProbeRows {
+  const int32_t *hit_i;
+  const uint32_t *hit_start, *pos;
+  __device__ __forceinline__ uint2 operator()(uint64_t h, uint64_t within) const {
+    return make_uint2((uint32_t)hit_i[h], pos[hit_start[h] + within]);
+  }
+};
+struct JoinRows {
+  const uint32_t *hit_astart, *hit_bstart, *hit_cb, *pos_a, *pos_b;
+  __device__ __forceinline__ uint2 operator()(uint64_t h, uint64_t within) const {
+    const uint32_t cb = hit_cb[h];
+    const uint64_t ia = within <= 0xFFFFFFFFull ? (uint64_t)((uint32_t)within / cb) : within / cb;
+    return make_uint2(pos_a[hit_astart[h] + ia], pos_b[hit_bstart[h] + (within - ia * cb)]);
+  }
+};
+
+// Rows [first, first + nrows) into the image img[bx + by * nx] (u64 counts), balanced by rows like the emit kernels
+// (block_segments).  Lanes of a warp hold consecutive rows, which along a diagonal or inside one hit mostly share a bin:
+// every run of equal bins among the lanes (compared with lane - 1) is summed by its first lane, which issues one 64-bit
+// atomic for the run.  Rows outside the window are dropped.
+template <int THREADS, class Rows>
+__global__ void __launch_bounds__(THREADS)
+dotplot_bin_kernel(const Rows rows, const uint64_t *__restrict__ row_off, uint64_t H, uint64_t first, uint64_t nrows,
+                   const uint64_t *__restrict__ blk_first, const DotAxis ax, const DotAxis ay, unsigned long long *__restrict__ img) {
+  constexpr int PER = 8, T = THREADS * PER;
+  __shared__ __align__(16) uint8_t s_flag[T];
+  __shared__ __align__(16) uint32_t s_seg[T];
+  __shared__ uint32_t s_warp[THREADS / 32];
+  __shared__ uint64_t s_first;
+  const uint64_t b0 = (uint64_t)blockIdx.x * T;
+  if (b0 >= nrows) return;
+  const uint64_t r0 = first + b0;
+  const uint64_t h0 = block_segments<THREADS, PER, uint64_t>(row_off, H, r0, blk_first[blockIdx.x], s_flag, s_seg, s_warp, &s_first);
+  uint32_t bins[PER];                                     // all rows' loads first, then the atomics: the loads overlap
+#pragma unroll
+  for (int j = 0; j < PER; ++j) {
+    const uint32_t s = j * THREADS + threadIdx.x;
+    bins[j] = DOT_NONE;
+    if (b0 + s < nrows) {                                 // every lane stays for the warp-wide run detection below
+      const uint64_t h = h0 + s_seg[s];
+      const uint2 xy = rows(h, r0 + s - row_off[h]);
+      const uint32_t bx = dot_bin(ax, xy.x), by = dot_bin(ay, xy.y);
+      if (bx != DOT_NONE && by != DOT_NONE) bins[j] = bx + by * ax.n;
+    }
+  }
+  const unsigned lane = lane_id();
+#pragma unroll
+  for (int j = 0; j < PER; ++j) {
+    const uint32_t bin = bins[j];
+    const uint32_t prev = __shfl_up_sync(FULL, bin, 1);
+    const bool head = lane == 0 || bin != prev;
+    const uint32_t heads = __ballot_sync(FULL, head);
+    if (head && bin != DOT_NONE) {
+      const uint32_t later = lane == 31 ? 0u : heads & (0xFFFFFFFFu << (lane + 1));
+      const uint32_t run = (later ? (uint32_t)__ffs(later) - 1 : 32u) - lane;
+      atomicAdd(img + bin, (unsigned long long)run);
+    }
+  }
+}
+
+// u64 counts -> doubles (exact below 2^53)
+__global__ void dotplot_finish_kernel(const unsigned long long *__restrict__ img, uint64_t n, double *__restrict__ out) {
+  for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
+    out[i] = (double)img[i];
 }
 
 }  // namespace kmg

@@ -12,6 +12,8 @@
  *   kmer_pair_pos(ptr.a, ptr.b)             replaces src/kmer_hash.c:1174-1203 (which crashes: test.R:330-331)
  *   count_kmers(ptr, params, seq)           replaces src/kmer_hash.c:548-591 (count.kmers: per-source counts)
  *   sequence_kmer_depth(ptr, seq, strands)  additive: per-window counts of a sequence's k-mers (seq.kmer.depth)
+ *   sequence_kmer_dotplot(ptr, seq, k, params), kmer_pair_dotplot(ptr.a, ptr.b, params)
+ *                                           additive: binned dot plots of seq.kmer.pos / kmer.pairs rows
  *   R_init_kmer_hash                        replaces src/kmer_hash.c:1221-1224
  *
  * Differences a user can observe: k-mers come out in the order of a mix of their 2-bit key (ascending key
@@ -434,6 +436,58 @@ SEXP sequence_kmer_depth(SEXP ptr_r, SEXP seq_r, SEXP strands_r) {
   return m;
 }
 
+/* seq.kmer.dotplot / kmer.pairs.dotplot (additive; INTEGRATION.md): the rows seq.kmer.pos or kmer.pairs would return,
+ * counted into an nx x ny double matrix on the device, so neither the 2^31-1 row limit nor the transfer of the rows
+ * applies.  Cell [bx, by] (1-based in R: [bx+1, by+1]) counts the rows with floor((x - x0) * nx / (x1 - x0)) = bx and
+ * floor((y - y0) * ny / (y1 - y0)) = by, over the half-open windows [x0, x1) x [y0, y1); max.count > 0 drops the k-mers
+ * with more positions. */
+static void dotplot_bins(const int *p, int *nx, int *ny) {
+  *nx = p[2];
+  *ny = p[5];
+  if (*nx < 1 || *ny < 1) error("bins must be positive");
+  if ((int64_t)*nx * *ny > (int64_t)INT_MAX)
+    error("a dot plot of %d x %d bins would have %lld cells, more than an R matrix can hold (2^31-1)", *nx, *ny, (long long)*nx * *ny);
+}
+
+/* params = as.integer(c(x0, x1, nx, y0, y1, ny, rc, max.count)) */
+SEXP sequence_kmer_dotplot(SEXP ptr_r, SEXP seq_r, SEXP k_r, SEXP params_r) {
+  kmer_handle *h = index_handle_or_error(ptr_r);
+  if (TYPEOF(seq_r) != STRSXP || length(seq_r) != 1) error("seq_r should be a single sequence");
+  if (TYPEOF(k_r) != INTSXP || length(k_r) != 1) error("k should be an integer of length 1");
+  if (TYPEOF(params_r) != INTSXP || length(params_r) != 8) error("params should be an integer vector of length 8");
+  const int k = INTEGER(k_r)[0];
+  SEXP s = STRING_ELT(seq_r, 0);
+  const char *allow = getenv("KMERGPU_ALLOW_K32");
+  const int kmax = (allow && allow[0] == '1') ? 32 : 31;
+  if (length(s) <= k || k > kmax || k < 1) error("the sequence should be longer than k and k should not be longer than 31");
+  const int *p = INTEGER(params_r);
+  if (p[6] != 0 && p[6] != 1) error("rc should be TRUE or FALSE");
+  if (p[7] < 0) error("max.count should be 0 (no limit) or positive");
+  int nx, ny;
+  dotplot_bins(p, &nx, &ny);
+  SEXP m = PROTECT(allocMatrix(REALSXP, nx, ny));
+  const int rc = kmg_query_dotplot(h->index, CHAR(s), (int64_t)length(s), k, p[6], p[0], p[1], nx, p[3], p[4], ny, (uint32_t)p[7], REAL(m));
+  UNPROTECT(1);
+  if (rc != KMG_OK) error("seq.kmer.dotplot failed: %s", kmg_last_error());
+  return m;
+}
+
+/* params = as.integer(c(a0, a1, nx, b0, b1, ny, max.count)): x = position in a, y = position in b */
+SEXP kmer_pair_dotplot(SEXP ptr_a, SEXP ptr_b, SEXP params_r) {
+  kmer_handle *a = index_handle_or_error(ptr_a);
+  kmer_handle *b = index_handle_or_error(ptr_b);
+  if (TYPEOF(params_r) != INTSXP || length(params_r) != 7) error("params should be an integer vector of length 7");
+  const int *p = INTEGER(params_r);
+  if (p[6] < 0) error("max.count should be 0 (no limit) or positive");
+  int nx, ny;
+  dotplot_bins(p, &nx, &ny);
+  SEXP m = PROTECT(allocMatrix(REALSXP, nx, ny));
+  const int rc = kmg_join_dotplot(a->index, b->index, p[0], p[1], nx, p[3], p[4], ny, (uint32_t)p[6], REAL(m));
+  UNPROTECT(1);
+  if (rc != KMG_OK) error("kmer.pairs.dotplot failed: %s", kmg_last_error());
+  return m;
+}
+
 static const R_CallMethodDef call_methods[] = {
     {"make_kmer_h_index", (DL_FUNC)&make_kmer_h_index, 3},
     {"kmer_positions", (DL_FUNC)&kmer_positions, 2},
@@ -443,6 +497,8 @@ static const R_CallMethodDef call_methods[] = {
     {"make_kmer_h_index_file", (DL_FUNC)&make_kmer_h_index_file, 4},
     {"count_kmers_file", (DL_FUNC)&count_kmers_file, 3},
     {"sequence_kmer_depth", (DL_FUNC)&sequence_kmer_depth, 3},
+    {"sequence_kmer_dotplot", (DL_FUNC)&sequence_kmer_dotplot, 4},
+    {"kmer_pair_dotplot", (DL_FUNC)&kmer_pair_dotplot, 3},
     {NULL, NULL, 0}};
 
 void R_init_kmer_hash(DllInfo *info) { R_registerRoutines(info, NULL, call_methods, NULL, NULL); }
