@@ -160,6 +160,26 @@ int kmg_query_dotplot(const kmg_index *idx, const char *q, int64_t qlen, int k, 
 int kmg_join_dotplot(const kmg_index *a, const kmg_index *b, int64_t x0, int64_t x1, int nx, int64_t y0, int64_t y1, int ny,
                      uint32_t max_count, double *out /* nx*ny */);
 
+/* ---- match segments: maximal diagonal runs of seq.kmer.pos rows, found on the device (additive) ---------------------
+ * S = the rows kmg_query_begin (rc = 0) or kmg_query_begin_rc (rc = 1) + kmg_query_emit give for (idx, q, qlen, k): i =
+ * 1-based END of the query window (with rc = 1 a coordinate of the reverse-complemented string), j = 1-based start in the
+ * index.  max_count > 0: k-mers with more than max_count positions in the index add no rows (as kmg_query_dotplot).
+ * A run is a maximal sequence of rows (i+t, j+t), t = 0..n-1, all in S: (i-1, j-1) and (i+n, j+n) are not in S.  Every
+ * row is in exactly one run, so the n of all runs sum to |S|.  When the query's k is the index's, a run of n rows means
+ * query bases [i-k+1, i+n-1] equal index bases [j, j+n+k-2] in 2-bit code (the window rule of the index aside).
+ * kmg_segments_begin finds the runs with n >= min_rows (0 and 1: every run) and reports their number R; emit writes them
+ * as interleaved int32 (i, j, n), column-major 3 x R like kmg_pairs, ordered by (i, j) of their first row (the order of
+ * the rows of kmg_query_emit), into device, pinned or pageable memory; emit_chunk writes runs [first, first+n).  The
+ * handle holds only the 12 R bytes of the result.  An empty index, query or intersection gives R = 0.
+ * KMG_ERR_ARG: NULL handle/st/out, rc not 0/1, runs outside [0, R); KMG_ERR_K and the query length check (KMG_ERR_RANGE)
+ * of kmg_query_begin; KMG_ERR_RANGE: more than 2^31 - 1 runs before the min_rows filter. */
+typedef struct kmg_segments kmg_segments;
+int kmg_segments_begin(const kmg_index *idx, const char *q, int64_t qlen, int k, int rc, uint32_t max_count,
+                       uint32_t min_rows, kmg_segments **st, uint64_t *R);
+int kmg_segments_emit(kmg_segments *st, int32_t *out /* 3R */);
+int kmg_segments_emit_chunk(kmg_segments *st, uint64_t first, uint64_t n, int32_t *out /* 3n */);
+int kmg_segments_free(kmg_segments *st);   /* NULL accepted */
+
 /* ---- sharded build (one process per GPU; the exchange itself is the host's NCCL all-to-all) ----
  * A rank holds bytes [g0,g1) of a global sequence of length L in device memory at d_seq (d_seq[0]
  * is byte g0) and owns the window starts [s0,s1), g0 <= max(s0-1,0), g1 >= min(L, s1+k-1).

@@ -21,7 +21,7 @@ from . import _lib
 from ._lib import KmgError, check
 
 __all__ = ["KmerHash", "KmerCounts", "SequenceFile", "make_kmer_hash_file", "count_kmers_file", "make_kmer_hash", "kmer_pos", "seq_kmer_pos", "kmer_pairs", "count_kmers", "kmer_spectrum",
-           "seq_kmer_depth", "seq_kmer_dotplot", "kmer_pairs_dotplot", "pinned_empty", "KmgError",
+           "seq_kmer_depth", "seq_kmer_dotplot", "kmer_pairs_dotplot", "seq_kmer_segments", "pinned_empty", "KmgError",
            "OPT_KMER", "OPT_POS", "OPT_PAIRS", "OPT_COUNT", "NA_INTEGER"]
 
 # opt.flag bits, src/kmer_hash.c:17 (pos_opt_flags) in the reference
@@ -623,6 +623,51 @@ def kmer_pairs_dotplot(ptr_a, ptr_b, *, a_range, b_range, bins=(1000, 1000), max
     nx, ny, (x0, x1), (y0, y1), mc, out = _dotplot_args(bins, (a_range, b_range), max_count, out)
     check(_L.kmg_join_dotplot(a._handle(), b._handle(), x0, x1, nx, y0, y1, ny, mc, _out_ptr(out)))
     return out
+
+
+def seq_kmer_segments(ptr, seq, k, *, reverse_complement=False, max_count=0, min_rows=1, allow_k32=False, out=None):
+    """seq.kmer.segments (additive; the R closure is in INTEGRATION.md): the rows seq_kmer_pos(ptr, seq, k,
+    reverse_complement=...) would return, joined on the device into match segments -- maximal diagonal runs of rows
+    (i + t, j + t), t = 0 .. n - 1.  Every row belongs to exactly one run.
+
+    Returns an (R, 3) int32 array of (i, j, n): the first row of the run (i = 1-based END of the query window, of the
+    reverse-complemented string with reverse_complement=True; j = 1-based start in the index) and its row count, ordered
+    by (i, j).  A run of n rows covers query bases [i - k + 1, i + n - 1] and index bases [j, j + n + k - 2].
+    max_count > 0 drops the k-mers with more positions in the index before the runs are found; only runs with
+    n >= min_rows are returned (0 and 1: all).  `out` may supply the result (numpy, pinned or a torch device tensor of at
+    least 3 R int32)."""
+    ix = _extract_index(ptr)
+    if isinstance(seq, (list, tuple)):
+        if len(seq) != 1:
+            raise ValueError("seq_r should be a single sequence")
+        seq = seq[0]
+    k = int(k)
+    p, n, keep = _seq_buffer(seq)
+    if n <= k or k > (32 if allow_k32 else 31):
+        raise ValueError("the sequence should be longer than k and k should not be longer than 31")
+    max_count, min_rows = int(max_count), int(min_rows)
+    if not 0 <= max_count < 2**32:
+        raise ValueError("max_count must be 0 (no limit) or a positive 32-bit count")
+    if not 0 <= min_rows < 2**32:
+        raise ValueError("min_rows must be a non-negative 32-bit count")
+    st, R = C.c_void_p(), C.c_uint64()
+    check(_L.kmg_segments_begin(ix._handle(), p, n, k, int(bool(reverse_complement)), max_count, min_rows,
+                                C.byref(st), C.byref(R)))
+    del keep
+    try:
+        R = R.value
+        if R > INT_MAX:
+            raise OverflowError(f"{R} segments exceed an R matrix extent")
+        if out is None:
+            out = np.empty((R, 3), np.int32)
+        else:
+            size = out.nbytes if isinstance(out, np.ndarray) else out.numel() * out.element_size()
+            if size < 12 * R:
+                raise ValueError(f"out holds {size} bytes; the {R} segments need {12 * R}")
+        check(_L.kmg_segments_emit(st, _out_ptr(out)))
+    finally:
+        _L.kmg_segments_free(st)
+    return out[:R] if isinstance(out, np.ndarray) and out.ndim == 2 else out
 
 
 def profile(enable: bool | None = None, reset: bool = False) -> dict:

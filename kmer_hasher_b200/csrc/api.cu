@@ -21,6 +21,7 @@
 #include "csr.cuh"
 #include "lookback.cuh"
 #include "probe.cuh"
+#include "segments.cuh"
 #include "sort.cuh"
 #include "windows.cuh"
 
@@ -1743,6 +1744,199 @@ extern "C" int kmg_join_dotplot(const kmg_index *a, const kmg_index *b, int64_t 
   const int rv = dotplot_run(rows, j->row_off, j->H, M, 8.0, dot_axis(x0, x1, nx), dot_axis(y0, y1, ny), out);
   kmg_join_free(j);
   return rv;
+}
+
+// ------------------------------------------------------------------------------------------------
+// match segments: maximal diagonal runs of a probe's rows (segments.cuh)
+// ------------------------------------------------------------------------------------------------
+struct kmg_segments {
+  int device = 0;
+  uint64_t R = 0;
+  int32_t *rows = nullptr;      // [3R]: (i, j, n) per run
+};
+constexpr uint64_t SEG_SLICE_ROWS = uint64_t(1) << 30;   // rows per mark launch: the block-start and status scratch stay small
+constexpr uint64_t SEG_CAP0 = uint64_t(1) << 26;         // starts / ends held before the first resize (20 bytes each)
+constexpr int SEG_PAIR_ITEMS = 8, SEG_PAIR_TILE = 256 * SEG_PAIR_ITEMS;
+
+// p[0, keep) moved into a fresh array of cap elements
+template <typename T>
+static int seg_grow(T *&p, uint64_t keep, uint64_t cap, cudaStream_t s) {
+  T *q = nullptr;
+  TRY(dalloc(&q, (size_t)cap, s));
+  if (keep) CU(cudaMemcpyAsync(q, p, keep * sizeof(T), cudaMemcpyDeviceToDevice, s));
+  dfree(p, s);
+  p = q;
+  return KMG_OK;
+}
+
+// Run starts (i, j) and run ends (diagonal key, i) of the probe st, each in row order, into arrays of at least R0 entries.
+static int segments_mark(const kmg_query *st, const uint32_t *pos, int2 *&starts, uint64_t *&ekey, uint32_t *&ei, uint64_t *R0) {
+  cudaStream_t s = g_ctx.stream();
+  const uint64_t M = st->M;
+  const uint64_t slice_tiles = ceil_div<uint64_t>(std::min(M, SEG_SLICE_ROWS), EMIT_TILE);
+  uint64_t cap = std::min(M, SEG_CAP0), bs = 0, be = 0;
+  uint64_t *blk = nullptr, *tot = nullptr;
+  Pair64 *status = nullptr;
+  uint32_t *ticket = nullptr;
+  auto body = [&]() -> int {
+    TRY(dalloc(&starts, (size_t)cap, s));
+    TRY(dalloc(&ekey, (size_t)cap, s));
+    TRY(dalloc(&ei, (size_t)cap, s));
+    TRY(dalloc(&blk, (size_t)slice_tiles, s));
+    TRY(dalloc(&status, (size_t)slice_tiles, s));
+    TRY(dalloc(&ticket, 1, s));
+    TRY(dalloc(&tot, 2, s));
+    for (uint64_t first = 0; first < M;) {
+      const uint64_t n = std::min(SEG_SLICE_ROWS, M - first);
+      const uint64_t tiles = ceil_div<uint64_t>(n, EMIT_TILE);
+      CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
+      CU(cudaMemsetAsync(ticket, 0, 4, s));
+      TRY(block_starts(st->row_off, st->H, first, n, s, blk));
+      LAUNCH("segments_mark", s, segments_mark_kernel<EMIT_THREADS><<<(unsigned)tiles, EMIT_THREADS, 0, s>>>(
+                                     st->hit_i, st->hit_start, st->row_off, st->H, M, pos, first, n, blk, status, ticket, bs, be,
+                                     cap, starts, ekey, ei, tot));
+      uint64_t h[2];
+      CU(cudaMemcpyAsync(h, tot, sizeof h, cudaMemcpyDeviceToHost, s));
+      CU(cudaStreamSynchronize(s));
+      const uint64_t need = std::max(bs + h[0], be + h[1]);
+      if (need > (uint64_t)INT32_MAX)
+        return fail(KMG_ERR_RANGE, "more than 2^31 - 1 runs (%llu so far) to pair", (unsigned long long)need);
+      if (need > cap) {                                   // the slice did not fit: keep what is done, make room, run it again
+        const uint64_t ncap = std::min<uint64_t>(std::min(M, (uint64_t)INT32_MAX), need + need / 4);
+        TRY(seg_grow(starts, bs, ncap, s));
+        TRY(seg_grow(ekey, be, ncap, s));
+        TRY(seg_grow(ei, be, ncap, s));
+        cap = ncap;
+        continue;
+      }
+      bs += h[0]; be += h[1];
+      first += n;
+    }
+    if (bs != be)
+      return fail(KMG_ERR_CUDA, "internal error: %llu run starts but %llu run ends", (unsigned long long)bs, (unsigned long long)be);
+    return KMG_OK;
+  };
+  const int rc = body();
+  dfree(blk, s); dfree(status, s); dfree(ticket, s); dfree(tot, s);
+  // rows (4 B) and one neighbouring position on either side; hits (16 B); the starts (8 B) and ends (12 B) written
+  if (rc == KMG_OK) prof_bytes("segments_mark", 12.0 * M + 16.0 * st->H + 20.0 * bs);
+  *R0 = bs;
+  return rc;
+}
+
+// The runs of the probe (idx, q, qlen, k, rc, max_count) with at least min_rows rows, as (i, j, n) triples in the order
+// of their first rows: *rows (device, 12 * *R bytes) or nullptr when *R = 0.
+static int segments_run(const kmg_index *ix, const char *q, int64_t qlen, int k, int rc, uint32_t max_count, uint32_t min_rows,
+                        int32_t **rows, uint64_t *R) {
+  *rows = nullptr;
+  *R = 0;
+  kmg_query *st = nullptr;
+  uint64_t M = 0;
+  TRY(query_seq(ix, q, qlen, k, rc == 1, max_count ? max_count : UINT32_MAX, &st, &M));
+  if (M == 0) { kmg_query_free(st); return KMG_OK; }
+  cudaStream_t s = g_ctx.stream();
+  int2 *starts = nullptr;
+  uint64_t *ekey = nullptr, *tot = nullptr;
+  uint32_t *ei = nullptr, *ticket = nullptr;
+  Pair64 *status = nullptr;
+  int32_t *tmp = nullptr, *out = nullptr;
+  kmg_index *ends = nullptr;
+  uint64_t R0 = 0;
+  auto body = [&]() -> int {
+    const int m = segments_mark(st, ix->pos, starts, ekey, ei, &R0);
+    kmg_query_free(st);                                   // the probe is done with: only the runs stay
+    st = nullptr;
+    TRY(m);
+    // the ends sorted by diagonal, i ascending inside one: keys d + 2^31 < 2^32 are the 32 bits of a 16-mer
+    TRY(kmg_build_records(ekey, ei, (int64_t)R0, 16, &ends));
+    dfree(ekey, s); dfree(ei, s);
+    const uint64_t tiles = ceil_div<uint64_t>(R0, SEG_PAIR_TILE);
+    TRY(dalloc(&tmp, (size_t)(3 * R0), s));
+    TRY(dalloc(&status, (size_t)tiles, s));
+    TRY(dalloc(&ticket, 1, s));
+    TRY(dalloc(&tot, 2, s));
+    CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
+    CU(cudaMemsetAsync(ticket, 0, 4, s));
+    LAUNCH("segments_pair", s, segments_pair_kernel<256, SEG_PAIR_ITEMS><<<(unsigned)tiles, 256, 0, s>>>(
+                                   starts, R0, ends->ukeys, ends->U, ends->ustart, ends->pos, min_rows, status, ticket, tmp, tot));
+    uint64_t h[2];
+    CU(cudaMemcpyAsync(h, tot, sizeof h, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    if (h[1] != M)
+      return fail(KMG_ERR_CUDA, "internal error: the runs hold %llu rows, the probe %llu", (unsigned long long)h[1], (unsigned long long)M);
+    prof_bytes("segments_pair", 8.0 * R0 + 12.0 * R0 + 12.0 * h[0]);   // starts; the diagonal's key and end; the triples
+    if (h[0] == R0) { out = tmp; tmp = nullptr; }
+    else if (h[0]) {                                      // keep exactly the runs that passed min_rows
+      TRY(dalloc(&out, (size_t)(3 * h[0]), s));
+      CU(cudaMemcpyAsync(out, tmp, 12 * h[0], cudaMemcpyDeviceToDevice, s));
+      CU(cudaStreamSynchronize(s));
+    }
+    *R = h[0];
+    return KMG_OK;
+  };
+  const int rv = body();
+  if (st) kmg_query_free(st);
+  cudaStreamSynchronize(s);
+  dfree(starts, s); dfree(ekey, s); dfree(ei, s); dfree(tot, s); dfree(ticket, s); dfree(status, s); dfree(tmp, s);
+  if (ends) kmg_free(ends);
+  if (rv != KMG_OK) { dfree(out, s); *R = 0; return rv; }
+  *rows = out;
+  return KMG_OK;
+}
+
+extern "C" int kmg_segments_begin(const kmg_index *ix, const char *q, int64_t qlen, int k, int rc, uint32_t max_count,
+                                  uint32_t min_rows, kmg_segments **st, uint64_t *R) {
+  if (!st) return fail(KMG_ERR_ARG, "st is NULL");
+  *st = nullptr;
+  if (!ix) return fail(KMG_ERR_ARG, "index is NULL");
+  if (rc != 0 && rc != 1) return fail(KMG_ERR_ARG, "rc must be 0 or 1");
+  kmg_segments *g = new (std::nothrow) kmg_segments();
+  if (!g) return fail(KMG_ERR_NOMEM, "host allocation failed");
+  g->device = ix->device;
+  int rv = segments_run(ix, q, qlen, k, rc, max_count, min_rows, &g->rows, &g->R);
+  if (rv == KMG_ERR_UNSTABLE) rv = segments_run(ix, q, qlen, k, rc, max_count, min_rows, &g->rows, &g->R);   // the sort now ranks by bitmap
+  if (rv != KMG_OK) { delete g; return rv; }
+  *st = g;
+  if (R) *R = g->R;
+  return KMG_OK;
+}
+
+extern "C" int kmg_segments_emit_chunk(kmg_segments *g, uint64_t first, uint64_t n, int32_t *out) {
+  if (!g) return fail(KMG_ERR_ARG, "segments handle is NULL");
+  TRY(ctx_init());
+  if (g->device != g_ctx.device)
+    return fail(KMG_ERR_ARG, "the segments live on device %d but this thread works on device %d", g->device, g_ctx.device);
+  if (first > g->R || n > g->R - first) return fail(KMG_ERR_ARG, "runs outside the result");
+  if (n == 0) return KMG_OK;
+  if (!out) return fail(KMG_ERR_ARG, "out is NULL");
+  const int32_t *rows = g->rows;
+  const int sms = g_ctx.sms;
+  int rc = stream_rows(n, 12, out, CHUNK_BYTES / 12, [=](uint64_t f, uint64_t cnt, void *dst, uint64_t *, cudaStream_t s) -> int {
+    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(3 * cnt, 256), (uint64_t)sms * 16);
+    LAUNCH("segments_emit", s, segments_emit_kernel<<<grid, 256, 0, s>>>(rows + 3 * (first + f), 3 * cnt, (int32_t *)dst));
+    return KMG_OK;
+  });
+  prof_bytes("segments_emit", 24.0 * n);
+  return rc;
+}
+
+extern "C" int kmg_segments_emit(kmg_segments *g, int32_t *out) {
+  if (!g) return fail(KMG_ERR_ARG, "segments handle is NULL");
+  return kmg_segments_emit_chunk(g, 0, g->R, out);
+}
+
+extern "C" int kmg_segments_free(kmg_segments *g) {
+  if (!g) return KMG_OK;
+  int prev = -1;
+  cudaGetDevice(&prev);
+  cudaSetDevice(g->device);
+  const bool mine = g_ctx.ready && g_ctx.device == g->device;
+  if (mine) cudaStreamSynchronize(g_ctx.stream()); else cudaDeviceSynchronize();
+  if (g->rows) g_arena[g->device & 63].put(g->rows, nullptr, true);
+  cudaGetLastError();
+  if (prev >= 0) cudaSetDevice(prev);
+  delete g;
+  return KMG_OK;
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -14,6 +14,8 @@
  *   sequence_kmer_depth(ptr, seq, strands)  additive: per-window counts of a sequence's k-mers (seq.kmer.depth)
  *   sequence_kmer_dotplot(ptr, seq, k, params), kmer_pair_dotplot(ptr.a, ptr.b, params)
  *                                           additive: binned dot plots of seq.kmer.pos / kmer.pairs rows
+ *   sequence_kmer_segments(ptr, seq, k, params)
+ *                                           additive: match segments, the diagonal runs of seq.kmer.pos rows
  *   R_init_kmer_hash                        replaces src/kmer_hash.c:1221-1224
  *
  * Differences a user can observe: k-mers come out in the order of a mix of their 2-bit key (ascending key
@@ -488,6 +490,50 @@ SEXP kmer_pair_dotplot(SEXP ptr_a, SEXP ptr_b, SEXP params_r) {
   return m;
 }
 
+/* seq.kmer.segments (additive; INTEGRATION.md): the rows seq.kmer.pos would return, joined on the device into maximal
+ * diagonal runs (i+t, j+t), t = 0..n-1, as a 3 x R integer matrix of (i, j, n) ordered by (i, j); seq.kmer.segments()
+ * names and transposes.  params = as.integer(c(rc, max.count, min.rows)): max.count > 0 drops the k-mers with more
+ * positions, min.rows keeps the runs of at least that many rows. */
+static void finalise_segments_guard(SEXP g) {
+  kmg_segments *st = (kmg_segments *)R_ExternalPtrAddr(g);
+  if (st) kmg_segments_free(st);
+  R_ClearExternalPtr(g);
+}
+
+SEXP sequence_kmer_segments(SEXP ptr_r, SEXP seq_r, SEXP k_r, SEXP params_r) {
+  kmer_handle *h = index_handle_or_error(ptr_r);
+  if (TYPEOF(seq_r) != STRSXP || length(seq_r) != 1) error("seq_r should be a single sequence");
+  if (TYPEOF(k_r) != INTSXP || length(k_r) != 1) error("k should be an integer of length 1");
+  if (TYPEOF(params_r) != INTSXP || length(params_r) != 3) error("params should be an integer vector of length 3");
+  const int k = INTEGER(k_r)[0];
+  SEXP s = STRING_ELT(seq_r, 0);
+  const char *allow = getenv("KMERGPU_ALLOW_K32");
+  const int kmax = (allow && allow[0] == '1') ? 32 : 31;
+  if (length(s) <= k || k > kmax || k < 1) error("the sequence should be longer than k and k should not be longer than 31");
+  const int *p = INTEGER(params_r);
+  if (p[0] != 0 && p[0] != 1) error("rc should be TRUE or FALSE");
+  if (p[1] < 0) error("max.count should be 0 (no limit) or positive");
+  if (p[2] < 0) error("min.rows should be 0 or positive");
+
+  kmg_segments *st = NULL;
+  uint64_t R = 0;
+  if (kmg_segments_begin(h->index, CHAR(s), (int64_t)length(s), k, p[0], (uint32_t)p[1], (uint32_t)p[2], &st, &R) != KMG_OK)
+    error("seq.kmer.segments failed: %s", kmg_last_error());
+  if (R > (uint64_t)INT_MAX) {
+    kmg_segments_free(st);
+    error("seq.kmer.segments would return %llu segments, more than an R matrix can hold (2^31-1)", (unsigned long long)R);
+  }
+  SEXP guard = PROTECT(R_MakeExternalPtr(st, R_NilValue, R_NilValue));
+  R_RegisterCFinalizerEx(guard, finalise_segments_guard, TRUE);
+  SEXP m = PROTECT(allocMatrix(INTSXP, 3, (int)R)); /* rows (i, j, n) */
+  const int rc = kmg_segments_emit(st, INTEGER(m));
+  kmg_segments_free(st);
+  R_ClearExternalPtr(guard);
+  UNPROTECT(2);
+  if (rc != KMG_OK) error("seq.kmer.segments failed: %s", kmg_last_error());
+  return m;
+}
+
 static const R_CallMethodDef call_methods[] = {
     {"make_kmer_h_index", (DL_FUNC)&make_kmer_h_index, 3},
     {"kmer_positions", (DL_FUNC)&kmer_positions, 2},
@@ -499,6 +545,7 @@ static const R_CallMethodDef call_methods[] = {
     {"sequence_kmer_depth", (DL_FUNC)&sequence_kmer_depth, 3},
     {"sequence_kmer_dotplot", (DL_FUNC)&sequence_kmer_dotplot, 4},
     {"kmer_pair_dotplot", (DL_FUNC)&kmer_pair_dotplot, 3},
+    {"sequence_kmer_segments", (DL_FUNC)&sequence_kmer_segments, 4},
     {NULL, NULL, 0}};
 
 void R_init_kmer_hash(DllInfo *info) { R_registerRoutines(info, NULL, call_methods, NULL, NULL); }
