@@ -179,6 +179,19 @@ int kmg_segments_begin(const kmg_index *idx, const char *q, int64_t qlen, int k,
 int kmg_segments_emit(kmg_segments *st, int32_t *out /* 3R */);
 int kmg_segments_emit_chunk(kmg_segments *st, uint64_t first, uint64_t n, int32_t *out /* 3n */);
 int kmg_segments_free(kmg_segments *st);   /* NULL accepted */
+/* kmer.pairs.segments: the runs of a join, for two indexes on one device (a == b allowed), x = 1-based position in a,
+ * y = 1-based position in b.  rc = 0: S = the rows kmg_join_begin + kmg_join_emit give (keys compared as raw 2-bit codes,
+ * whatever k each index has), runs (x+t, y+t) as above.  rc = 1: S = the rows (x, y) where b's k-mer at y is the code-space
+ * reverse complement of a's k-mer at x (codes reversed, each code ^ 2; needs one k, else KMG_ERR_K), and a run is
+ * antiparallel: rows (x+t, y-t), t = 0..n-1, all in S, (x-1, y+1) and (x+n, y-n) not in S.  max_count > 0: a k-mer with
+ * more than max_count positions in either index adds no rows (rc = 1: a's k-mer in a, its reverse complement in b).
+ * min_rows, R, the (x, y, n) triples of each run's first (smallest x) row ordered by (x, y), the handle and its emit /
+ * emit_chunk / free are those of kmg_segments_begin.  With one k, forward: a[x, x+n+k-2] equals b[y, y+n+k-2] in 2-bit
+ * code; rc = 1: a[x, x+n+k-2] is the code-space reverse complement of b[y-n+1, y+k-1] (the window rule aside).  An empty
+ * index or no shared k-mer gives R = 0.  KMG_ERR_ARG: NULL a, b or st, rc not 0/1, indexes on different devices;
+ * KMG_ERR_RANGE: more than 2^31 - 1 runs before the min_rows filter. */
+int kmg_join_segments_begin(const kmg_index *a, const kmg_index *b, int rc, uint32_t max_count,
+                            uint32_t min_rows, kmg_segments **st, uint64_t *R);
 
 /* ---- sharded build (one process per GPU; the exchange itself is the host's NCCL all-to-all) ----
  * A rank holds bytes [g0,g1) of a global sequence of length L in device memory at d_seq (d_seq[0]

@@ -21,7 +21,7 @@ from . import _lib
 from ._lib import KmgError, check
 
 __all__ = ["KmerHash", "KmerCounts", "SequenceFile", "make_kmer_hash_file", "count_kmers_file", "make_kmer_hash", "kmer_pos", "seq_kmer_pos", "kmer_pairs", "count_kmers", "kmer_spectrum",
-           "seq_kmer_depth", "seq_kmer_dotplot", "kmer_pairs_dotplot", "seq_kmer_segments", "pinned_empty", "KmgError",
+           "seq_kmer_depth", "seq_kmer_dotplot", "kmer_pairs_dotplot", "seq_kmer_segments", "kmer_pairs_segments", "pinned_empty", "KmgError",
            "OPT_KMER", "OPT_POS", "OPT_PAIRS", "OPT_COUNT", "NA_INTEGER"]
 
 # opt.flag bits, src/kmer_hash.c:17 (pos_opt_flags) in the reference
@@ -645,15 +645,43 @@ def seq_kmer_segments(ptr, seq, k, *, reverse_complement=False, max_count=0, min
     p, n, keep = _seq_buffer(seq)
     if n <= k or k > (32 if allow_k32 else 31):
         raise ValueError("the sequence should be longer than k and k should not be longer than 31")
+    max_count, min_rows = _segments_limits(max_count, min_rows)
+    st, R = C.c_void_p(), C.c_uint64()
+    check(_L.kmg_segments_begin(ix._handle(), p, n, k, int(bool(reverse_complement)), max_count, min_rows,
+                                C.byref(st), C.byref(R)))
+    del keep
+    return _segments_emit(st, R, out)
+
+
+def kmer_pairs_segments(ptr_a, ptr_b, *, reverse_complement=False, max_count=0, min_rows=1, out=None):
+    """kmer.pairs.segments (additive; the R closure is in INTEGRATION.md): the rows kmer_pairs(ptr_a, ptr_b) would return,
+    joined on the device into match segments -- maximal diagonal runs of rows (x + t, y + t), t = 0 .. n - 1, x = 1-based
+    position in ptr_a, y = in ptr_b.  Every row belongs to exactly one run.
+
+    reverse_complement=True joins each k-mer of ptr_a with its code-space reverse complement in ptr_b (both indexes must
+    have the same k) and the runs are antiparallel: rows (x + t, y - t).  Returns an (R, 3) int32 array of (x, y, n), the
+    run's first row (its smallest x) and its row count, ordered by (x, y).  With one k, a forward run covers a[x, x+n+k-2]
+    = b[y, y+n+k-2]; an antiparallel one a[x, x+n+k-2] = reverse complement of b[y-n+1, y+k-1].  max_count > 0 drops the
+    k-mers with more positions in either index; min_rows and `out` as in seq_kmer_segments."""
+    a, b = _extract_index(ptr_a), _extract_index(ptr_b)
+    max_count, min_rows = _segments_limits(max_count, min_rows)
+    st, R = C.c_void_p(), C.c_uint64()
+    check(_L.kmg_join_segments_begin(a._handle(), b._handle(), int(bool(reverse_complement)), max_count, min_rows,
+                                     C.byref(st), C.byref(R)))
+    return _segments_emit(st, R, out)
+
+
+def _segments_limits(max_count, min_rows):
     max_count, min_rows = int(max_count), int(min_rows)
     if not 0 <= max_count < 2**32:
         raise ValueError("max_count must be 0 (no limit) or a positive 32-bit count")
     if not 0 <= min_rows < 2**32:
         raise ValueError("min_rows must be a non-negative 32-bit count")
-    st, R = C.c_void_p(), C.c_uint64()
-    check(_L.kmg_segments_begin(ix._handle(), p, n, k, int(bool(reverse_complement)), max_count, min_rows,
-                                C.byref(st), C.byref(R)))
-    del keep
+    return max_count, min_rows
+
+
+def _segments_emit(st, R, out):
+    """The R runs of the segments handle st into `out` (allocated when None); st is freed."""
     try:
         R = R.value
         if R > INT_MAX:

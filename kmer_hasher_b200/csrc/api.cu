@@ -1770,6 +1770,7 @@ static int seg_grow(T *&p, uint64_t keep, uint64_t cap, cudaStream_t s) {
 }
 
 // Run starts (i, j) and run ends (diagonal key, i) of the probe st, each in row order, into arrays of at least R0 entries.
+template <bool ANTI>
 static int segments_mark(const kmg_query *st, const uint32_t *pos, int2 *&starts, uint64_t *&ekey, uint32_t *&ei, uint64_t *R0) {
   cudaStream_t s = g_ctx.stream();
   const uint64_t M = st->M;
@@ -1792,7 +1793,7 @@ static int segments_mark(const kmg_query *st, const uint32_t *pos, int2 *&starts
       CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
       CU(cudaMemsetAsync(ticket, 0, 4, s));
       TRY(block_starts(st->row_off, st->H, first, n, s, blk));
-      LAUNCH("segments_mark", s, segments_mark_kernel<EMIT_THREADS><<<(unsigned)tiles, EMIT_THREADS, 0, s>>>(
+      LAUNCH("segments_mark", s, segments_mark_kernel<EMIT_THREADS, ANTI><<<(unsigned)tiles, EMIT_THREADS, 0, s>>>(
                                      st->hit_i, st->hit_start, st->row_off, st->H, M, pos, first, n, blk, status, ticket, bs, be,
                                      cap, starts, ekey, ei, tot));
       uint64_t h[2];
@@ -1824,15 +1825,13 @@ static int segments_mark(const kmg_query *st, const uint32_t *pos, int2 *&starts
   return rc;
 }
 
-// The runs of the probe (idx, q, qlen, k, rc, max_count) with at least min_rows rows, as (i, j, n) triples in the order
-// of their first rows: *rows (device, 12 * *R bytes) or nullptr when *R = 0.
-static int segments_run(const kmg_index *ix, const char *q, int64_t qlen, int k, int rc, uint32_t max_count, uint32_t min_rows,
-                        int32_t **rows, uint64_t *R) {
+// The runs of the probe st (freed here, on every path) with at least min_rows rows, as (i, j, n) triples in the order of
+// their first rows: *rows (device, 12 * *R bytes) or nullptr when *R = 0.  ANTI: antiparallel runs (segments.cuh).
+template <bool ANTI>
+static int segments_of(kmg_query *st, uint32_t min_rows, int32_t **rows, uint64_t *R) {
   *rows = nullptr;
   *R = 0;
-  kmg_query *st = nullptr;
-  uint64_t M = 0;
-  TRY(query_seq(ix, q, qlen, k, rc == 1, max_count ? max_count : UINT32_MAX, &st, &M));
+  const uint64_t M = st->M;
   if (M == 0) { kmg_query_free(st); return KMG_OK; }
   cudaStream_t s = g_ctx.stream();
   int2 *starts = nullptr;
@@ -1843,11 +1842,11 @@ static int segments_run(const kmg_index *ix, const char *q, int64_t qlen, int k,
   kmg_index *ends = nullptr;
   uint64_t R0 = 0;
   auto body = [&]() -> int {
-    const int m = segments_mark(st, ix->pos, starts, ekey, ei, &R0);
+    const int m = segments_mark<ANTI>(st, st->idx->pos, starts, ekey, ei, &R0);
     kmg_query_free(st);                                   // the probe is done with: only the runs stay
     st = nullptr;
     TRY(m);
-    // the ends sorted by diagonal, i ascending inside one: keys d + 2^31 < 2^32 are the 32 bits of a 16-mer
+    // the ends sorted by diagonal, i ascending inside one: keys below 2^32 (segment_key) are the 32 bits of a 16-mer
     TRY(kmg_build_records(ekey, ei, (int64_t)R0, 16, &ends));
     dfree(ekey, s); dfree(ei, s);
     const uint64_t tiles = ceil_div<uint64_t>(R0, SEG_PAIR_TILE);
@@ -1857,7 +1856,7 @@ static int segments_run(const kmg_index *ix, const char *q, int64_t qlen, int k,
     TRY(dalloc(&tot, 2, s));
     CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
     CU(cudaMemsetAsync(ticket, 0, 4, s));
-    LAUNCH("segments_pair", s, segments_pair_kernel<256, SEG_PAIR_ITEMS><<<(unsigned)tiles, 256, 0, s>>>(
+    LAUNCH("segments_pair", s, segments_pair_kernel<256, SEG_PAIR_ITEMS, ANTI><<<(unsigned)tiles, 256, 0, s>>>(
                                    starts, R0, ends->ukeys, ends->U, ends->ustart, ends->pos, min_rows, status, ticket, tmp, tot));
     uint64_t h[2];
     CU(cudaMemcpyAsync(h, tot, sizeof h, cudaMemcpyDeviceToHost, s));
@@ -1884,6 +1883,110 @@ static int segments_run(const kmg_index *ix, const char *q, int64_t qlen, int k,
   return KMG_OK;
 }
 
+// The runs of the probe (idx, q, qlen, k, rc, max_count), as segments_of
+static int segments_run(const kmg_index *ix, const char *q, int64_t qlen, int k, int rc, uint32_t max_count, uint32_t min_rows,
+                        int32_t **rows, uint64_t *R) {
+  *rows = nullptr;
+  *R = 0;
+  kmg_query *st = nullptr;
+  uint64_t M = 0;
+  TRY(query_seq(ix, q, qlen, k, rc == 1, max_count ? max_count : UINT32_MAX, &st, &M));
+  return segments_of<false>(st, min_rows, rows, R);
+}
+
+// kmer.pairs(a, b) as a probe of b (probe.cuh, "kmer.pairs.segments"): the hits are a's positions x, ascending, whose k-mer
+// b holds (rc: whose code-space reverse complement b holds), each with b's position list of it, so the rows come out in
+// (x, y) order.  max_count: a k-mer with more positions in a, or whose match has more in b, gives no hit.
+static int join_probe(const kmg_index *a, const kmg_index *cb, bool rc, uint32_t max_count, kmg_query **out) {
+  *out = nullptr;
+  kmg_index *b = const_cast<kmg_index *>(cb);
+  cudaStream_t s = g_ctx.stream();
+  kmg_query *q = new (std::nothrow) kmg_query();
+  if (!q) return fail(KMG_ERR_NOMEM, "host allocation failed");
+  q->idx = b;
+  if (a->U == 0 || b->U == 0) { *out = q; return KMG_OK; }
+  int rv = ensure_hash(b);
+  if (rv != KMG_OK) { delete q; return rv; }
+  const uint64_t U = a->U, N = a->N;
+  uint64_t *rkeys = nullptr, *blk = nullptr;
+  uint2 *found = nullptr, *found_pos = nullptr;
+  uint32_t *d_last = nullptr, *ticket = nullptr;
+  QueryStats *qs = nullptr;
+  Pair64 *status = nullptr;
+  uint32_t X = 0;                                         // a's largest position: found_pos has one entry per x in [1, X]
+  auto body = [&]() -> int {
+    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(U, 256), (uint64_t)g_ctx.sms * 16);
+    TRY(dalloc(&d_last, 1, s));
+    CU(cudaMemsetAsync(d_last, 0, 4, s));
+    LAUNCH("last_pos", s, last_pos_kernel<<<grid, 256, 0, s>>>(a->ustart, a->pos, U, d_last));
+    CU(cudaMemcpyAsync(&X, d_last, 4, cudaMemcpyDeviceToHost, s));
+    const uint64_t *keys = a->ukeys;
+    if (rc) {
+      TRY(dalloc(&rkeys, (size_t)U, s));
+      LAUNCH("revcomp_keys", s, revcomp_keys_kernel<<<grid, 256, 0, s>>>(a->ukeys, U, a->k, rkeys));
+      keys = rkeys;
+    }
+    TRY(dalloc(&found, (size_t)U, s));
+    const KeyHash kt{b->hash, b->hash_nb, b->hash_hbits};
+    const SeqView sv{};
+    LAUNCH("probe_lookup_rec", s, probe_lookup_kernel<PROBE_THREADS, PROBE_ITEMS, false><<<(unsigned)ceil_div<uint64_t>(U, PROBE_TILE), PROBE_THREADS, 0, s>>>(
+                                      sv, keys, (int64_t)U, nullptr, kt, found));
+    CU(cudaStreamSynchronize(s));
+    dfree(rkeys, s);
+    TRY(dalloc(&found_pos, (size_t)X, s));
+    CU(cudaMemsetAsync(found_pos, 0, (size_t)X * sizeof(uint2), s));
+    TRY(dalloc(&blk, (size_t)ceil_div<uint64_t>(std::min(N, SEG_SLICE_ROWS), EMIT_TILE), s));
+    for (uint64_t first = 0; first < N; first += SEG_SLICE_ROWS) {
+      const uint64_t n = std::min(SEG_SLICE_ROWS, N - first);
+      TRY(block_starts(a->ustart, U, first, n, s, blk));
+      LAUNCH("join_scatter", s, join_scatter_kernel<EMIT_THREADS><<<(unsigned)ceil_div<uint64_t>(n, EMIT_TILE), EMIT_THREADS, 0, s>>>(
+                                    a->ustart, U, a->pos, found, max_count, first, n, blk, found_pos));
+    }
+    const uint64_t tiles = ceil_div<uint64_t>(X, COMPACT_TILE);
+    TRY(dalloc(&q->hit_i, (size_t)X, s));
+    TRY(dalloc(&q->hit_start, (size_t)X, s));
+    TRY(dalloc(&q->row_off, (size_t)X, s));
+    TRY(dalloc(&qs, 1, s));
+    TRY(dalloc(&status, (size_t)tiles, s));
+    TRY(dalloc(&ticket, 1, s));
+    CU(cudaMemsetAsync(qs, 0, sizeof(QueryStats), s));
+    CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
+    CU(cudaMemsetAsync(ticket, 0, 4, s));
+    LAUNCH("probe_compact", s, probe_compact_kernel<PROBE_THREADS, COMPACT_ITEMS, true><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
+                                   found_pos, 1, nullptr, (int64_t)X, nullptr, q->hit_i, q->hit_start, q->row_off, qs, status, ticket,
+                                   max_count));
+    QueryStats h;
+    CU(cudaMemcpyAsync(&h, qs, sizeof h, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    q->H = h.H; q->M = h.M;
+    return KMG_OK;
+  };
+  rv = body();
+  cudaStreamSynchronize(s);
+  dfree(d_last, s); dfree(rkeys, s); dfree(found, s); dfree(blk, s); dfree(found_pos, s);
+  dfree(qs, s); dfree(status, s); dfree(ticket, s);
+  if (rv != KMG_OK) { kmg_query_free(q); return rv; }
+  prof_bytes("last_pos", 8.0 * U);
+  if (rc) prof_bytes("revcomp_keys", 16.0 * U);
+  prof_bytes("probe_lookup_rec", 8.0 * U + 128.0 * U + 8.0 * U);
+  // per position: its k-mer's found entry and list bounds (read once per k-mer), the position, one 8-byte write (a
+  // 32-byte sector of DRAM when it scatters) for a shared k-mer; the memset of found_pos
+  prof_bytes("join_scatter", 16.0 * U + 4.0 * N + 32.0 * (double)q->H + 8.0 * X);
+  prof_bytes("probe_compact", 8.0 * X + 16.0 * q->H);
+  *out = q;
+  return KMG_OK;
+}
+
+// The runs of the rows of kmer.pairs(a, b) (rc: of a's k-mers reverse-complemented, antiparallel runs), as segments_of
+static int join_segments_run(const kmg_index *a, const kmg_index *b, int rc, uint32_t max_count, uint32_t min_rows,
+                             int32_t **rows, uint64_t *R) {
+  *rows = nullptr;
+  *R = 0;
+  kmg_query *st = nullptr;
+  TRY(join_probe(a, b, rc == 1, max_count ? max_count : UINT32_MAX, &st));
+  return rc ? segments_of<true>(st, min_rows, rows, R) : segments_of<false>(st, min_rows, rows, R);
+}
+
 extern "C" int kmg_segments_begin(const kmg_index *ix, const char *q, int64_t qlen, int k, int rc, uint32_t max_count,
                                   uint32_t min_rows, kmg_segments **st, uint64_t *R) {
   if (!st) return fail(KMG_ERR_ARG, "st is NULL");
@@ -1895,6 +1998,26 @@ extern "C" int kmg_segments_begin(const kmg_index *ix, const char *q, int64_t ql
   g->device = ix->device;
   int rv = segments_run(ix, q, qlen, k, rc, max_count, min_rows, &g->rows, &g->R);
   if (rv == KMG_ERR_UNSTABLE) rv = segments_run(ix, q, qlen, k, rc, max_count, min_rows, &g->rows, &g->R);   // the sort now ranks by bitmap
+  if (rv != KMG_OK) { delete g; return rv; }
+  *st = g;
+  if (R) *R = g->R;
+  return KMG_OK;
+}
+
+extern "C" int kmg_join_segments_begin(const kmg_index *a, const kmg_index *b, int rc, uint32_t max_count, uint32_t min_rows,
+                                       kmg_segments **st, uint64_t *R) {
+  if (!st) return fail(KMG_ERR_ARG, "st is NULL");
+  *st = nullptr;
+  if (!a || !b) return fail(KMG_ERR_ARG, "index is NULL");
+  if (rc != 0 && rc != 1) return fail(KMG_ERR_ARG, "rc must be 0 or 1");
+  if (a->device != b->device) return fail(KMG_ERR_ARG, "the two indexes live on different devices (%d, %d)", a->device, b->device);
+  if (rc && a->k != b->k) return fail(KMG_ERR_K, "the reverse complement needs indexes of one k (here %d and %d)", a->k, b->k);
+  TRY(use_index(a));
+  kmg_segments *g = new (std::nothrow) kmg_segments();
+  if (!g) return fail(KMG_ERR_NOMEM, "host allocation failed");
+  g->device = a->device;
+  int rv = join_segments_run(a, b, rc, max_count, min_rows, &g->rows, &g->R);
+  if (rv == KMG_ERR_UNSTABLE) rv = join_segments_run(a, b, rc, max_count, min_rows, &g->rows, &g->R);   // the sort now ranks by bitmap
   if (rv != KMG_OK) { delete g; return rv; }
   *st = g;
   if (R) *R = g->R;

@@ -576,6 +576,53 @@ join_emit_kernel(const uint32_t *__restrict__ hit_astart, const uint32_t *__rest
   }
 }
 
+// ---- kmer.pairs.segments: a join laid out as a probe of b in a's position order ----------------------------------------
+// probe_lookup_kernel looks a's distinct keys up in b's table (found[u] = b's (start, count) of k-mer u); join_scatter_kernel
+// spreads them over a's positions (found_pos[x - 1]) and probe_compact_kernel<.., true> with coord0 = 1 compacts those into
+// hits x ascending, each with b's list: the probe shape segments_mark_kernel walks.
+
+// a's keys in code-space reverse complement (revcomp_key), for the antiparallel join
+__global__ void revcomp_keys_kernel(const uint64_t *__restrict__ in, uint64_t U, int k, uint64_t *__restrict__ out) {
+  for (uint64_t u = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; u < U; u += (uint64_t)gridDim.x * blockDim.x)
+    out[u] = revcomp_key(ld_stream_u64(in + u), k);
+}
+
+// *out = max(*out, a's largest position): lists ascend, so that is the largest last entry of a list (U reads, not N)
+__global__ void last_pos_kernel(const uint32_t *__restrict__ ustart, const uint32_t *__restrict__ pos, uint64_t U, uint32_t *out) {
+  uint32_t m = 0;
+  for (uint64_t u = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; u < U; u += (uint64_t)gridDim.x * blockDim.x)
+    m = max(m, __ldg(pos + __ldg(ustart + u + 1) - 1));
+  m = __reduce_max_sync(FULL, m);
+  if (lane_id() == 0 && m) atomicMax(out, m);
+}
+
+// Rows [first, first + nrows) of a's position lists, balanced by rows as positions_kernel (a list may hold thousands of
+// positions): position x of k-mer u gets found_pos[x - 1] = found[u] if b holds the k-mer and a's list has at most
+// max_count positions.  k-mers have disjoint positions, so no entry is written twice; found_pos starts zeroed (misses).
+template <int THREADS>
+__global__ void __launch_bounds__(THREADS)
+join_scatter_kernel(const uint32_t *__restrict__ ustart, uint64_t U, const uint32_t *__restrict__ pos,
+                    const uint2 *__restrict__ found, uint32_t max_count, uint64_t first, uint64_t nrows,
+                    const uint64_t *__restrict__ blk_first, uint2 *__restrict__ found_pos) {
+  constexpr int PER = 8, T = THREADS * PER;
+  __shared__ __align__(16) uint8_t s_flag[T];
+  __shared__ __align__(16) uint32_t s_seg[T];
+  __shared__ uint32_t s_warp[THREADS / 32];
+  __shared__ uint64_t s_first;
+  const uint64_t b0 = (uint64_t)blockIdx.x * T;
+  if (b0 >= nrows) return;
+  const uint64_t r0 = first + b0;
+  const uint64_t u0 = block_segments<THREADS, PER, uint32_t>(ustart, U, r0, blk_first[blockIdx.x], s_flag, s_seg, s_warp, &s_first);
+#pragma unroll
+  for (int j = 0; j < PER; ++j) {
+    const uint32_t s = j * THREADS + threadIdx.x;
+    if (b0 + s >= nrows) continue;
+    const uint64_t u = u0 + s_seg[s];
+    const uint2 f = __ldg(found + u);
+    if (f.y != 0 && __ldg(ustart + u + 1) - __ldg(ustart + u) <= max_count) found_pos[ld_stream_u32(pos + r0 + s) - 1] = f;
+  }
+}
+
 // ---- dot plots: the rows of a probe or a join counted into an nx x ny image -----------------------------------------
 // One axis of the image: a coordinate v is in the window iff 0 <= v - lo < range, and goes to bin floor((v - lo) * n / range).
 // (v - lo) * n < 2^31 * 2^31, so the quotient is exact from the host's inv = floor((2^64 - 1) / range): umulhi(p, inv) is

@@ -6,6 +6,9 @@
 // rows that start a run and the rows that end one and compacts both in row order; the ends are then sorted by diagonal
 // (kmg_build_records, stable, so i ascends inside a diagonal) and segments_pair_kernel pairs each start with the first end
 // of its diagonal at or after it: runs of one diagonal do not overlap, so its k-th start and k-th end belong together.
+// ANTI (kmer.pairs.segments with the reverse complement): runs are antiparallel, rows (i + t, j - t); the row (i, j)
+// continues one from (i - 1, j + 1) and into (i + 1, j - 1), and a run's anti-diagonal is i + j.  The rows of a hit
+// still ascend in j, so the starts still come out in (i, j) order.
 #pragma once
 #include "common.cuh"
 #include "csr.cuh"
@@ -30,11 +33,17 @@ __device__ __forceinline__ bool sorted_has(const uint32_t *__restrict__ p, uint3
   return lo < n && __ldg(p + lo) == v;
 }
 
+// The key of the diagonal (i - j + 2^31) or, with ANTI, of the anti-diagonal (i + j) of the row (i, j): below 2^32 either way.
+template <bool ANTI>
+__device__ __forceinline__ uint64_t segment_key(int64_t i, int64_t j) {
+  return (uint64_t)(ANTI ? i + j : i - j + (int64_t(1) << 31));
+}
+
 // Rows [first, first + nrows) of a probe (hits hit_i / hit_start / row_off[0, H), M rows in all), balanced by rows like
-// probe_emit_kernel.  Writes the run starts as (i, j) and the run ends as (key = i - j + 2^31, i), each in row order, from
+// probe_emit_kernel.  Writes the run starts as (i, j) and the run ends as (segment_key(i, j), i), each in row order, from
 // the bases (base_s, base_e) on; entries at or past `cap` are counted but not written.  tot: (starts, ends) of the slice.
 // Tiles take their number from `ticket` so that the chained scan of their counts (pair_lookback) cannot deadlock.
-template <int THREADS>
+template <int THREADS, bool ANTI>
 __global__ void __launch_bounds__(THREADS)
 segments_mark_kernel(const int32_t *__restrict__ hit_i, const uint32_t *__restrict__ hit_start, const uint64_t *__restrict__ row_off,
                      uint64_t H, uint64_t M, const uint32_t *__restrict__ pos, uint64_t first, uint64_t nrows,
@@ -72,15 +81,28 @@ segments_mark_kernel(const int32_t *__restrict__ hit_i, const uint32_t *__restri
       const uint32_t hs = hit_start[h];
       const uint32_t j = pos[hs + within];
       bool pred = false, succ = false;
-      if (h > 0 && hit_i[h - 1] == i - 1 && j > 0) {
-        const uint32_t ps = hit_start[h - 1];
-        if (ps == hs) pred = within > 0 && pos[hs + within - 1] == j - 1;     // the same list: j - 1 would sit just before j
-        else pred = sorted_has(pos + ps, (uint32_t)(o - row_off[h - 1]), j - 1, (uint32_t)within);
-      }
-      if (h + 1 < H && hit_i[h + 1] == i + 1) {
-        const uint32_t ns = hit_start[h + 1];
-        if (ns == hs) succ = within + 1 < o1 - o && pos[hs + within + 1] == j + 1;
-        else succ = sorted_has(pos + ns, (uint32_t)((h + 2 < H ? row_off[h + 2] : M) - o1), j + 1, (uint32_t)within);
+      if constexpr (!ANTI) {
+        if (h > 0 && hit_i[h - 1] == i - 1 && j > 0) {
+          const uint32_t ps = hit_start[h - 1];
+          if (ps == hs) pred = within > 0 && pos[hs + within - 1] == j - 1;     // the same list: j - 1 would sit just before j
+          else pred = sorted_has(pos + ps, (uint32_t)(o - row_off[h - 1]), j - 1, (uint32_t)within);
+        }
+        if (h + 1 < H && hit_i[h + 1] == i + 1) {
+          const uint32_t ns = hit_start[h + 1];
+          if (ns == hs) succ = within + 1 < o1 - o && pos[hs + within + 1] == j + 1;
+          else succ = sorted_has(pos + ns, (uint32_t)((h + 2 < H ? row_off[h + 2] : M) - o1), j + 1, (uint32_t)within);
+        }
+      } else {                                            // (i - 1, j + 1) and (i + 1, j - 1); positions are >= 1
+        if (h > 0 && hit_i[h - 1] == i - 1) {
+          const uint32_t ps = hit_start[h - 1];
+          if (ps == hs) pred = within + 1 < o1 - o && pos[hs + within + 1] == j + 1;
+          else pred = sorted_has(pos + ps, (uint32_t)(o - row_off[h - 1]), j + 1, (uint32_t)within);
+        }
+        if (h + 1 < H && hit_i[h + 1] == i + 1) {
+          const uint32_t ns = hit_start[h + 1];
+          if (ns == hs) succ = within > 0 && pos[hs + within - 1] == j - 1;
+          else succ = sorted_has(pos + ns, (uint32_t)((h + 2 < H ? row_off[h + 2] : M) - o1), j - 1, (uint32_t)within);
+        }
       }
       st = !pred; en = !succ;
       vi[r] = i; vj[r] = j;
@@ -115,18 +137,19 @@ segments_mark_kernel(const int32_t *__restrict__ hit_i, const uint32_t *__restri
     if (me[r] >> lane & 1u) {
       const uint64_t at = be + s_ce[r * WARPS + warp] + __popc(me[r] & lt);
       if (at < cap) {
-        end_key[at] = (uint64_t)((int64_t)vi[r] - (int64_t)vj[r] + (int64_t(1) << 31));
+        end_key[at] = segment_key<ANTI>(vi[r], (int64_t)vj[r]);
         end_i[at] = (uint32_t)vi[r];
       }
     }
   }
 }
 
-// Pair the starts [0, R0) with the ends sorted by diagonal (dkeys[0, U) ascending, the ends' i in ei[dstart[u],
-// dstart[u+1]) ascending): n = (first end i >= i on the start's diagonal) - i + 1.  The runs with n >= min_rows go to
-// out as (i, j, n) triples in the starts' order (a chained scan, tiles numbered by `ticket`).  tot: (runs kept, sum of
-// n over all runs); a start without an end adds 0 to the sum, which the host checks against the probe's row count.
-template <int THREADS, int ITEMS>
+// Pair the starts [0, R0) with the ends sorted by diagonal, or anti-diagonal with ANTI (dkeys[0, U) ascending, the ends'
+// i in ei[dstart[u], dstart[u+1]) ascending): n = (first end i >= i on the start's diagonal) - i + 1.  The runs with
+// n >= min_rows go to out as (i, j, n) triples in the starts' order (a chained scan, tiles numbered by `ticket`).
+// tot: (runs kept, sum of n over all runs); a start without an end adds 0 to the sum, which the host checks against the
+// probe's row count.
+template <int THREADS, int ITEMS, bool ANTI>
 __global__ void __launch_bounds__(THREADS)
 segments_pair_kernel(const int2 *__restrict__ starts, uint64_t R0, const uint64_t *__restrict__ dkeys, uint64_t U,
                      const uint32_t *__restrict__ dstart, const uint32_t *__restrict__ ei, uint32_t min_rows, Pair64 *status,
@@ -151,7 +174,7 @@ segments_pair_kernel(const int2 *__restrict__ starts, uint64_t R0, const uint64_
     v[t] = make_int2(0, 0);
     if (t0 + t >= R0) continue;
     v[t] = starts[t0 + t];
-    const uint64_t key = (uint64_t)((int64_t)v[t].x - (int64_t)v[t].y + (int64_t(1) << 31));
+    const uint64_t key = segment_key<ANTI>(v[t].x, v[t].y);
     uint64_t lo = 0, len = U;                             // the diagonal: lower bound of key in dkeys
     while (len > 0) {
       const uint64_t half = len >> 1;

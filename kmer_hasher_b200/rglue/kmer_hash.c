@@ -16,6 +16,8 @@
  *                                           additive: binned dot plots of seq.kmer.pos / kmer.pairs rows
  *   sequence_kmer_segments(ptr, seq, k, params)
  *                                           additive: match segments, the diagonal runs of seq.kmer.pos rows
+ *   kmer_pair_segments(ptr.a, ptr.b, params)
+ *                                           additive: match segments of kmer.pairs rows, on either strand
  *   R_init_kmer_hash                        replaces src/kmer_hash.c:1221-1224
  *
  * Differences a user can observe: k-mers come out in the order of a mix of their 2-bit key (ascending key
@@ -500,28 +502,21 @@ static void finalise_segments_guard(SEXP g) {
   R_ClearExternalPtr(g);
 }
 
-SEXP sequence_kmer_segments(SEXP ptr_r, SEXP seq_r, SEXP k_r, SEXP params_r) {
-  kmer_handle *h = index_handle_or_error(ptr_r);
-  if (TYPEOF(seq_r) != STRSXP || length(seq_r) != 1) error("seq_r should be a single sequence");
-  if (TYPEOF(k_r) != INTSXP || length(k_r) != 1) error("k should be an integer of length 1");
+/* params = as.integer(c(rc, max.count, min.rows)), checked */
+static const int *segments_params(SEXP params_r) {
   if (TYPEOF(params_r) != INTSXP || length(params_r) != 3) error("params should be an integer vector of length 3");
-  const int k = INTEGER(k_r)[0];
-  SEXP s = STRING_ELT(seq_r, 0);
-  const char *allow = getenv("KMERGPU_ALLOW_K32");
-  const int kmax = (allow && allow[0] == '1') ? 32 : 31;
-  if (length(s) <= k || k > kmax || k < 1) error("the sequence should be longer than k and k should not be longer than 31");
   const int *p = INTEGER(params_r);
   if (p[0] != 0 && p[0] != 1) error("rc should be TRUE or FALSE");
   if (p[1] < 0) error("max.count should be 0 (no limit) or positive");
   if (p[2] < 0) error("min.rows should be 0 or positive");
+  return p;
+}
 
-  kmg_segments *st = NULL;
-  uint64_t R = 0;
-  if (kmg_segments_begin(h->index, CHAR(s), (int64_t)length(s), k, p[0], (uint32_t)p[1], (uint32_t)p[2], &st, &R) != KMG_OK)
-    error("seq.kmer.segments failed: %s", kmg_last_error());
+/* The R runs of st as a 3 x R INTSXP matrix; st is freed on every path (a guard frees it if the allocation fails). */
+static SEXP segments_matrix(kmg_segments *st, uint64_t R, const char *what) {
   if (R > (uint64_t)INT_MAX) {
     kmg_segments_free(st);
-    error("seq.kmer.segments would return %llu segments, more than an R matrix can hold (2^31-1)", (unsigned long long)R);
+    error("%s would return %llu segments, more than an R matrix can hold (2^31-1)", what, (unsigned long long)R);
   }
   SEXP guard = PROTECT(R_MakeExternalPtr(st, R_NilValue, R_NilValue));
   R_RegisterCFinalizerEx(guard, finalise_segments_guard, TRUE);
@@ -530,8 +525,41 @@ SEXP sequence_kmer_segments(SEXP ptr_r, SEXP seq_r, SEXP k_r, SEXP params_r) {
   kmg_segments_free(st);
   R_ClearExternalPtr(guard);
   UNPROTECT(2);
-  if (rc != KMG_OK) error("seq.kmer.segments failed: %s", kmg_last_error());
+  if (rc != KMG_OK) error("%s failed: %s", what, kmg_last_error());
   return m;
+}
+
+SEXP sequence_kmer_segments(SEXP ptr_r, SEXP seq_r, SEXP k_r, SEXP params_r) {
+  kmer_handle *h = index_handle_or_error(ptr_r);
+  if (TYPEOF(seq_r) != STRSXP || length(seq_r) != 1) error("seq_r should be a single sequence");
+  if (TYPEOF(k_r) != INTSXP || length(k_r) != 1) error("k should be an integer of length 1");
+  const int k = INTEGER(k_r)[0];
+  SEXP s = STRING_ELT(seq_r, 0);
+  const char *allow = getenv("KMERGPU_ALLOW_K32");
+  const int kmax = (allow && allow[0] == '1') ? 32 : 31;
+  if (TYPEOF(params_r) != INTSXP || length(params_r) != 3) error("params should be an integer vector of length 3");
+  if (length(s) <= k || k > kmax || k < 1) error("the sequence should be longer than k and k should not be longer than 31");
+  const int *p = segments_params(params_r);
+  kmg_segments *st = NULL;
+  uint64_t R = 0;
+  if (kmg_segments_begin(h->index, CHAR(s), (int64_t)length(s), k, p[0], (uint32_t)p[1], (uint32_t)p[2], &st, &R) != KMG_OK)
+    error("seq.kmer.segments failed: %s", kmg_last_error());
+  return segments_matrix(st, R, "seq.kmer.segments");
+}
+
+/* kmer.pairs.segments (additive; INTEGRATION.md): the rows kmer.pairs would return (rc: of a's k-mers joined with their
+ * reverse complements in b, needing one k), joined on the device into maximal runs -- (x+t, y+t), or antiparallel
+ * (x+t, y-t) with rc -- as a 3 x R integer matrix of (x, y, n) ordered by (x, y); kmer.pairs.segments() names and
+ * transposes.  params = as.integer(c(rc, max.count, min.rows)), as for seq.kmer.segments (max.count: in either index). */
+SEXP kmer_pair_segments(SEXP ptr_a, SEXP ptr_b, SEXP params_r) {
+  kmer_handle *a = index_handle_or_error(ptr_a);
+  kmer_handle *b = index_handle_or_error(ptr_b);
+  const int *p = segments_params(params_r);
+  kmg_segments *st = NULL;
+  uint64_t R = 0;
+  if (kmg_join_segments_begin(a->index, b->index, p[0], (uint32_t)p[1], (uint32_t)p[2], &st, &R) != KMG_OK)
+    error("kmer.pairs.segments failed: %s", kmg_last_error());
+  return segments_matrix(st, R, "kmer.pairs.segments");
 }
 
 static const R_CallMethodDef call_methods[] = {
@@ -546,6 +574,7 @@ static const R_CallMethodDef call_methods[] = {
     {"sequence_kmer_dotplot", (DL_FUNC)&sequence_kmer_dotplot, 4},
     {"kmer_pair_dotplot", (DL_FUNC)&kmer_pair_dotplot, 3},
     {"sequence_kmer_segments", (DL_FUNC)&sequence_kmer_segments, 4},
+    {"kmer_pair_segments", (DL_FUNC)&kmer_pair_segments, 3},
     {NULL, NULL, 0}};
 
 void R_init_kmer_hash(DllInfo *info) { R_registerRoutines(info, NULL, call_methods, NULL, NULL); }
