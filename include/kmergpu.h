@@ -193,6 +193,33 @@ int kmg_segments_free(kmg_segments *st);   /* NULL accepted */
 int kmg_join_segments_begin(const kmg_index *a, const kmg_index *b, int rc, uint32_t max_count,
                             uint32_t min_rows, kmg_segments **st, uint64_t *R);
 
+/* ---- chains: match segments joined across mismatches and short indels, found on the device (additive) ---------------
+ * Input: the R runs a kmg_segments handle holds (after its own max_count and min_rows).  A run s = (i, j, n) has its first
+ * row (i, j) and its last row (I, J) = (i+n-1, j+n-1), or (i+n-1, j-n+1) for antiparallel runs (kmg_join_segments_begin
+ * with rc = 1).  For an ordered pair (s, t): gq = i_t - I_s - 1, gr = j_t - J_s - 1 (antiparallel: J_s - j_t - 1); gq - gr
+ * is the difference of the two runs' diagonal keys (i - j, or i + j antiparallel).  t may follow s iff 0 <= gq <= G,
+ * 0 <= gr <= G and |gq - gr| <= W (G = max_gap, W = max_shift): runs that overlap in either coordinate never follow one
+ * another.  The cost c(s, t) = (max(gq, gr), |gq - gr|, gq) is compared lexicographically; succ(s) is the t of least cost
+ * that may follow s, pred(t) the s of least cost that t may follow (both unique when they exist).  s -> t is a link iff
+ * succ(s) = t and pred(t) = s, and a chain is a maximal path of links (a run without one is a chain of one).  Per chain:
+ * (i, j) = first row of its first run, (I, J) = last row of its last run, n = the sum of its runs' n, m = its number of
+ * runs; interleaved int32 (i, j, I, J, n, m), column-major 6 x C, ordered by (i, j), only chains with n >= min_rows (0 and
+ * 1 keep all).  Before that filter the m sum to R and the n to the runs' n.  G = 0 gives the runs themselves (m = 1).  An
+ * isolated substitution leaves gq = gr = k on one diagonal, a 1-base indel (k, k-1) or (k-1, k), so G >= k bridges
+ * isolated differences and W is the longest indel bridged.  Bases covered, for one k: seq.kmer.segments query
+ * [i-k+1, I], index [j, J+k-1]; a forward join a [i, I+k-1], b [j, J+k-1]; an antiparallel join a [i, I+k-1], b [J, j+k-1].
+ * kmg_chains_begin leaves seg unchanged (it can still be emitted, and is freed by its owner); the chains handle holds
+ * only the 24 C bytes of the result; emit / emit_chunk write to device, pinned or pageable memory like
+ * kmg_segments_emit.  C may be NULL; an empty handle gives C = 0.  KMG_ERR_ARG: NULL seg or st, max_gap >= 2^31,
+ * max_shift > max_gap or > 1024 (the search visits every occupied diagonal of the band), seg on another device than the
+ * calling thread, chains outside [0, C). */
+typedef struct kmg_chains kmg_chains;
+int kmg_chains_begin(const kmg_segments *seg, uint32_t max_gap, uint32_t max_shift, uint32_t min_rows,
+                     kmg_chains **st, uint64_t *C);
+int kmg_chains_emit(kmg_chains *st, int32_t *out /* 6C */);
+int kmg_chains_emit_chunk(kmg_chains *st, uint64_t first, uint64_t n, int32_t *out /* 6n */);
+int kmg_chains_free(kmg_chains *st);   /* NULL accepted */
+
 /* ---- sharded build (one process per GPU; the exchange itself is the host's NCCL all-to-all) ----
  * A rank holds bytes [g0,g1) of a global sequence of length L in device memory at d_seq (d_seq[0]
  * is byte g0) and owns the window starts [s0,s1), g0 <= max(s0-1,0), g1 >= min(L, s1+k-1).

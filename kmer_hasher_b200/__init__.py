@@ -21,7 +21,7 @@ from . import _lib
 from ._lib import KmgError, check
 
 __all__ = ["KmerHash", "KmerCounts", "SequenceFile", "make_kmer_hash_file", "count_kmers_file", "make_kmer_hash", "kmer_pos", "seq_kmer_pos", "kmer_pairs", "count_kmers", "kmer_spectrum",
-           "seq_kmer_depth", "seq_kmer_dotplot", "kmer_pairs_dotplot", "seq_kmer_segments", "kmer_pairs_segments", "pinned_empty", "KmgError",
+           "seq_kmer_depth", "seq_kmer_dotplot", "kmer_pairs_dotplot", "seq_kmer_segments", "kmer_pairs_segments", "seq_kmer_chains", "kmer_pairs_chains", "pinned_empty", "KmgError",
            "OPT_KMER", "OPT_POS", "OPT_PAIRS", "OPT_COUNT", "NA_INTEGER"]
 
 # opt.flag bits, src/kmer_hash.c:17 (pos_opt_flags) in the reference
@@ -669,6 +669,89 @@ def kmer_pairs_segments(ptr_a, ptr_b, *, reverse_complement=False, max_count=0, 
     check(_L.kmg_join_segments_begin(a._handle(), b._handle(), int(bool(reverse_complement)), max_count, min_rows,
                                      C.byref(st), C.byref(R)))
     return _segments_emit(st, R, out)
+
+
+def seq_kmer_chains(ptr, seq, k, *, max_gap, max_shift, reverse_complement=False, max_count=0, min_run=1, min_rows=1,
+                    allow_k32=False, out=None):
+    """seq.kmer.chains (additive; the R closure is in INTEGRATION.md): the match segments seq_kmer_segments(ptr, seq, k,
+    reverse_complement=..., max_count=..., min_rows=min_run) would return, joined on the device across mismatches and
+    short indels into chains.
+
+    For runs s, t with last row (I_s, J_s) = (i_s + n_s - 1, j_s + n_s - 1), the gaps are gq = i_t - I_s - 1 and
+    gr = j_t - J_s - 1; t may follow s iff 0 <= gq, gr <= max_gap and |gq - gr| <= max_shift, at cost (max(gq, gr),
+    |gq - gr|, gq).  s -> t is a link when t is the least-cost successor of s and s the least-cost predecessor of t; a
+    chain is a maximal path of links.  Returns a (C, 6) int32 array of (i, j, I, J, n, m): the first row of the first run,
+    the last row of the last run, the rows n and the runs m of the chain, ordered by (i, j), only chains with
+    n >= min_rows.  A chain covers query bases [i - k + 1, I] and index bases [j, J + k - 1].  max_gap >= k bridges
+    isolated substitutions; max_shift is the longest indel bridged (at most max_gap and 1024).  max_gap = 0 gives the
+    segments themselves.  `out` may supply the result (numpy, pinned or a torch device tensor of at least 6 C int32)."""
+    ix = _extract_index(ptr)
+    if isinstance(seq, (list, tuple)):
+        if len(seq) != 1:
+            raise ValueError("seq_r should be a single sequence")
+        seq = seq[0]
+    k = int(k)
+    p, n, keep = _seq_buffer(seq)
+    if n <= k or k > (32 if allow_k32 else 31):
+        raise ValueError("the sequence should be longer than k and k should not be longer than 31")
+    max_count, min_run = _segments_limits(max_count, min_run)
+    max_gap, max_shift, min_rows = _chains_limits(max_gap, max_shift, min_rows)
+    st, R = C.c_void_p(), C.c_uint64()
+    check(_L.kmg_segments_begin(ix._handle(), p, n, k, int(bool(reverse_complement)), max_count, min_run,
+                                C.byref(st), C.byref(R)))
+    del keep
+    return _chains_emit(st, max_gap, max_shift, min_rows, out)
+
+
+def kmer_pairs_chains(ptr_a, ptr_b, *, max_gap, max_shift, reverse_complement=False, max_count=0, min_run=1, min_rows=1,
+                      out=None):
+    """kmer.pairs.chains (additive; the R closure is in INTEGRATION.md): the match segments kmer_pairs_segments(ptr_a,
+    ptr_b, reverse_complement=..., max_count=..., min_rows=min_run) would return, joined into chains as in
+    seq_kmer_chains.  With reverse_complement=True the runs are antiparallel: a run's last row is (x + n - 1, y - n + 1)
+    and gr = J_s - y_t - 1.  Returns a (C, 6) int32 array of (a, b, a_end, b_end, n, m) ordered by (a, b).  With one k a
+    forward chain covers a[a, a_end + k - 1] and b[b, b_end + k - 1], an antiparallel one a[a, a_end + k - 1] and
+    b[b_end, b + k - 1]."""
+    a, b = _extract_index(ptr_a), _extract_index(ptr_b)
+    max_count, min_run = _segments_limits(max_count, min_run)
+    max_gap, max_shift, min_rows = _chains_limits(max_gap, max_shift, min_rows)
+    st, R = C.c_void_p(), C.c_uint64()
+    check(_L.kmg_join_segments_begin(a._handle(), b._handle(), int(bool(reverse_complement)), max_count, min_run,
+                                     C.byref(st), C.byref(R)))
+    return _chains_emit(st, max_gap, max_shift, min_rows, out)
+
+
+def _chains_limits(max_gap, max_shift, min_rows):
+    max_gap, max_shift, min_rows = int(max_gap), int(max_shift), int(min_rows)
+    if not 0 <= max_gap < 2**31:
+        raise ValueError("max_gap must be a non-negative count below 2^31")
+    if not 0 <= max_shift <= min(max_gap, 1024):
+        raise ValueError("max_shift must be between 0 and min(max_gap, 1024)")
+    if not 0 <= min_rows < 2**32:
+        raise ValueError("min_rows must be a non-negative 32-bit count")
+    return max_gap, max_shift, min_rows
+
+
+def _chains_emit(seg, max_gap, max_shift, min_rows, out):
+    """The chains of the segments handle seg into `out` (allocated when None); seg is freed."""
+    st, Cn = C.c_void_p(), C.c_uint64()
+    try:
+        check(_L.kmg_chains_begin(seg, max_gap, max_shift, min_rows, C.byref(st), C.byref(Cn)))
+    finally:
+        _L.kmg_segments_free(seg)
+    try:
+        Cn = Cn.value
+        if Cn > INT_MAX:
+            raise OverflowError(f"{Cn} chains exceed an R matrix extent")
+        if out is None:
+            out = np.empty((Cn, 6), np.int32)
+        else:
+            size = out.nbytes if isinstance(out, np.ndarray) else out.numel() * out.element_size()
+            if size < 24 * Cn:
+                raise ValueError(f"out holds {size} bytes; the {Cn} chains need {24 * Cn}")
+        check(_L.kmg_chains_emit(st, _out_ptr(out)))
+    finally:
+        _L.kmg_chains_free(st)
+    return out[:Cn] if isinstance(out, np.ndarray) and out.ndim == 2 else out
 
 
 def _segments_limits(max_count, min_rows):

@@ -53,6 +53,10 @@ SIGNATURES = {
     "kmg_segments_emit_chunk": (C.c_int, [vp, C.c_uint64, C.c_uint64, vp]),
     "kmg_segments_free": (C.c_int, [vp]),
     "kmg_join_segments_begin": (C.c_int, [vp, vp, C.c_int, C.c_uint32, C.c_uint32, C.POINTER(vp), u64p]),
+    "kmg_chains_begin": (C.c_int, [vp, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(vp), u64p]),
+    "kmg_chains_emit": (C.c_int, [vp, vp]),
+    "kmg_chains_emit_chunk": (C.c_int, [vp, C.c_uint64, C.c_uint64, vp]),
+    "kmg_chains_free": (C.c_int, [vp]),
     "kmg_shard_sample": (C.c_int, [vp, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int, vp]),
     "kmg_shard_partition": (C.c_int, [vp, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int,
                                       u64p, C.c_int, vp, vp, u64p]),

@@ -1751,6 +1751,7 @@ extern "C" int kmg_join_dotplot(const kmg_index *a, const kmg_index *b, int64_t 
 // ------------------------------------------------------------------------------------------------
 struct kmg_segments {
   int device = 0;
+  bool anti = false;            // antiparallel runs (kmg_join_segments_begin with rc = 1): the chains' orientation
   uint64_t R = 0;
   int32_t *rows = nullptr;      // [3R]: (i, j, n) per run
 };
@@ -2016,6 +2017,7 @@ extern "C" int kmg_join_segments_begin(const kmg_index *a, const kmg_index *b, i
   kmg_segments *g = new (std::nothrow) kmg_segments();
   if (!g) return fail(KMG_ERR_NOMEM, "host allocation failed");
   g->device = a->device;
+  g->anti = rc == 1;
   int rv = join_segments_run(a, b, rc, max_count, min_rows, &g->rows, &g->R);
   if (rv == KMG_ERR_UNSTABLE) rv = join_segments_run(a, b, rc, max_count, min_rows, &g->rows, &g->R);   // the sort now ranks by bitmap
   if (rv != KMG_OK) { delete g; return rv; }
@@ -2049,6 +2051,179 @@ extern "C" int kmg_segments_emit(kmg_segments *g, int32_t *out) {
 }
 
 extern "C" int kmg_segments_free(kmg_segments *g) {
+  if (!g) return KMG_OK;
+  int prev = -1;
+  cudaGetDevice(&prev);
+  cudaSetDevice(g->device);
+  const bool mine = g_ctx.ready && g_ctx.device == g->device;
+  if (mine) cudaStreamSynchronize(g_ctx.stream()); else cudaDeviceSynchronize();
+  if (g->rows) g_arena[g->device & 63].put(g->rows, nullptr, true);
+  cudaGetLastError();
+  if (prev >= 0) cudaSetDevice(prev);
+  delete g;
+  return KMG_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// chains: the runs of a segments handle joined across mismatches and short indels (segments.cuh)
+// ------------------------------------------------------------------------------------------------
+struct kmg_chains {
+  int device = 0;
+  uint64_t C = 0;
+  int32_t *rows = nullptr;      // [6C]: (i, j, I, J, n, m) per chain
+};
+constexpr int CHAIN_COMPACT_ITEMS = 8, CHAIN_COMPACT_TILE = 256 * CHAIN_COMPACT_ITEMS;
+constexpr int CHAIN_MAX_ROUNDS = 40;                      // pointer jumping halves every chain per round: 31 rounds reach 2^31 runs
+
+// The chains of the R runs `runs` (12 R bytes, (i, j) order) with n >= min_rows, as (i, j, I, J, n, m) rows in the order of
+// their first runs: *rows (device, 24 * *C bytes) or nullptr when *C = 0.  ANTI: antiparallel runs.
+template <bool ANTI>
+static int chains_of(const int32_t *runs, uint64_t R, uint32_t G, uint32_t W, uint32_t min_rows, int32_t **rows, uint64_t *C) {
+  *rows = nullptr;
+  *C = 0;
+  if (R == 0) return KMG_OK;
+  cudaStream_t s = g_ctx.stream();
+  uint64_t *key = nullptr, *tot = nullptr;
+  uint32_t *run = nullptr, *si = nullptr, *sI = nullptr, *flag = nullptr, *ticket = nullptr;
+  int32_t *succ = nullptr, *pred = nullptr, *head = nullptr, *tmp = nullptr, *out = nullptr;
+  unsigned long long *nsum = nullptr, *nm = nullptr, *last = nullptr;
+  Pair64 *status = nullptr;
+  kmg_index *diag = nullptr;
+  int rounds = 0;
+  auto body = [&]() -> int {
+    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(R, 256), (uint64_t)g_ctx.sms * 16);
+    TRY(dalloc(&key, (size_t)R, s));
+    TRY(dalloc(&run, (size_t)R, s));
+    LAUNCH("chains_keys", s, chains_keys_kernel<ANTI><<<grid, 256, 0, s>>>(runs, R, key, run));
+    // the runs by diagonal, i ascending inside one (stable): keys below 2^32 (segment_key) are the 32 bits of a 16-mer
+    TRY(kmg_build_records(key, run, (int64_t)R, 16, &diag));
+    dfree(key, s); dfree(run, s);
+    TRY(dalloc(&si, (size_t)R, s));
+    TRY(dalloc(&sI, (size_t)R, s));
+    LAUNCH("chains_gather", s, chains_gather_kernel<<<grid, 256, 0, s>>>(runs, diag->pos, R, si, sI));
+    TRY(dalloc(&succ, (size_t)R, s));
+    TRY(dalloc(&pred, (size_t)R, s));
+    TRY(dalloc(&nsum, 1, s));
+    CU(cudaMemsetAsync(nsum, 0, 8, s));
+    LAUNCH("chains_link", s, chains_link_kernel<ANTI><<<(unsigned)ceil_div<uint64_t>(R, 256), 256, 0, s>>>(
+                                 runs, R, diag->ukeys, diag->U, diag->ustart, diag->pos, si, sI, G, W, succ, pred, nsum));
+    const uint64_t U = diag->U;
+    kmg_free(diag);
+    diag = nullptr;
+    dfree(si, s); dfree(sI, s);
+    TRY(dalloc(&head, (size_t)R, s));
+    LAUNCH("chains_heads", s, chains_heads_kernel<<<grid, 256, 0, s>>>(succ, pred, R, head));
+    dfree(succ, s); dfree(pred, s);
+    // the first run of every chain by pointer jumping: a round that moves no pointer ends it
+    TRY(dalloc(&flag, 1, s));
+    for (uint32_t moved = 1; moved;) {
+      if (++rounds > CHAIN_MAX_ROUNDS) return fail(KMG_ERR_CUDA, "internal error: pointer jumping did not settle in %d rounds", CHAIN_MAX_ROUNDS);
+      CU(cudaMemsetAsync(flag, 0, 4, s));
+      LAUNCH("chains_jump", s, chains_jump_kernel<<<grid, 256, 0, s>>>(head, R, flag));
+      CU(cudaMemcpyAsync(&moved, flag, 4, cudaMemcpyDeviceToHost, s));
+      CU(cudaStreamSynchronize(s));
+    }
+    TRY(dalloc(&nm, (size_t)R, s));
+    TRY(dalloc(&last, (size_t)R, s));
+    CU(cudaMemsetAsync(nm, 0, R * 8, s));
+    CU(cudaMemsetAsync(last, 0, R * 8, s));
+    LAUNCH("chains_aggregate", s, chains_aggregate_kernel<ANTI><<<grid, 256, 0, s>>>(runs, head, R, nm, last));
+    const uint64_t tiles = ceil_div<uint64_t>(R, CHAIN_COMPACT_TILE);
+    TRY(dalloc(&tmp, (size_t)(6 * R), s));
+    TRY(dalloc(&status, (size_t)tiles, s));
+    TRY(dalloc(&ticket, 1, s));
+    TRY(dalloc(&tot, 3, s));
+    CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
+    CU(cudaMemsetAsync(ticket, 0, 4, s));
+    LAUNCH("chains_compact", s, chains_compact_kernel<256, CHAIN_COMPACT_ITEMS, ANTI><<<(unsigned)tiles, 256, 0, s>>>(
+                                    runs, head, nm, last, R, min_rows, status, ticket, tmp, tot));
+    uint64_t h[3], n_runs = 0;
+    CU(cudaMemcpyAsync(h, tot, sizeof h, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(&n_runs, nsum, 8, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    if (h[1] != R || h[2] != n_runs)
+      return fail(KMG_ERR_CUDA, "internal error: the chains hold %llu runs of %llu rows, the handle %llu runs of %llu rows",
+                  (unsigned long long)h[1], (unsigned long long)h[2], (unsigned long long)R, (unsigned long long)n_runs);
+    // runs (12 B) and their keys (8 B); the gathered i and I; the link search (the runs, one lower bound over the U
+    // diagonal keys and the candidates' i / I, counted as 64 B per run); head, aggregates, the rows written
+    prof_bytes("chains_keys", 24.0 * R);
+    prof_bytes("chains_gather", 24.0 * R);
+    prof_bytes("chains_link", 12.0 * R + 8.0 * U + 64.0 * R + 8.0 * R);
+    prof_bytes("chains_heads", 16.0 * R);
+    prof_bytes("chains_jump", 8.0 * R * rounds);
+    prof_bytes("chains_aggregate", 16.0 * R + 16.0 * (R - h[0]));
+    prof_bytes("chains_compact", 16.0 * R + 24.0 * h[0]);
+    if (h[0] == R) { out = tmp; tmp = nullptr; }
+    else if (h[0]) {                                      // keep exactly the chains that passed min_rows
+      TRY(dalloc(&out, (size_t)(6 * h[0]), s));
+      CU(cudaMemcpyAsync(out, tmp, 24 * h[0], cudaMemcpyDeviceToDevice, s));
+      CU(cudaStreamSynchronize(s));
+    }
+    *C = h[0];
+    return KMG_OK;
+  };
+  const int rv = body();
+  cudaStreamSynchronize(s);
+  dfree(key, s); dfree(run, s); dfree(si, s); dfree(sI, s); dfree(succ, s); dfree(pred, s); dfree(head, s);
+  dfree(nsum, s); dfree(flag, s); dfree(nm, s); dfree(last, s); dfree(tmp, s); dfree(status, s); dfree(ticket, s);
+  dfree(tot, s);
+  if (diag) kmg_free(diag);
+  if (rv != KMG_OK) { dfree(out, s); *C = 0; return rv; }
+  *rows = out;
+  return KMG_OK;
+}
+
+extern "C" int kmg_chains_begin(const kmg_segments *seg, uint32_t max_gap, uint32_t max_shift, uint32_t min_rows,
+                                kmg_chains **st, uint64_t *C) {
+  if (!st) return fail(KMG_ERR_ARG, "st is NULL");
+  *st = nullptr;
+  if (!seg) return fail(KMG_ERR_ARG, "segments handle is NULL");
+  if (max_gap > (uint32_t)INT32_MAX) return fail(KMG_ERR_ARG, "max_gap must be below 2^31");
+  if (max_shift > max_gap) return fail(KMG_ERR_ARG, "max_shift (%u) must not exceed max_gap (%u)", max_shift, max_gap);
+  if (max_shift > 1024) return fail(KMG_ERR_ARG, "max_shift must be at most 1024");
+  TRY(ctx_init());
+  if (seg->device != g_ctx.device)
+    return fail(KMG_ERR_ARG, "the segments live on device %d but this thread works on device %d", seg->device, g_ctx.device);
+  kmg_chains *g = new (std::nothrow) kmg_chains();
+  if (!g) return fail(KMG_ERR_NOMEM, "host allocation failed");
+  g->device = seg->device;
+  auto run = [&]() {
+    return seg->anti ? chains_of<true>(seg->rows, seg->R, max_gap, max_shift, min_rows, &g->rows, &g->C)
+                     : chains_of<false>(seg->rows, seg->R, max_gap, max_shift, min_rows, &g->rows, &g->C);
+  };
+  int rv = run();
+  if (rv == KMG_ERR_UNSTABLE) rv = run();                 // the sort now ranks by bitmap
+  if (rv != KMG_OK) { delete g; return rv; }
+  *st = g;
+  if (C) *C = g->C;
+  return KMG_OK;
+}
+
+extern "C" int kmg_chains_emit_chunk(kmg_chains *g, uint64_t first, uint64_t n, int32_t *out) {
+  if (!g) return fail(KMG_ERR_ARG, "chains handle is NULL");
+  TRY(ctx_init());
+  if (g->device != g_ctx.device)
+    return fail(KMG_ERR_ARG, "the chains live on device %d but this thread works on device %d", g->device, g_ctx.device);
+  if (first > g->C || n > g->C - first) return fail(KMG_ERR_ARG, "chains outside the result");
+  if (n == 0) return KMG_OK;
+  if (!out) return fail(KMG_ERR_ARG, "out is NULL");
+  const int32_t *rows = g->rows;
+  const int sms = g_ctx.sms;
+  int rc = stream_rows(n, 24, out, CHUNK_BYTES / 24, [=](uint64_t f, uint64_t cnt, void *dst, uint64_t *, cudaStream_t s) -> int {
+    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(6 * cnt, 256), (uint64_t)sms * 16);
+    LAUNCH("chains_emit", s, segments_emit_kernel<<<grid, 256, 0, s>>>(rows + 6 * (first + f), 6 * cnt, (int32_t *)dst));
+    return KMG_OK;
+  });
+  prof_bytes("chains_emit", 48.0 * n);
+  return rc;
+}
+
+extern "C" int kmg_chains_emit(kmg_chains *g, int32_t *out) {
+  if (!g) return fail(KMG_ERR_ARG, "chains handle is NULL");
+  return kmg_chains_emit_chunk(g, 0, g->C, out);
+}
+
+extern "C" int kmg_chains_free(kmg_chains *g) {
   if (!g) return KMG_OK;
   int prev = -1;
   cudaGetDevice(&prev);

@@ -18,6 +18,8 @@
  *                                           additive: match segments, the diagonal runs of seq.kmer.pos rows
  *   kmer_pair_segments(ptr.a, ptr.b, params)
  *                                           additive: match segments of kmer.pairs rows, on either strand
+ *   sequence_kmer_chains(ptr, seq, k, params), kmer_pair_chains(ptr.a, ptr.b, params)
+ *                                           additive: match segments joined across mismatches and short indels
  *   R_init_kmer_hash                        replaces src/kmer_hash.c:1221-1224
  *
  * Differences a user can observe: k-mers come out in the order of a mix of their 2-bit key (ascending key
@@ -562,6 +564,77 @@ SEXP kmer_pair_segments(SEXP ptr_a, SEXP ptr_b, SEXP params_r) {
   return segments_matrix(st, R, "kmer.pairs.segments");
 }
 
+/* seq.kmer.chains / kmer.pairs.chains (additive; INTEGRATION.md): the match segments of seq.kmer.segments or
+ * kmer.pairs.segments (min.run = their min.rows), joined on the device across mismatches and short indels into chains,
+ * as a 6 x C integer matrix of (i, j, i.end, j.end, n, m) ordered by (i, j); the closures name and transpose.
+ * params = as.integer(c(rc, max.count, min.run, max.gap, max.shift, min.rows)). */
+static void finalise_chains_guard(SEXP g) {
+  kmg_chains *st = (kmg_chains *)R_ExternalPtrAddr(g);
+  if (st) kmg_chains_free(st);
+  R_ClearExternalPtr(g);
+}
+
+/* params checked */
+static const int *chains_params(SEXP params_r) {
+  if (TYPEOF(params_r) != INTSXP || length(params_r) != 6) error("params should be an integer vector of length 6");
+  const int *p = INTEGER(params_r);
+  if (p[0] != 0 && p[0] != 1) error("rc should be TRUE or FALSE");
+  if (p[1] < 0) error("max.count should be 0 (no limit) or positive");
+  if (p[2] < 0) error("min.run should be 0 or positive");
+  if (p[3] < 0) error("max.gap should be 0 or positive");
+  if (p[4] < 0 || p[4] > p[3] || p[4] > 1024) error("max.shift should be between 0 and min(max.gap, 1024)");
+  if (p[5] < 0) error("min.rows should be 0 or positive");
+  return p;
+}
+
+/* The chains of seg (freed here, on every path) as a 6 x C INTSXP matrix (a guard frees the chains if the allocation fails). */
+static SEXP chains_matrix(kmg_segments *seg, const int *p, const char *what) {
+  kmg_chains *st = NULL;
+  uint64_t C = 0;
+  const int rv = kmg_chains_begin(seg, (uint32_t)p[3], (uint32_t)p[4], (uint32_t)p[5], &st, &C);
+  kmg_segments_free(seg);
+  if (rv != KMG_OK) error("%s failed: %s", what, kmg_last_error());
+  if (C > (uint64_t)INT_MAX) {
+    kmg_chains_free(st);
+    error("%s would return %llu chains, more than an R matrix can hold (2^31-1)", what, (unsigned long long)C);
+  }
+  SEXP guard = PROTECT(R_MakeExternalPtr(st, R_NilValue, R_NilValue));
+  R_RegisterCFinalizerEx(guard, finalise_chains_guard, TRUE);
+  SEXP m = PROTECT(allocMatrix(INTSXP, 6, (int)C)); /* rows (i, j, i.end, j.end, n, m) */
+  const int rc = kmg_chains_emit(st, INTEGER(m));
+  kmg_chains_free(st);
+  R_ClearExternalPtr(guard);
+  UNPROTECT(2);
+  if (rc != KMG_OK) error("%s failed: %s", what, kmg_last_error());
+  return m;
+}
+
+SEXP sequence_kmer_chains(SEXP ptr_r, SEXP seq_r, SEXP k_r, SEXP params_r) {
+  kmer_handle *h = index_handle_or_error(ptr_r);
+  if (TYPEOF(seq_r) != STRSXP || length(seq_r) != 1) error("seq_r should be a single sequence");
+  if (TYPEOF(k_r) != INTSXP || length(k_r) != 1) error("k should be an integer of length 1");
+  const int k = INTEGER(k_r)[0];
+  SEXP s = STRING_ELT(seq_r, 0);
+  const char *allow = getenv("KMERGPU_ALLOW_K32");
+  const int kmax = (allow && allow[0] == '1') ? 32 : 31;
+  const int *p = chains_params(params_r);
+  if (length(s) <= k || k > kmax || k < 1) error("the sequence should be longer than k and k should not be longer than 31");
+  kmg_segments *seg = NULL;
+  if (kmg_segments_begin(h->index, CHAR(s), (int64_t)length(s), k, p[0], (uint32_t)p[1], (uint32_t)p[2], &seg, NULL) != KMG_OK)
+    error("seq.kmer.chains failed: %s", kmg_last_error());
+  return chains_matrix(seg, p, "seq.kmer.chains");
+}
+
+SEXP kmer_pair_chains(SEXP ptr_a, SEXP ptr_b, SEXP params_r) {
+  kmer_handle *a = index_handle_or_error(ptr_a);
+  kmer_handle *b = index_handle_or_error(ptr_b);
+  const int *p = chains_params(params_r);
+  kmg_segments *seg = NULL;
+  if (kmg_join_segments_begin(a->index, b->index, p[0], (uint32_t)p[1], (uint32_t)p[2], &seg, NULL) != KMG_OK)
+    error("kmer.pairs.chains failed: %s", kmg_last_error());
+  return chains_matrix(seg, p, "kmer.pairs.chains");
+}
+
 static const R_CallMethodDef call_methods[] = {
     {"make_kmer_h_index", (DL_FUNC)&make_kmer_h_index, 3},
     {"kmer_positions", (DL_FUNC)&kmer_positions, 2},
@@ -575,6 +648,8 @@ static const R_CallMethodDef call_methods[] = {
     {"kmer_pair_dotplot", (DL_FUNC)&kmer_pair_dotplot, 3},
     {"sequence_kmer_segments", (DL_FUNC)&sequence_kmer_segments, 4},
     {"kmer_pair_segments", (DL_FUNC)&kmer_pair_segments, 3},
+    {"sequence_kmer_chains", (DL_FUNC)&sequence_kmer_chains, 4},
+    {"kmer_pair_chains", (DL_FUNC)&kmer_pair_chains, 3},
     {NULL, NULL, 0}};
 
 void R_init_kmer_hash(DllInfo *info) { R_registerRoutines(info, NULL, call_methods, NULL, NULL); }
