@@ -547,8 +547,8 @@ def kmer_pairs(ptr_a, ptr_b, *, out: np.ndarray | None = None) -> np.ndarray:
 
     M x 2 int32 array, columns (a, b): for every k-mer that both indexes hold, each of its 1-based
     positions in `ptr_a` paired with each of its positions in `ptr_b` (a position outer, b position
-    inner), k-mers of `ptr_a` in ascending key order.  (The reference's own routine crashes on its
-    bucket walk, test.R:330-331; this is its evident intent.)
+    inner), k-mers of `ptr_a` in its own k-mer order (kmg_index_order: ascending key for do_sort=True).
+    (The reference's own routine crashes on its bucket walk, test.R:330-331; this is its evident intent.)
     """
     a, b = _extract_index(ptr_a), _extract_index(ptr_b)
     st, M = C.c_void_p(), C.c_uint64()
