@@ -9,8 +9,10 @@
 #include <atomic>
 #include <condition_variable>
 #include <deque>
+#include <initializer_list>
 #include <thread>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <type_traits>
@@ -317,6 +319,59 @@ static void dfree(T *&p, cudaStream_t s) {
   p = nullptr;
 }
 
+// One arena block of T owned by a scope: given back on the stream it was taken on when the scope ends, earlier by
+// reset(), never once release() has handed it to an index or handle.  It cannot be copied, so a block has one owner;
+// kernels and the emit lambdas of stream_rows take the raw pointer.  The unnamed namespace keeps
+// these helpers out of the library's exported symbols.
+namespace {
+template <typename T>
+class DevBuf {
+  T *p_ = nullptr;
+  cudaStream_t s_;
+ public:
+  explicit DevBuf(cudaStream_t s, T *owned = nullptr) : p_(owned), s_(s) {}
+  DevBuf(const DevBuf &) = delete;
+  DevBuf &operator=(const DevBuf &) = delete;
+  ~DevBuf() { reset(); }
+  int alloc(size_t count) { reset(); return dalloc(&p_, count, s_); }   // gives back the block it held first
+  void reset(T *owned = nullptr) { dfree(p_, s_); p_ = owned; }
+  T *release() { T *p = p_; p_ = nullptr; return p; }
+  T *get() const { return p_; }
+  operator T *() const { return p_; }
+};
+
+// Handles owned by a scope until they are handed out: freed by their kmg_*_free on every other path.
+template <auto Free>
+struct Freer { template <class H> void operator()(H *h) const { Free(h); } };
+using IndexPtr = std::unique_ptr<kmg_index, Freer<kmg_free>>;
+using QueryPtr = std::unique_ptr<kmg_query, Freer<kmg_query_free>>;
+using JoinPtr = std::unique_ptr<kmg_join, Freer<kmg_join_free>>;
+using SegmentsPtr = std::unique_ptr<kmg_segments, Freer<kmg_segments_free>>;
+using ChainsPtr = std::unique_ptr<kmg_chains, Freer<kmg_chains_free>>;
+using ReadsPtr = std::unique_ptr<kmg_reads, Freer<kmg_reads_free>>;
+}  // namespace
+
+// A handle's arrays back to the arena of its device.  May run on a finaliser thread that never used the library, so the
+// device's work is waited for first and the blocks are made reusable by any stream.
+static void release_on_device(int device, std::initializer_list<void *> ptrs) {
+  int prev = -1;
+  cudaGetDevice(&prev);
+  cudaSetDevice(device);
+  const bool mine = g_ctx.ready && g_ctx.device == device;
+  if (mine) cudaStreamSynchronize(g_ctx.stream()); else cudaDeviceSynchronize();
+  for (void *p : ptrs) g_arena[device & 63].put(p, nullptr, true);
+  cudaGetLastError();
+  if (prev >= 0) cudaSetDevice(prev);
+}
+
+// A handle is used on the device it lives on: this thread's streams, events and arena belong to its current device
+// (kmg_set_device), so a handle of another device is refused rather than driven with the wrong resources.
+static int use_device(int device, const char *what) {
+  TRY(ctx_init());
+  if (device == g_ctx.device) return KMG_OK;
+  return fail(KMG_ERR_ARG, "%s on device %d but this thread works on device %d: call kmg_set_device(%d) first", what, device, g_ctx.device, device);
+}
+
 // ------------------------------------------------------------------------------------------------
 // pageable host buffers at PCIe speed: pinned staging + host copy threads
 // ------------------------------------------------------------------------------------------------
@@ -431,22 +486,19 @@ static PtrKind ptr_kind(const void *p) {
   return PK_HOST_PAGEABLE;
 }
 
-// The sequence on the device: 16 bytes of front padding (so base[-1] exists), data, zero padding to
-// a multiple of 16 plus one spare group.
-struct DevSeq {
-  uint8_t *buf = nullptr;
-  uint8_t *base = nullptr;   // buf + 16 + lead
-  int64_t len = 0;
-};
-static int upload_seq(const void *src, int64_t len, cudaStream_t s, DevSeq *out) {
-  size_t cap = 16 + (size_t)((len + 15) / 16) * 16 + 16;
-  TRY(dalloc(&out->buf, cap, s));
-  out->base = out->buf + 16;
-  out->len = len;
-  CU(cudaMemsetAsync(out->buf, 0, 16, s));
-  CU(cudaMemsetAsync(out->buf + cap - 32, 0, 32, s));
-  if (len > (int64_t)(8 << 20) && staged_transfers() && ptr_kind(src) == PK_HOST_PAGEABLE) return staged_upload(out->base, src, (size_t)len, s);
-  if (len > 0) CU(cudaMemcpyAsync(out->base, src, (size_t)len, cudaMemcpyDefault, s));
+// A sequence on the device: 16 bytes of front padding (so base[-1] exists), len bytes from base = buf + 16, zero
+// padding to a multiple of 16 plus one spare group.
+static int seq_alloc(DevBuf<uint8_t> &buf, int64_t len, cudaStream_t s) {
+  const size_t cap = 16 + (size_t)((len + 15) / 16) * 16 + 16;
+  TRY(buf.alloc(cap));
+  CU(cudaMemsetAsync(buf, 0, 16, s));
+  CU(cudaMemsetAsync(buf + cap - 32, 0, 32, s));
+  return KMG_OK;
+}
+static int upload_seq(const void *src, int64_t len, cudaStream_t s, DevBuf<uint8_t> &buf) {
+  TRY(seq_alloc(buf, len, s));
+  if (len > (int64_t)(8 << 20) && staged_transfers() && ptr_kind(src) == PK_HOST_PAGEABLE) return staged_upload(buf + 16, src, (size_t)len, s);
+  if (len > 0) CU(cudaMemcpyAsync(buf + 16, src, (size_t)len, cudaMemcpyDefault, s));
   return KMG_OK;
 }
 
@@ -618,13 +670,12 @@ extern "C" int64_t kmg_tune_get(const char *key, int64_t arg) {
 static int lane_order_failures(uint32_t *failures) {
   TRY(ctx_init());
   cudaStream_t s = g_ctx.stream();
-  uint32_t *bad = nullptr;
-  TRY(dalloc(&bad, 1, s));
+  DevBuf<uint32_t> bad(s);
+  TRY(bad.alloc(1));
   CU(cudaMemsetAsync(bad, 0, 4, s));
   LAUNCH("lane_order_selftest", s, lane_order_selftest_kernel<<<g_ctx.sms * 4, 256, 0, s>>>(bad));
   CU(cudaMemcpyAsync(failures, bad, 4, cudaMemcpyDeviceToHost, s));
   CU(cudaStreamSynchronize(s));
-  dfree(bad, s);
   return KMG_OK;
 }
 extern "C" int kmg_selftest_lane_order(uint32_t *failures) {
@@ -690,10 +741,11 @@ static uint32_t record_tile(int rb) {
 
 // Scratch shared by the sort passes of one build.
 struct SortScratch {
-  uint32_t *small = nullptr;     // hist[(MAX_PASSES+1)][MAX_NB] | gbase[(MAX_PASSES+1)][MAX_NB] | common[RADIX] | tickets[16] | IndexStats
-  uint64_t *status = nullptr;    // [tiles][bins]
+  DevBuf<uint32_t> small;        // hist[(MAX_PASSES+1)][MAX_NB] | gbase[(MAX_PASSES+1)][MAX_NB] | common[RADIX] | tickets[16] | IndexStats
+  DevBuf<uint64_t> status;       // [tiles][bins]
   size_t small_words = 0, status_words = 0;
   static constexpr size_t H = (size_t)(MAX_PASSES + 1) * MAX_NB;
+  explicit SortScratch(cudaStream_t s) : small(s), status(s) {}
   uint32_t *hist(int r) const { return small + (size_t)r * MAX_NB; }
   uint32_t *gbase(int r) const { return small + H + (size_t)r * MAX_NB; }
   uint32_t *common() const { return small + 2 * H; }
@@ -707,13 +759,12 @@ static int scratch_clear(SortScratch &sc, cudaStream_t s) {
 }
 static int scratch_alloc(SortScratch &sc, int64_t n_upper, cudaStream_t s, int rb = RADIX_BITS) {
   sc.small_words = 2 * SortScratch::H + RADIX + 16 + sizeof(IndexStats) / 4;
-  TRY(dalloc(&sc.small, sc.small_words, s));
+  TRY(sc.small.alloc(sc.small_words));
   const size_t tiles = (size_t)ceil_div<int64_t>(n_upper > 0 ? n_upper : 1, SORT_TILE_MIN) + MAX_SEGS + 1;   // segment-aligned tiles: one partial tile per segment
   sc.status_words = tiles << rb;
-  TRY(dalloc(&sc.status, sc.status_words, s));
+  TRY(sc.status.alloc(sc.status_words));
   return scratch_clear(sc, s);
 }
-static void scratch_free(SortScratch &sc, cudaStream_t s) { dfree(sc.small, s); dfree(sc.status, s); }
 
 template <class... A>
 static int launch_scan_hist(int rb, cudaStream_t s, A... args) {
@@ -730,13 +781,13 @@ static int launch_scan_hist(int rb, cudaStream_t s, A... args) {
 static int finish_index(kmg_index *ix, SortScratch &sc, uint64_t *keys_sorted, uint32_t *pos_sorted,
                         int64_t n_upper, cudaStream_t s, bool hashed = false) {
   IndexStats *st = sc.stats();
-  uint64_t *ukeys = nullptr;
-  uint32_t *ustart = nullptr;
-  Pair64 *status2 = nullptr;
+  DevBuf<uint64_t> ukeys(s);
+  DevBuf<uint32_t> ustart(s);
+  DevBuf<Pair64> status2(s);
   const int64_t tiles = ceil_div<int64_t>(n_upper > 0 ? n_upper : 1, RLE_TILE);
-  TRY(dalloc(&ukeys, (size_t)n_upper, s));
-  TRY(dalloc(&ustart, (size_t)n_upper + 1, s));
-  TRY(dalloc(&status2, (size_t)tiles, s));
+  TRY(ukeys.alloc((size_t)n_upper));
+  TRY(ustart.alloc((size_t)n_upper + 1));
+  TRY(status2.alloc((size_t)tiles));
   CU(cudaMemsetAsync(status2, 0, (size_t)tiles * sizeof(Pair64), s));
   LAUNCH("rle", s, rle_kernel<RLE_THREADS, RLE_ITEMS><<<(unsigned)tiles, RLE_THREADS, 0, s>>>(
                        keys_sorted, pos_sorted, st, ukeys, ustart, status2, sc.ticket(MAX_PASSES + 1), hashed));
@@ -745,18 +796,18 @@ static int finish_index(kmg_index *ix, SortScratch &sc, uint64_t *keys_sorted, u
   CU(cudaStreamSynchronize(s));
   ix->N = h.n; ix->U = h.U; ix->unstable = h.unstable != 0;
   ix->have_stats = false;       // P, multi, max count: on first demand (ensure_stats)
-  dfree(status2, s);
+  status2.reset();
   // keep exact-size arrays when the over-allocation is large
   if (h.U * 2 < (uint64_t)n_upper) {
-    uint64_t *uk2; uint32_t *us2;
-    TRY(dalloc(&uk2, (size_t)h.U, s));
-    TRY(dalloc(&us2, (size_t)h.U + 1, s));
+    DevBuf<uint64_t> uk2(s);
+    DevBuf<uint32_t> us2(s);
+    TRY(uk2.alloc((size_t)h.U));
+    TRY(us2.alloc((size_t)h.U + 1));
     CU(cudaMemcpyAsync(uk2, ukeys, h.U * sizeof(uint64_t), cudaMemcpyDeviceToDevice, s));
     CU(cudaMemcpyAsync(us2, ustart, (h.U + 1) * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
-    dfree(ukeys, s); dfree(ustart, s);
-    ukeys = uk2; ustart = us2;
+    ukeys.reset(uk2.release()); ustart.reset(us2.release());
   }
-  ix->ukeys = ukeys; ix->ustart = ustart; ix->pos = pos_sorted;
+  ix->ukeys = ukeys.release(); ix->ustart = ustart.release(); ix->pos = pos_sorted;
   const double N = (double)h.n, U = (double)h.U;
   prof_bytes("rle", 12 * N + 12 * U);
   return KMG_OK;
@@ -796,16 +847,15 @@ static int sort_tail(SortScratch &sc, SortPlan plan, int first_pass, bool has_ne
 }
 
 // Collisions of the low bits of the mix: partition those groups by the whole mix (sk, sp: scratch of the
-// same size).  Returns the detect counters through h_cnt after the caller's next synchronisation.
+// same size).  Returns the detect counters through h_cnt after the caller's next synchronisation; the task lists are in
+// fixmem until then.
 static int fix_groups(SortScratch &sc, int bits, uint64_t *keys, uint32_t *pos, uint64_t *sk, uint32_t *sp, int64_t n_upper, cudaStream_t s,
-                      uint32_t *h_cnt /* [4], pinned or stack read after a sync */, uint32_t **fixmem_out) {
+                      uint32_t *h_cnt /* [4], pinned or stack read after a sync */, DevBuf<uint32_t> &fixmem) {
   FixLists fl{};
-  uint32_t *fixmem = nullptr;
   fl.small_cap = g_fix_cap > 0 ? (uint32_t)g_fix_cap : (uint32_t)std::max<int64_t>(1 << 20, n_upper / 8);
   fl.big_cap = 1 << 16;
   const size_t words = 4 + CLAIM_SLOTS + 2 * (size_t)fl.small_cap + 2 * (size_t)fl.big_cap;
-  TRY(dalloc(&fixmem, words, s));
-  *fixmem_out = fixmem;
+  TRY(fixmem.alloc(words));
   CU(cudaMemsetAsync(fixmem, 0, (4 + CLAIM_SLOTS) * sizeof(uint32_t), s));
   fl.counters = fixmem; fl.claim = fixmem + 4;
   fl.small_tasks = reinterpret_cast<uint2 *>(fixmem + 4 + CLAIM_SLOTS);
@@ -829,9 +879,9 @@ static int build_grouped(const SeqView &sv, SortPlan plan, kmg_index *ix, SortSc
                          uint32_t *&pb, int64_t n_upper, cudaStream_t s, bool *overflow, bool regions, bool *region_overflow) {
   const int R = plan.passes, rb = plan.rb, NB = 1 << rb;
   const uint32_t mask = (1u << rb) - 1;
-  uint64_t *kr = nullptr, *d_counts = nullptr;
-  uint32_t *pr = nullptr, *d_over = nullptr;
-  TileSegs *segs = nullptr;
+  DevBuf<uint64_t> kr(s), d_counts(s);
+  DevBuf<uint32_t> pr(s), d_over(s);
+  DevBuf<TileSegs> segs(s);
   uint32_t h_over = 0;
   regions = regions && R > 1 && NB <= MAX_SEGS && n_upper <= (int64_t)1600000000;   // region offsets are 32-bit signed in the pass
   const uint32_t cap = (uint32_t)(((uint64_t)(n_upper / NB) * 5 / 4 + 4096 + 15) & ~uint64_t(15));
@@ -840,71 +890,63 @@ static int build_grouped(const SeqView &sv, SortPlan plan, kmg_index *ix, SortSc
   } else if (regions && n_upper >= (int64_t)REGION_SAMPLE_STRIDE * 4096) {
     // A repeat-rich sequence puts a k-mer's every copy into one bin: ask a 1-in-251 sample whether the heaviest bin stays
     // clear of a region's size; if not, take the histogram path right away instead of finding out the expensive way.
-    uint32_t *d_s = nullptr, h_est = 0;
-    TRY(dalloc(&d_s, (size_t)MAX_NB + 1, s));
-    int rc0 = KMG_OK;
-    if (cudaMemsetAsync(d_s, 0, (MAX_NB + 1) * sizeof(uint32_t), s) != cudaSuccess) rc0 = fail(KMG_ERR_CUDA, "memset failed");
-    if (rc0 == KMG_OK) {
-      const unsigned g = (unsigned)std::min<int64_t>(ceil_div<int64_t>(n_upper / REGION_SAMPLE_STRIDE, 256), (int64_t)g_ctx.sms * 8);
-      region_sample_kernel<<<g, 256, 0, s>>>(sv, REGION_SAMPLE_STRIDE, mask, d_s);
-      region_estimate_kernel<<<1, 256, 0, s>>>(d_s, NB, REGION_SAMPLE_STRIDE, d_s + MAX_NB);
-      if (cudaMemcpyAsync(&h_est, d_s + MAX_NB, 4, cudaMemcpyDeviceToHost, s) != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess)
-        rc0 = fail(KMG_ERR_CUDA, "region estimate failed: %s", cudaGetErrorString(cudaGetLastError()));
-    }
-    dfree(d_s, s);
-    TRY(rc0);
+    DevBuf<uint32_t> d_s(s);
+    uint32_t h_est = 0;
+    TRY(d_s.alloc((size_t)MAX_NB + 1));
+    if (cudaMemsetAsync(d_s, 0, (MAX_NB + 1) * sizeof(uint32_t), s) != cudaSuccess) return fail(KMG_ERR_CUDA, "memset failed");
+    const unsigned g = (unsigned)std::min<int64_t>(ceil_div<int64_t>(n_upper / REGION_SAMPLE_STRIDE, 256), (int64_t)g_ctx.sms * 8);
+    region_sample_kernel<<<g, 256, 0, s>>>(sv, REGION_SAMPLE_STRIDE, mask, d_s);
+    region_estimate_kernel<<<1, 256, 0, s>>>(d_s, NB, REGION_SAMPLE_STRIDE, d_s + MAX_NB);
+    if (cudaMemcpyAsync(&h_est, d_s + MAX_NB, 4, cudaMemcpyDeviceToHost, s) != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess)
+      return fail(KMG_ERR_CUDA, "region estimate failed: %s", cudaGetErrorString(cudaGetLastError()));
     if ((uint64_t)h_est * 10 > (uint64_t)cap * 9) regions = false;       // within 10 % of a region: not worth the risk
   } else if (regions) {
     regions = false;                                       // small inputs: the sweep is cheap and the slack relatively small
   }
-  auto body = [&]() -> int {
-    PassParams<DigitBin, DigitBin> P{};
-    P.sv = sv; P.keys_out = ka; P.pos_out = pa;
-    P.gbase = sc.gbase(0); P.hist_next = sc.hist(1);
-    P.status = sc.status; P.ticket = sc.ticket(0); P.epoch = 1;
-    P.hashed = 1;
-    P.dbg = g_sort_dbg;
-    P.bin = DigitBin{0, mask}; P.next = DigitBin{rb, mask};
-    if (regions) {
-      TRY(dalloc(&kr, (size_t)NB * cap, s));
-      TRY(dalloc(&pr, (size_t)NB * cap, s));
-      TRY(dalloc(&d_counts, (size_t)MAX_SEGS, s));
-      TRY(dalloc(&d_over, 4, s));
-      TRY(dalloc(&segs, 1, s));
-      CU(cudaMemsetAsync(d_counts, 0, MAX_SEGS * sizeof(uint64_t), s));
-      LAUNCH("region_gbase", s, region_gbase_kernel<<<1, 256, 0, s>>>(sc.gbase(0), NB, cap, d_over));
-      P.keys_out = kr; P.pos_out = pr;
-      P.bin_counts = d_counts; P.bin_cap = cap; P.bin_overflow = d_over;
+  PassParams<DigitBin, DigitBin> P{};
+  P.sv = sv; P.keys_out = ka; P.pos_out = pa;
+  P.gbase = sc.gbase(0); P.hist_next = sc.hist(1);
+  P.status = sc.status; P.ticket = sc.ticket(0); P.epoch = 1;
+  P.hashed = 1;
+  P.dbg = g_sort_dbg;
+  P.bin = DigitBin{0, mask}; P.next = DigitBin{rb, mask};
+  if (regions) {
+    TRY(kr.alloc((size_t)NB * cap));
+    TRY(pr.alloc((size_t)NB * cap));
+    TRY(d_counts.alloc((size_t)MAX_SEGS));
+    TRY(d_over.alloc(4));
+    TRY(segs.alloc(1));
+    CU(cudaMemsetAsync(d_counts, 0, MAX_SEGS * sizeof(uint64_t), s));
+    LAUNCH("region_gbase", s, region_gbase_kernel<<<1, 256, 0, s>>>(sc.gbase(0), NB, cap, d_over));
+    P.keys_out = kr; P.pos_out = pr;
+    P.bin_counts = d_counts; P.bin_cap = cap; P.bin_overflow = d_over;
+    TRY((launch_pass<true, DigitBin, DigitBin, true>("sort_pass_seq", P, n_upper, s, rb)));
+    TRY(launch_scan_hist(rb, s, sc.hist(1), sc.gbase(1), (uint64_t *)nullptr));
+    LAUNCH("tile_segs", s, tile_segs_kernel<<<1, MAX_SEGS, 0, s>>>(d_counts, NB, (uint64_t)cap, record_tile(rb), segs, &sc.stats()->n));
+    CU(cudaMemcpyAsync(&h_over, d_over, 4, cudaMemcpyDeviceToHost, s));
+    // second pass: regions -> (ka, pa); afterwards the region arrays are free
+    uint64_t *rk = kr;
+    uint32_t *rp = pr;
+    TRY(sort_tail(sc, plan, 1, true, rk, rp, ka, pa, n_upper, s, nullptr, segs, NB, 2));
+    std::swap(rk, ka); std::swap(rp, pa);                  // sort_tail swapped (in, out): the data is in what it calls `rk`
+    TRY(sort_tail(sc, plan, 2, true, ka, pa, kb, pb, n_upper, s));
+  } else {
+    const int64_t tiles = ceil_div<int64_t>(n_upper, HIST_TILE);
+    const unsigned hgrid = (unsigned)std::min<int64_t>(tiles, (int64_t)g_ctx.sms * 2);
+    LAUNCH("hist_seq", s, hist_seq_kernel<HIST_THREADS, HIST_ITEMS, HashDigitBin><<<hgrid, HIST_THREADS, 0, s>>>(sv, sc.hist(0), HashDigitBin{0, mask}));
+    TRY(launch_scan_hist(rb, s, sc.hist(0), sc.gbase(0), &sc.stats()->n));
+    if (R > 1) {
       TRY((launch_pass<true, DigitBin, DigitBin, true>("sort_pass_seq", P, n_upper, s, rb)));
       TRY(launch_scan_hist(rb, s, sc.hist(1), sc.gbase(1), (uint64_t *)nullptr));
-      LAUNCH("tile_segs", s, tile_segs_kernel<<<1, MAX_SEGS, 0, s>>>(d_counts, NB, (uint64_t)cap, record_tile(rb), segs, &sc.stats()->n));
-      CU(cudaMemcpyAsync(&h_over, d_over, 4, cudaMemcpyDeviceToHost, s));
-      // second pass: regions -> (ka, pa); afterwards the region arrays are free
-      TRY(sort_tail(sc, plan, 1, true, kr, pr, ka, pa, n_upper, s, nullptr, segs, NB, 2));
-      std::swap(kr, ka); std::swap(pr, pa);                  // sort_tail swapped (in, out): the data is in what it calls `kr`
-      TRY(sort_tail(sc, plan, 2, true, ka, pa, kb, pb, n_upper, s));
     } else {
-      const int64_t tiles = ceil_div<int64_t>(n_upper, HIST_TILE);
-      const unsigned hgrid = (unsigned)std::min<int64_t>(tiles, (int64_t)g_ctx.sms * 2);
-      LAUNCH("hist_seq", s, hist_seq_kernel<HIST_THREADS, HIST_ITEMS, HashDigitBin><<<hgrid, HIST_THREADS, 0, s>>>(sv, sc.hist(0), HashDigitBin{0, mask}));
-      TRY(launch_scan_hist(rb, s, sc.hist(0), sc.gbase(0), &sc.stats()->n));
-      if (R > 1) {
-        TRY((launch_pass<true, DigitBin, DigitBin, true>("sort_pass_seq", P, n_upper, s, rb)));
-        TRY(launch_scan_hist(rb, s, sc.hist(1), sc.gbase(1), (uint64_t *)nullptr));
-      } else {
-        TRY((launch_pass<true, DigitBin, DigitBin, false>("sort_pass_seq", P, n_upper, s, rb)));
-      }
-      TRY(sort_tail(sc, plan, 1, true, ka, pa, kb, pb, n_upper, s));   // records ordered by the low bits of the mix, in (ka, pa)
+      TRY((launch_pass<true, DigitBin, DigitBin, false>("sort_pass_seq", P, n_upper, s, rb)));
     }
-    return KMG_OK;
-  };
-  int rc = body();
+    TRY(sort_tail(sc, plan, 1, true, ka, pa, kb, pb, n_upper, s));   // records ordered by the low bits of the mix, in (ka, pa)
+  }
   uint32_t h_cnt[4] = {0, 0, 0, 0};
-  uint32_t *fixmem = nullptr;
-  if (rc == KMG_OK) rc = fix_groups(sc, plan.bits(), ka, pa, kb, pb, n_upper, s, h_cnt, &fixmem);   // kb, pb are free: scratch
-  if (rc == KMG_OK) rc = finish_index(ix, sc, ka, pa, n_upper, s, true);      // synchronises
-  dfree(fixmem, s);
-  dfree(kr, s); dfree(pr, s); dfree(d_counts, s); dfree(d_over, s); dfree(segs, s);
+  DevBuf<uint32_t> fixmem(s);
+  TRY(fix_groups(sc, plan.bits(), ka, pa, kb, pb, n_upper, s, h_cnt, fixmem));   // kb, pb are free: scratch
+  TRY(finish_index(ix, sc, ka, pa, n_upper, s, true));      // synchronises
   *overflow = h_cnt[2] != 0;
   *region_overflow = h_over != 0;
   if (log_on()) fprintf(stderr, "[kmergpu] grouped build on %d bits: %u short and %u long groups fixed\n", plan.bits(), h_cnt[0], h_cnt[1]);
@@ -915,70 +957,7 @@ static int build_grouped(const SeqView &sv, SortPlan plan, kmg_index *ix, SortSc
   if (R > 2) prof_bytes("sort_pass_hist", 24 * N * (R - 2));
   if (R > 1) prof_bytes("sort_pass", 24 * N);
   prof_bytes("group_detect", 8 * N);
-  return rc;
-}
-
-// One attempt at an index of the windows of `sv` (the caller retries once if the position lists came out unordered).
-static int build_attempt(const SeqView &sv, int k, kmg_index *ix, int order, cudaStream_t s) {
-  const int64_t n_upper = sv.nstarts;
-  SortScratch sc;
-  uint64_t *ka = nullptr, *kb = nullptr;
-  uint32_t *pa = nullptr, *pb = nullptr;
-  auto body = [&]() -> int {
-    const int R = num_passes(k);
-    const bool grouped = grouped_for(k, order, n_upper);
-    const SortPlan gp = grouped_plan(n_upper);
-    TRY(scratch_alloc(sc, n_upper, s, grouped ? gp.rb : RADIX_BITS));
-    TRY(dalloc(&ka, (size_t)n_upper, s));
-    TRY(dalloc(&pa, (size_t)n_upper, s));
-    if (R > 1) { TRY(dalloc(&kb, (size_t)n_upper, s)); TRY(dalloc(&pb, (size_t)n_upper, s)); }
-    if (grouped) {
-      bool overflow = false, region_overflow = false;
-      TRY(build_grouped(sv, gp, ix, sc, ka, pa, kb, pb, n_upper, s, &overflow, g_no_regions != 1, &region_overflow));
-      if (region_overflow) {                              // a bin outgrew its region (a huge repeat): once more with the histogram
-        g_region_rebuilds.fetch_add(1);
-        if (log_on()) fprintf(stderr, "[kmergpu] a first-pass bin outgrew its region: rebuilding with the histogram sweep\n");
-        void *old[3] = {ix->ukeys, ix->ustart, nullptr};
-        for (void *p : old) g_arena[ix->device & 63].put(p, s, false);
-        ix->ukeys = nullptr; ix->ustart = nullptr; ix->pos = nullptr; ix->hbits = 0; ix->unstable = false;
-        TRY(scratch_clear(sc, s));
-        overflow = false;
-        TRY(build_grouped(sv, gp, ix, sc, ka, pa, kb, pb, n_upper, s, &overflow, false, &region_overflow));
-      }
-      if (!overflow) { pa = nullptr; ix->grouped = true; return KMG_OK; }
-      // more colliding groups than the task lists hold (not seen in practice): rebuild sorted by key
-      void *old[3] = {ix->ukeys, ix->ustart, nullptr};
-      for (void *p : old) g_arena[ix->device & 63].put(p, s, false);
-      ix->ukeys = nullptr; ix->ustart = nullptr; ix->pos = nullptr; ix->hbits = 0;
-      scratch_free(sc, s);
-      TRY(scratch_alloc(sc, n_upper, s, RADIX_BITS));
-    }
-    const int64_t tiles = ceil_div<int64_t>(n_upper, HIST_TILE);
-    const unsigned hgrid = (unsigned)std::min<int64_t>(tiles, (int64_t)g_ctx.sms * 2);
-    LAUNCH("hist_all", s, hist_all_kernel<HIST_THREADS, HIST_ITEMS><<<hgrid, HIST_THREADS, 0, s>>>(sv, sc.common(), sc.hist(0), MAX_NB));
-    LAUNCH("hist_finish", s, hist_finish_kernel<<<R, RADIX, 0, s>>>(k, sc.common(), sc.hist(0), sc.gbase(0), MAX_NB, &sc.stats()->n));
-    {
-      PassParams<DigitBin, DigitBin> P{};
-      P.sv = sv; P.keys_out = ka; P.pos_out = pa;
-      P.gbase = sc.gbase(0);
-      P.status = sc.status; P.ticket = sc.ticket(0); P.epoch = 1;
-      P.dbg = g_sort_dbg;
-      P.bin = DigitBin{0}; P.next = DigitBin{RADIX_BITS};
-      TRY((launch_pass<true, DigitBin, DigitBin, false>("sort_pass_seq", P, n_upper, s)));
-    }
-    TRY(sort_tail(sc, SortPlan{RADIX_BITS, R}, 1, false, ka, pa, kb, pb, n_upper, s));   // result ends in (ka, pa)
-    TRY(finish_index(ix, sc, ka, pa, n_upper, s));
-    pa = nullptr;                                          // now owned by the index
-    const double N = (double)ix->N, L = (double)sv.avail;
-    prof_bytes("hist_all", L);
-    prof_bytes("sort_pass_seq", L + 12 * N);
-    if (R > 1) prof_bytes("sort_pass", 24 * N * (R - 1));
-    return KMG_OK;
-  };
-  const int rc = body();
-  dfree(ka, s); dfree(kb, s); dfree(pa, s); dfree(pb, s);
-  scratch_free(sc, s);
-  return rc;
+  return KMG_OK;
 }
 
 static void release_index_arrays(kmg_index *ix, cudaStream_t s) {
@@ -988,37 +967,90 @@ static void release_index_arrays(kmg_index *ix, cudaStream_t s) {
   ix->grouped = false; ix->hbits = 0; ix->unstable = false;
 }
 
+// One attempt at an index of the windows of `sv` (the caller retries once if the position lists came out unordered).
+static int build_attempt(const SeqView &sv, int k, kmg_index *ix, int order, cudaStream_t s) {
+  const int64_t n_upper = sv.nstarts;
+  const int R = num_passes(k);
+  const bool grouped = grouped_for(k, order, n_upper);
+  const SortPlan gp = grouped_plan(n_upper);
+  SortScratch sc(s);
+  DevBuf<uint64_t> k0(s), k1(s);
+  DevBuf<uint32_t> p0(s), p1(s);
+  TRY(scratch_alloc(sc, n_upper, s, grouped ? gp.rb : RADIX_BITS));
+  TRY(k0.alloc((size_t)n_upper));
+  TRY(p0.alloc((size_t)n_upper));
+  if (R > 1) { TRY(k1.alloc((size_t)n_upper)); TRY(p1.alloc((size_t)n_upper)); }
+  uint64_t *ka = k0, *kb = k1;                             // the passes ping-pong between the two pairs
+  uint32_t *pa = p0, *pb = p1;
+  if (grouped) {
+    bool overflow = false, region_overflow = false;
+    TRY(build_grouped(sv, gp, ix, sc, ka, pa, kb, pb, n_upper, s, &overflow, g_no_regions != 1, &region_overflow));
+    if (region_overflow) {                              // a bin outgrew its region (a huge repeat): once more with the histogram
+      g_region_rebuilds.fetch_add(1);
+      if (log_on()) fprintf(stderr, "[kmergpu] a first-pass bin outgrew its region: rebuilding with the histogram sweep\n");
+      ix->pos = nullptr;                                // pa: still ours
+      release_index_arrays(ix, s);
+      TRY(scratch_clear(sc, s));
+      overflow = false;
+      TRY(build_grouped(sv, gp, ix, sc, ka, pa, kb, pb, n_upper, s, &overflow, false, &region_overflow));
+    }
+    if (!overflow) { (pa == p0.get() ? p0 : p1).release(); ix->grouped = true; return KMG_OK; }
+    // more colliding groups than the task lists hold (not seen in practice): rebuild sorted by key
+    ix->pos = nullptr;
+    release_index_arrays(ix, s);
+    sc.small.reset(); sc.status.reset();
+    TRY(scratch_alloc(sc, n_upper, s, RADIX_BITS));
+  }
+  const int64_t tiles = ceil_div<int64_t>(n_upper, HIST_TILE);
+  const unsigned hgrid = (unsigned)std::min<int64_t>(tiles, (int64_t)g_ctx.sms * 2);
+  LAUNCH("hist_all", s, hist_all_kernel<HIST_THREADS, HIST_ITEMS><<<hgrid, HIST_THREADS, 0, s>>>(sv, sc.common(), sc.hist(0), MAX_NB));
+  LAUNCH("hist_finish", s, hist_finish_kernel<<<R, RADIX, 0, s>>>(k, sc.common(), sc.hist(0), sc.gbase(0), MAX_NB, &sc.stats()->n));
+  {
+    PassParams<DigitBin, DigitBin> P{};
+    P.sv = sv; P.keys_out = ka; P.pos_out = pa;
+    P.gbase = sc.gbase(0);
+    P.status = sc.status; P.ticket = sc.ticket(0); P.epoch = 1;
+    P.dbg = g_sort_dbg;
+    P.bin = DigitBin{0}; P.next = DigitBin{RADIX_BITS};
+    TRY((launch_pass<true, DigitBin, DigitBin, false>("sort_pass_seq", P, n_upper, s)));
+  }
+  TRY(sort_tail(sc, SortPlan{RADIX_BITS, R}, 1, false, ka, pa, kb, pb, n_upper, s));   // result ends in (ka, pa)
+  TRY(finish_index(ix, sc, ka, pa, n_upper, s));
+  (pa == p0.get() ? p0 : p1).release();                    // now owned by the index
+  const double N = (double)ix->N, L = (double)sv.avail;
+  prof_bytes("hist_all", L);
+  prof_bytes("sort_pass_seq", L + 12 * N);
+  if (R > 1) prof_bytes("sort_pass", 24 * N * (R - 1));
+  return KMG_OK;
+}
+
 static int build_from_view(const SeqView &sv, int k, kmg_index **out, int order = KMG_ORDER_SORTED) {
   cudaStream_t s = g_ctx.stream();
-  kmg_index *ix = new (std::nothrow) kmg_index();
+  const int64_t n_upper = sv.nstarts;
+  if (n_upper > (int64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "%lld windows exceed the 32-bit coordinates of the reference", (long long)n_upper);
+  IndexPtr ix(new (std::nothrow) kmg_index());
   if (!ix) return fail(KMG_ERR_NOMEM, "host allocation failed");
   ix->device = g_ctx.device;
   ix->k = k;
-  const int64_t n_upper = sv.nstarts;
   if (n_upper <= 0) {                      // shorter than k: an empty index, as the C core gives
-    int rc = dalloc(&ix->ustart, 1, s);
-    if (rc == KMG_OK && cudaMemsetAsync(ix->ustart, 0, 4, s) != cudaSuccess) rc = fail(KMG_ERR_CUDA, "memset failed");
-    if (rc != KMG_OK) { delete ix; return rc; }
+    TRY(dalloc(&ix->ustart, 1, s));
+    if (cudaMemsetAsync(ix->ustart, 0, 4, s) != cudaSuccess) return fail(KMG_ERR_CUDA, "memset failed");
     cudaStreamSynchronize(s);
-    *out = ix;
+    *out = ix.release();
     return KMG_OK;
   }
-  if (n_upper > (int64_t)INT32_MAX) { delete ix; return fail(KMG_ERR_RANGE, "%lld windows exceed the 32-bit coordinates of the reference", (long long)n_upper); }
-  int rc = build_attempt(sv, k, ix, order, s);
-  if (rc == KMG_OK && ix->unstable) {
+  TRY(build_attempt(sv, k, ix.get(), order, s));
+  if (ix->unstable) {
     // A k-mer's positions are not ascending: the one-atomic rank variant's hardware assumption failed here.
     // Never use it on this device again and redo the build with the bitmap variant, which assumes nothing.
     const bool was_atomic = rank_variant() >= 3;
-    release_index_arrays(ix, s);
-    if (!was_atomic) rc = fail(KMG_ERR_CUDA, "internal error: position lists not ascending after a stable sort");
-    else {
-      demote_rank_variant();
-      rc = build_attempt(sv, k, ix, order, s);
-      if (rc == KMG_OK && ix->unstable) rc = fail(KMG_ERR_CUDA, "internal error: position lists not ascending after a stable sort");
-    }
+    release_index_arrays(ix.get(), s);
+    if (!was_atomic) return fail(KMG_ERR_CUDA, "internal error: position lists not ascending after a stable sort");
+    demote_rank_variant();
+    TRY(build_attempt(sv, k, ix.get(), order, s));
+    if (ix->unstable) return fail(KMG_ERR_CUDA, "internal error: position lists not ascending after a stable sort");
   }
-  if (rc != KMG_OK) { cudaStreamSynchronize(s); kmg_free(ix); return rc; }
-  *out = ix;
+  *out = ix.release();
   return KMG_OK;
 }
 
@@ -1047,13 +1079,12 @@ extern "C" int kmg_build_ordered(const char *seq, int64_t len, int k, int order,
   const double t0 = wall_ms();
   TRY(ctx_init());
   cudaStream_t s = g_ctx.stream();
-  DevSeq ds;
-  TRY(upload_seq(seq, len, s, &ds));
+  DevBuf<uint8_t> dseq(s);
+  TRY(upload_seq(seq, len, s, dseq));
   const double t1 = wall_ms();
   SeqView sv;
-  sv.base = ds.base; sv.nstarts = len - k + 1 > 0 ? len - k + 1 : 0; sv.avail = len; sv.s0 = 0; sv.L = len; sv.k = k;
-  int rc = build_from_view(sv, k, out, order);
-  dfree(ds.buf, s);
+  sv.base = dseq + 16; sv.nstarts = len - k + 1 > 0 ? len - k + 1 : 0; sv.avail = len; sv.s0 = 0; sv.L = len; sv.k = k;
+  const int rc = build_from_view(sv, k, out, order);
   if (log_on())
     fprintf(stderr, "[kmergpu] build len=%lld k=%d: upload(enqueue) %.3f ms, build %.3f ms (host wall clock)\n", (long long)len, k, t1 - t0, wall_ms() - t1);
   return rc;
@@ -1061,21 +1092,12 @@ extern "C" int kmg_build_ordered(const char *seq, int64_t len, int k, int order,
 
 extern "C" int kmg_free(kmg_index *ix) {
   if (!ix) return KMG_OK;
-  // may run on a finaliser thread that never used the library: make the blocks reusable by anyone
-  int prev = -1;
-  cudaGetDevice(&prev);
-  cudaSetDevice(ix->device);
-  const bool mine = g_ctx.ready && g_ctx.device == ix->device;
-  if (mine) cudaStreamSynchronize(g_ctx.stream()); else cudaDeviceSynchronize();
-  void *ptrs[6] = {ix->ukeys, ix->ustart, ix->pos, ix->hash, ix->multi_u, ix->pair_off};
-  for (void *p : ptrs) g_arena[ix->device & 63].put(p, nullptr, true);
-  cudaGetLastError();
-  if (prev >= 0) cudaSetDevice(prev);
+  release_on_device(ix->device, {ix->ukeys, ix->ustart, ix->pos, ix->hash, ix->multi_u, ix->pair_off});
   delete ix;
   return KMG_OK;
 }
 
-static int use_index(const kmg_index *ix);
+static int use_index(const kmg_index *ix) { return ix ? use_device(ix->device, "the index lives") : fail(KMG_ERR_ARG, "index is NULL"); }
 // P, multi and the longest list: one sweep of ustart (4U bytes), taken the first time something asks for them -- the pair
 // matrix's extent (kmg_sizes with P != NULL), kmg_index_stats, kmg_pairs*.  make.kmer.hash + kmer.pos(2|8) never does.
 static int ensure_stats(const kmg_index *cix) {
@@ -1085,19 +1107,14 @@ static int ensure_stats(const kmg_index *cix) {
   if (ix->U == 0) { ix->P = 0; ix->multi = 0; ix->maxc = 0; ix->have_stats = true; return KMG_OK; }
   TRY(use_index(ix));
   cudaStream_t s = g_ctx.stream();
-  IndexStats *st = nullptr, h;
-  TRY(dalloc(&st, 1, s));
-  auto body = [&]() -> int {
-    CU(cudaMemsetAsync(st, 0, sizeof(IndexStats), s));
-    const unsigned sgrid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(ix->U, 256 * 16), (uint64_t)g_ctx.sms * 8);
-    LAUNCH("stats", s, stats_kernel<256><<<sgrid, 256, 0, s>>>(ix->ustart, ix->U, st));
-    CU(cudaMemcpyAsync(&h, st, sizeof h, cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    return KMG_OK;
-  };
-  const int rc = body();
-  dfree(st, s);
-  TRY(rc);
+  DevBuf<IndexStats> st(s);
+  IndexStats h;
+  TRY(st.alloc(1));
+  CU(cudaMemsetAsync(st, 0, sizeof(IndexStats), s));
+  const unsigned sgrid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(ix->U, 256 * 16), (uint64_t)g_ctx.sms * 8);
+  LAUNCH("stats", s, stats_kernel<256><<<sgrid, 256, 0, s>>>(ix->ustart, ix->U, st));
+  CU(cudaMemcpyAsync(&h, st, sizeof h, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
   ix->P = h.P; ix->multi = h.multi; ix->maxc = h.maxc;
   ix->have_stats = true;
   prof_bytes("stats", 4.0 * (double)ix->U);
@@ -1124,16 +1141,6 @@ extern "C" int kmg_index_stats(const kmg_index *ix, uint64_t *multi, uint32_t *m
 // ------------------------------------------------------------------------------------------------
 // extraction
 // ------------------------------------------------------------------------------------------------
-// An index is used on the device it lives on: this thread's streams, events and arena belong to its current device
-// (kmg_set_device), so an index of another device is refused rather than driven with the wrong resources.
-static int use_index(const kmg_index *ix) {
-  if (!ix) return fail(KMG_ERR_ARG, "index is NULL");
-  TRY(ctx_init());
-  if (ix->device != g_ctx.device)
-    return fail(KMG_ERR_ARG, "the index lives on device %d but this thread works on device %d: call kmg_set_device(%d) first", ix->device, g_ctx.device, ix->device);
-  return KMG_OK;
-}
-
 // Run `emit(first, rows, d_dst)` over [0,total) rows of `row_bytes` each and land them at `out`.
 // Device destinations are written in place; host destinations go through two device chunks so the
 // copy of chunk c overlaps the kernel of chunk c+1.
@@ -1146,13 +1153,15 @@ static int stream_rows_staged(uint64_t total, size_t row_bytes, void *out, Emit 
   cudaStream_t s = g_ctx.stream(), cs = g_ctx.copy;
   const uint64_t chunk_rows = std::max<uint64_t>(1, STAGE_BYTES / row_bytes);
   const int64_t nchunks = (int64_t)ceil_div<uint64_t>(total, chunk_rows);
-  uint64_t *blk = nullptr;
-  char *buf[2] = {nullptr, nullptr};
-  TRY(dalloc(&blk, (size_t)ceil_div<uint64_t>(chunk_rows, EMIT_TILE), s));
-  int rc = dalloc(&buf[0], chunk_rows * row_bytes, s);
-  if (rc == KMG_OK && nchunks > 1) rc = dalloc(&buf[1], chunk_rows * row_bytes, s);
+  DevBuf<uint64_t> blk(s);
+  DevBuf<char> buf0(s), buf1(s);
+  TRY(blk.alloc((size_t)ceil_div<uint64_t>(chunk_rows, EMIT_TILE)));
+  TRY(buf0.alloc(chunk_rows * row_bytes));
+  if (nchunks > 1) TRY(buf1.alloc(chunk_rows * row_bytes));
+  char *buf[2] = {buf0, buf1};
   cudaEvent_t *ev = g_ctx.ev;                          // ev[0..1] kernel done, ev[4..6] slot filled (= device buffer free again)
   int64_t issued = 0, retired = 0;
+  int rc = KMG_OK;                                     // on a failure the copies in flight are still drained
   while (rc == KMG_OK && retired < nchunks) {
     while (rc == KMG_OK && issued < nchunks && issued - retired < 2) {
       const int64_t c = issued;
@@ -1180,7 +1189,6 @@ static int stream_rows_staged(uint64_t total, size_t row_bytes, void *out, Emit 
   for (int64_t c = std::max<int64_t>(0, retired - STAGE_SLOTS); c < retired; ++c) g_pool.wait((int)c);
   cudaStreamSynchronize(cs);
   cudaStreamSynchronize(s);
-  dfree(buf[0], s); dfree(buf[1], s); dfree(blk, s);
   if (rc == KMG_OK) {
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) rc = fail(KMG_ERR_CUDA, "extraction failed: %s", cudaGetErrorString(e));
@@ -1194,25 +1202,25 @@ static int stream_rows(uint64_t total, size_t row_bytes, void *out, uint64_t chu
   cudaStream_t s = g_ctx.stream();
   const bool to_device = ptr_kind(out) == PK_DEVICE;
   if (!to_device) chunk_rows = std::min<uint64_t>(chunk_rows, total);
-  uint64_t *blk = nullptr;                             // first segment of every EMIT_TILE-row block of the chunk being emitted
-  TRY(dalloc(&blk, (size_t)ceil_div<uint64_t>(to_device ? total : chunk_rows, EMIT_TILE), s));
+  DevBuf<uint64_t> blk(s);                             // first segment of every EMIT_TILE-row block of the chunk being emitted
+  TRY(blk.alloc((size_t)ceil_div<uint64_t>(to_device ? total : chunk_rows, EMIT_TILE)));
   if (to_device) {
-    int rc = emit((uint64_t)0, total, out, blk, s);
-    if (rc == KMG_OK && cudaStreamSynchronize(s) != cudaSuccess) rc = fail(KMG_ERR_CUDA, "extraction failed: %s", cudaGetErrorString(cudaGetLastError()));
-    dfree(blk, s);
-    return rc;
+    TRY(emit((uint64_t)0, total, out, blk, s));
+    if (cudaStreamSynchronize(s) != cudaSuccess) return fail(KMG_ERR_CUDA, "extraction failed: %s", cudaGetErrorString(cudaGetLastError()));
+    return KMG_OK;
   }
   if (staged_transfers() && total * row_bytes > (uint64_t)(8 << 20) && ptr_kind(out) == PK_HOST_PAGEABLE) {
-    dfree(blk, s);
+    blk.reset();
     return stream_rows_staged(total, row_bytes, out, emit);
   }
-  char *buf[2] = {nullptr, nullptr};
-  int rc = dalloc(&buf[0], chunk_rows * row_bytes, s);
-  if (rc == KMG_OK && total > chunk_rows) rc = dalloc(&buf[1], chunk_rows * row_bytes, s);
-  if (rc != KMG_OK) { dfree(buf[0], s); dfree(blk, s); return rc; }
+  DevBuf<char> buf0(s), buf1(s);
+  TRY(buf0.alloc(chunk_rows * row_bytes));
+  if (total > chunk_rows) TRY(buf1.alloc(chunk_rows * row_bytes));
+  char *buf[2] = {buf0, buf1};
   cudaStream_t cs = g_ctx.copy;
   cudaEvent_t *ev = g_ctx.ev;                        // ev[0..1] kernel done, ev[2..3] copy done
   uint64_t done = 0;
+  int rc = KMG_OK;                                   // on a failure the copies in flight are still drained
   for (int c = 0; done < total && rc == KMG_OK; ++c, done += chunk_rows) {
     const int b = c & 1;
     const uint64_t rows = std::min<uint64_t>(chunk_rows, total - done);
@@ -1227,7 +1235,6 @@ static int stream_rows(uint64_t total, size_t row_bytes, void *out, uint64_t chu
   }
   cudaStreamSynchronize(cs);
   cudaStreamSynchronize(s);
-  dfree(buf[0], s); dfree(buf[1], s); dfree(blk, s);
   if (rc == KMG_OK) {
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) rc = fail(KMG_ERR_CUDA, "extraction failed: %s", cudaGetErrorString(e));
@@ -1309,21 +1316,20 @@ static int ensure_pair_index(kmg_index *ix) {
   std::lock_guard<std::mutex> g(ix->mu);
   if (ix->pair_off || ix->multi == 0) return KMG_OK;
   cudaStream_t s = g_ctx.stream();
-  uint32_t *multi_u = nullptr, *ticket = nullptr;
-  uint64_t *pair_off = nullptr;
-  Pair64 *status = nullptr;
+  DevBuf<uint32_t> multi_u(s), ticket(s);
+  DevBuf<uint64_t> pair_off(s);
+  DevBuf<Pair64> status(s);
   const uint64_t tiles = ceil_div<uint64_t>(ix->U, PIDX_TILE);
-  TRY(dalloc(&multi_u, ix->multi, s));
-  TRY(dalloc(&pair_off, ix->multi, s));
-  TRY(dalloc(&status, tiles, s));
-  TRY(dalloc(&ticket, 1, s));
+  TRY(multi_u.alloc(ix->multi));
+  TRY(pair_off.alloc(ix->multi));
+  TRY(status.alloc(tiles));
+  TRY(ticket.alloc(1));
   CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
   CU(cudaMemsetAsync(ticket, 0, 4, s));
   LAUNCH("pair_index", s, pair_index_kernel<PIDX_THREADS, PIDX_ITEMS><<<(unsigned)tiles, PIDX_THREADS, 0, s>>>(
                               ix->ustart, ix->U, multi_u, pair_off, status, ticket));
   CU(cudaStreamSynchronize(s));
-  dfree(status, s); dfree(ticket, s);
-  ix->multi_u = multi_u; ix->pair_off = pair_off;
+  ix->multi_u = multi_u.release(); ix->pair_off = pair_off.release();
   prof_bytes("pair_index", 4.0 * ix->U + 12.0 * ix->multi);
   return KMG_OK;
 }
@@ -1365,44 +1371,37 @@ static int ensure_hash(kmg_index *ix) {
   if (ix->hash || ix->U == 0) return KMG_OK;
   cudaStream_t s = g_ctx.stream();
   const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(ix->U, 256), (uint64_t)g_ctx.sms * 32);
-  uint4 *slots = nullptr;
+  DevBuf<uint4> slots(s);
   // grouped index: the k-mers are in ascending order of the sorted bits of their mix, which a monotone bucket function
   // turns into ascending bucket order: the table is streamed out (one bucket per k-mer on average = load 0.5)
   const bool stream = ix->grouped && ix->hbits >= 8 && ix->hbits <= 56 && !g_hash_cas && (ix->hbits >= 40 || ix->U + ix->U / 4 <= (uint64_t(1) << ix->hbits));
   if (stream) {
     const uint64_t nb = std::max<uint64_t>(ix->U + ix->U / 4, 4);      // 1.25 buckets of two slots per k-mer: load 0.4
-    uint64_t *d_last = nullptr;
-    TRY(dalloc(&slots, nb * BUCKET_SLOTS, s));
-    int rc = dalloc(&d_last, 1, s);
-    if (rc != KMG_OK) { dfree(slots, s); return rc; }
-    auto body = [&]() -> int {
-      KeyHash kt{slots, nb, ix->hbits};
-      uint64_t h_last = 0;
-      LAUNCH("hash_stream", s, hash_stream_kernel<<<grid, 256, 0, s>>>(ix->ukeys, ix->ustart, ix->U, kt, d_last));
-      CU(cudaMemcpyAsync(&h_last, d_last, 8, cudaMemcpyDeviceToHost, s));
-      CU(cudaStreamSynchronize(s));
-      if (h_last + 1 < nb) CU(cudaMemsetAsync(slots + (h_last + 1) * BUCKET_SLOTS, 0, (nb - h_last - 1) * BUCKET_SLOTS * sizeof(uint4), s));
-      constexpr int OV_ITEMS = 8;
-      const unsigned ogrid = (unsigned)ceil_div<uint64_t>(ix->U, 256 * OV_ITEMS);
-      LAUNCH("hash_insert", s, hash_overflow_kernel<OV_ITEMS><<<ogrid, 256, 0, s>>>(ix->ukeys, ix->ustart, ix->U, kt));
-      CU(cudaStreamSynchronize(s));
-      return KMG_OK;
-    };
-    rc = body();
-    dfree(d_last, s);
-    if (rc != KMG_OK) { dfree(slots, s); return rc; }
-    ix->hash = slots; ix->hash_nb = nb; ix->hash_hbits = ix->hbits;
+    DevBuf<uint64_t> d_last(s);
+    TRY(slots.alloc(nb * BUCKET_SLOTS));
+    TRY(d_last.alloc(1));
+    KeyHash kt{slots, nb, ix->hbits};
+    uint64_t h_last = 0;
+    LAUNCH("hash_stream", s, hash_stream_kernel<<<grid, 256, 0, s>>>(ix->ukeys, ix->ustart, ix->U, kt, d_last));
+    CU(cudaMemcpyAsync(&h_last, d_last, 8, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    if (h_last + 1 < nb) CU(cudaMemsetAsync(slots + (h_last + 1) * BUCKET_SLOTS, 0, (nb - h_last - 1) * BUCKET_SLOTS * sizeof(uint4), s));
+    constexpr int OV_ITEMS = 8;
+    const unsigned ogrid = (unsigned)ceil_div<uint64_t>(ix->U, 256 * OV_ITEMS);
+    LAUNCH("hash_insert", s, hash_overflow_kernel<OV_ITEMS><<<ogrid, 256, 0, s>>>(ix->ukeys, ix->ustart, ix->U, kt));
+    CU(cudaStreamSynchronize(s));
+    ix->hash = slots.release(); ix->hash_nb = nb; ix->hash_hbits = ix->hbits;
     prof_bytes("hash_stream", 12.0 * ix->U + 16.0 * BUCKET_SLOTS * nb);
     prof_bytes("hash_insert", 8.0 * ix->U);
     return KMG_OK;
   }
   uint64_t cap = 4 * BUCKET_SLOTS;
   while (cap < 2 * ix->U) cap <<= 1;                          // load <= 0.5
-  TRY(dalloc(&slots, cap, s));
+  TRY(slots.alloc(cap));
   CU(cudaMemsetAsync(slots, 0, cap * sizeof(uint4), s));
   LAUNCH("hash_insert", s, hash_insert_kernel<<<grid, 256, 0, s>>>(ix->ukeys, IndexPayload{ix->ustart}, ix->U, KeyHash{slots, cap / BUCKET_SLOTS, 0}, false));
   CU(cudaStreamSynchronize(s));
-  ix->hash = slots; ix->hash_nb = cap / BUCKET_SLOTS; ix->hash_hbits = 0;
+  ix->hash = slots.release(); ix->hash_nb = cap / BUCKET_SLOTS; ix->hash_hbits = 0;
   prof_bytes("hash_insert", 12.0 * ix->U + 16.0 * ix->U);
   return KMG_OK;
 }
@@ -1412,54 +1411,47 @@ static int query_common(const kmg_index *cix, bool from_seq, const SeqView &sv, 
                         uint32_t max_count = UINT32_MAX) {
   kmg_index *ix = const_cast<kmg_index *>(cix);
   cudaStream_t s = g_ctx.stream();
-  kmg_query *q = new (std::nothrow) kmg_query();
+  QueryPtr q(new (std::nothrow) kmg_query());
   if (!q) return fail(KMG_ERR_NOMEM, "host allocation failed");
   q->idx = ix;
   const int64_t total = from_seq ? sv.nstarts : n;
-  if (total <= 0 || ix->U == 0) { *out = q; if (M) *M = 0; return KMG_OK; }
-  int rc = ensure_hash(ix);
-  if (rc != KMG_OK) { delete q; return rc; }
-  QueryStats *qs = nullptr;
-  Pair64 *status = nullptr;
-  uint32_t *ticket = nullptr;
-  uint2 *found = nullptr;
-  auto body = [&]() -> int {
-    const uint64_t tiles = ceil_div<uint64_t>((uint64_t)total, COMPACT_TILE);
-    TRY(dalloc(&q->hit_i, (size_t)total, s));
-    TRY(dalloc(&q->hit_start, (size_t)total, s));
-    TRY(dalloc(&q->row_off, (size_t)total, s));
-    TRY(dalloc(&qs, 1, s));
-    TRY(dalloc(&status, tiles, s));
-    TRY(dalloc(&ticket, 1, s));
-    CU(cudaMemsetAsync(qs, 0, sizeof(QueryStats), s));
-    CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
-    CU(cudaMemsetAsync(ticket, 0, 4, s));
-    KeyHash kt{ix->hash, ix->hash_nb, ix->hash_hbits};
-    TRY(dalloc(&found, (size_t)total, s));
-    const unsigned ltiles = (unsigned)ceil_div<uint64_t>((uint64_t)total, PROBE_TILE);
-    if (from_seq) {
-      LAUNCH("probe_lookup", s, probe_lookup_kernel<PROBE_THREADS, PROBE_ITEMS, true><<<ltiles, PROBE_THREADS, 0, s>>>(sv, nullptr, 0, nullptr, kt, found));
-      LAUNCH("probe_compact", s, probe_compact_kernel<PROBE_THREADS, COMPACT_ITEMS, true><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
-                                     found, sv.s0 + sv.k, nullptr, total, nullptr, q->hit_i, q->hit_start, q->row_off, qs, status, ticket, max_count));
-    } else {
-      LAUNCH("probe_lookup_rec", s, probe_lookup_kernel<PROBE_THREADS, PROBE_ITEMS, false><<<ltiles, PROBE_THREADS, 0, s>>>(sv, d_keys, n, d_n, kt, found, mixed));
-      LAUNCH("probe_compact", s, probe_compact_kernel<PROBE_THREADS, COMPACT_ITEMS, false><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
-                                     found, 0, d_i, n, d_n, q->hit_i, q->hit_start, q->row_off, qs, status, ticket, max_count));
-    }
-    QueryStats h;
-    CU(cudaMemcpyAsync(&h, qs, sizeof h, cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    q->H = h.H; q->M = h.M;
-    return KMG_OK;
-  };
-  rc = body();
-  dfree(qs, s); dfree(status, s); dfree(ticket, s); dfree(found, s);
-  if (rc != KMG_OK) { cudaStreamSynchronize(s); kmg_query_free(q); return rc; }
+  if (total <= 0 || ix->U == 0) { if (M) *M = 0; *out = q.release(); return KMG_OK; }
+  TRY(ensure_hash(ix));
+  DevBuf<QueryStats> qs(s);
+  DevBuf<Pair64> status(s);
+  DevBuf<uint32_t> ticket(s);
+  DevBuf<uint2> found(s);
+  const uint64_t tiles = ceil_div<uint64_t>((uint64_t)total, COMPACT_TILE);
+  TRY(dalloc(&q->hit_i, (size_t)total, s));
+  TRY(dalloc(&q->hit_start, (size_t)total, s));
+  TRY(dalloc(&q->row_off, (size_t)total, s));
+  TRY(qs.alloc(1));
+  TRY(status.alloc(tiles));
+  TRY(ticket.alloc(1));
+  CU(cudaMemsetAsync(qs, 0, sizeof(QueryStats), s));
+  CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
+  CU(cudaMemsetAsync(ticket, 0, 4, s));
+  KeyHash kt{ix->hash, ix->hash_nb, ix->hash_hbits};
+  TRY(found.alloc((size_t)total));
+  const unsigned ltiles = (unsigned)ceil_div<uint64_t>((uint64_t)total, PROBE_TILE);
+  if (from_seq) {
+    LAUNCH("probe_lookup", s, probe_lookup_kernel<PROBE_THREADS, PROBE_ITEMS, true><<<ltiles, PROBE_THREADS, 0, s>>>(sv, nullptr, 0, nullptr, kt, found));
+    LAUNCH("probe_compact", s, probe_compact_kernel<PROBE_THREADS, COMPACT_ITEMS, true><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
+                                   found, sv.s0 + sv.k, nullptr, total, nullptr, q->hit_i, q->hit_start, q->row_off, qs, status, ticket, max_count));
+  } else {
+    LAUNCH("probe_lookup_rec", s, probe_lookup_kernel<PROBE_THREADS, PROBE_ITEMS, false><<<ltiles, PROBE_THREADS, 0, s>>>(sv, d_keys, n, d_n, kt, found, mixed));
+    LAUNCH("probe_compact", s, probe_compact_kernel<PROBE_THREADS, COMPACT_ITEMS, false><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
+                                   found, 0, d_i, n, d_n, q->hit_i, q->hit_start, q->row_off, qs, status, ticket, max_count));
+  }
+  QueryStats h;
+  CU(cudaMemcpyAsync(&h, qs, sizeof h, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  q->H = h.H; q->M = h.M;
   // a lookup moves one 128-byte line of HBM (measured: tools/micro/gups.cu), whatever it uses of it
   prof_bytes(from_seq ? "probe_lookup" : "probe_lookup_rec", (from_seq ? (double)sv.avail : 8.0 * total) + 128.0 * total + 8.0 * total);
   prof_bytes("probe_compact", 8.0 * total + 16.0 * q->H);
-  *out = q;
   if (M) *M = q->M;
+  *out = q.release();
   return KMG_OK;
 }
 
@@ -1472,30 +1464,21 @@ static int query_seq(const kmg_index *ix, const char *qseq, int64_t qlen, int k,
   if (qlen + 1 > (int64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "query longer than int coordinates");
   TRY(use_index(ix));
   cudaStream_t s = g_ctx.stream();
-  DevSeq fwd, rev;
-  auto body = [&]() -> int {
-    TRY(upload_seq(qseq, qlen, s, &fwd));
-    const uint8_t *base = fwd.base;
-    if (rc) {
-      const size_t cap = 16 + (size_t)((qlen + 15) / 16) * 16 + 16;
-      TRY(dalloc(&rev.buf, cap, s));
-      rev.base = rev.buf + 16; rev.len = qlen;
-      CU(cudaMemsetAsync(rev.buf, 0, 16, s));
-      CU(cudaMemsetAsync(rev.buf + cap - 32, 0, 32, s));
-      if (qlen > 0) {
-        const unsigned grid = (unsigned)std::min<int64_t>(ceil_div<int64_t>(qlen, 256), (int64_t)g_ctx.sms * 16);
-        LAUNCH("revcomp", s, revcomp_kernel<<<grid, 256, 0, s>>>(fwd.base, qlen, rev.base));
-        prof_bytes("revcomp", 2.0 * qlen);
-      }
-      base = rev.base;
+  DevBuf<uint8_t> fwd(s), rev(s);
+  TRY(upload_seq(qseq, qlen, s, fwd));
+  const uint8_t *base = fwd + 16;
+  if (rc) {
+    TRY(seq_alloc(rev, qlen, s));
+    if (qlen > 0) {
+      const unsigned grid = (unsigned)std::min<int64_t>(ceil_div<int64_t>(qlen, 256), (int64_t)g_ctx.sms * 16);
+      LAUNCH("revcomp", s, revcomp_kernel<<<grid, 256, 0, s>>>(fwd + 16, qlen, rev + 16));
+      prof_bytes("revcomp", 2.0 * qlen);
     }
-    SeqView sv;
-    sv.base = base; sv.nstarts = qlen - k + 1 > 0 ? qlen - k + 1 : 0; sv.avail = qlen; sv.s0 = 0; sv.L = qlen; sv.k = k;
-    return query_common(ix, true, sv, nullptr, nullptr, 0, st, M, nullptr, false, max_count);
-  };
-  const int rv = body();
-  dfree(fwd.buf, s); dfree(rev.buf, s);              // on every path
-  return rv;
+    base = rev + 16;
+  }
+  SeqView sv;
+  sv.base = base; sv.nstarts = qlen - k + 1 > 0 ? qlen - k + 1 : 0; sv.avail = qlen; sv.s0 = 0; sv.L = qlen; sv.k = k;
+  return query_common(ix, true, sv, nullptr, nullptr, 0, st, M, nullptr, false, max_count);
 }
 
 extern "C" int kmg_query_begin(const kmg_index *ix, const char *qseq, int64_t qlen, int k, kmg_query **st, uint64_t *M) {
@@ -1542,16 +1525,7 @@ extern "C" int kmg_query_emit(kmg_query *q, int32_t *out) {
 }
 extern "C" int kmg_query_free(kmg_query *q) {
   if (!q) return KMG_OK;
-  const int dev = q->idx ? q->idx->device : g_ctx.device;
-  int prev = -1;
-  cudaGetDevice(&prev);
-  cudaSetDevice(dev);
-  const bool mine = g_ctx.ready && g_ctx.device == dev;
-  if (mine) cudaStreamSynchronize(g_ctx.stream()); else cudaDeviceSynchronize();
-  void *ptrs[3] = {q->hit_i, q->hit_start, q->row_off};
-  for (void *p : ptrs) g_arena[dev & 63].put(p, nullptr, true);
-  cudaGetLastError();
-  if (prev >= 0) cudaSetDevice(prev);
+  release_on_device(q->idx ? q->idx->device : g_ctx.device, {q->hit_i, q->hit_start, q->row_off});
   delete q;
   return KMG_OK;
 }
@@ -1568,16 +1542,7 @@ struct kmg_join {
 
 extern "C" int kmg_join_free(kmg_join *j) {
   if (!j) return KMG_OK;
-  const int dev = j->a ? j->a->device : g_ctx.device;
-  int prev = -1;
-  cudaGetDevice(&prev);
-  cudaSetDevice(dev);
-  const bool mine = g_ctx.ready && g_ctx.device == dev;
-  if (mine) cudaStreamSynchronize(g_ctx.stream()); else cudaDeviceSynchronize();
-  void *ptrs[4] = {j->hit_astart, j->hit_bstart, j->hit_cb, j->row_off};
-  for (void *p : ptrs) g_arena[dev & 63].put(p, nullptr, true);
-  cudaGetLastError();
-  if (prev >= 0) cudaSetDevice(prev);
+  release_on_device(j->a ? j->a->device : g_ctx.device, {j->hit_astart, j->hit_bstart, j->hit_cb, j->row_off});
   delete j;
   return KMG_OK;
 }
@@ -1590,49 +1555,42 @@ static int join_begin(const kmg_index *a, const kmg_index *cb, uint32_t max_coun
   TRY(use_index(a));
   kmg_index *b = const_cast<kmg_index *>(cb);
   cudaStream_t s = g_ctx.stream();
-  kmg_join *j = new (std::nothrow) kmg_join();
+  JoinPtr j(new (std::nothrow) kmg_join());
   if (!j) return fail(KMG_ERR_NOMEM, "host allocation failed");
   j->a = a; j->b = b;
-  if (a->U == 0 || b->U == 0) { *out = j; if (M) *M = 0; return KMG_OK; }
-  int rc = ensure_hash(b);
-  if (rc != KMG_OK) { delete j; return rc; }
-  QueryStats *qs = nullptr;
-  Pair64 *status = nullptr;
-  uint32_t *ticket = nullptr;
-  uint2 *found = nullptr;
+  if (a->U == 0 || b->U == 0) { if (M) *M = 0; *out = j.release(); return KMG_OK; }
+  TRY(ensure_hash(b));
+  DevBuf<QueryStats> qs(s);
+  DevBuf<Pair64> status(s);
+  DevBuf<uint32_t> ticket(s);
+  DevBuf<uint2> found(s);
   const uint64_t U = a->U;
-  auto body = [&]() -> int {
-    const uint64_t tiles = ceil_div<uint64_t>(U, PROBE_TILE);
-    TRY(dalloc(&j->hit_astart, (size_t)U, s));
-    TRY(dalloc(&j->hit_bstart, (size_t)U, s));
-    TRY(dalloc(&j->hit_cb, (size_t)U, s));
-    TRY(dalloc(&j->row_off, (size_t)U, s));
-    TRY(dalloc(&found, (size_t)U, s));
-    TRY(dalloc(&qs, 1, s));
-    TRY(dalloc(&status, tiles, s));
-    TRY(dalloc(&ticket, 1, s));
-    CU(cudaMemsetAsync(qs, 0, sizeof(QueryStats), s));
-    CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
-    CU(cudaMemsetAsync(ticket, 0, 4, s));
-    KeyHash kt{b->hash, b->hash_nb, b->hash_hbits};
-    SeqView sv{};
-    LAUNCH("probe_lookup_rec", s, probe_lookup_kernel<PROBE_THREADS, PROBE_ITEMS, false><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
-                                      sv, a->ukeys, (int64_t)U, nullptr, kt, found));
-    LAUNCH("join_compact", s, join_compact_kernel<PROBE_THREADS, PROBE_ITEMS><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
-                                  found, a->ustart, U, j->hit_astart, j->hit_bstart, j->hit_cb, j->row_off, qs, status, ticket, max_count));
-    QueryStats h;
-    CU(cudaMemcpyAsync(&h, qs, sizeof h, cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    j->H = h.H; j->M = h.M;
-    return KMG_OK;
-  };
-  rc = body();
-  dfree(qs, s); dfree(status, s); dfree(ticket, s); dfree(found, s);
-  if (rc != KMG_OK) { cudaStreamSynchronize(s); kmg_join_free(j); return rc; }
+  const uint64_t tiles = ceil_div<uint64_t>(U, PROBE_TILE);
+  TRY(dalloc(&j->hit_astart, (size_t)U, s));
+  TRY(dalloc(&j->hit_bstart, (size_t)U, s));
+  TRY(dalloc(&j->hit_cb, (size_t)U, s));
+  TRY(dalloc(&j->row_off, (size_t)U, s));
+  TRY(found.alloc((size_t)U));
+  TRY(qs.alloc(1));
+  TRY(status.alloc(tiles));
+  TRY(ticket.alloc(1));
+  CU(cudaMemsetAsync(qs, 0, sizeof(QueryStats), s));
+  CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
+  CU(cudaMemsetAsync(ticket, 0, 4, s));
+  KeyHash kt{b->hash, b->hash_nb, b->hash_hbits};
+  SeqView sv{};
+  LAUNCH("probe_lookup_rec", s, probe_lookup_kernel<PROBE_THREADS, PROBE_ITEMS, false><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
+                                    sv, a->ukeys, (int64_t)U, nullptr, kt, found));
+  LAUNCH("join_compact", s, join_compact_kernel<PROBE_THREADS, PROBE_ITEMS><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
+                                found, a->ustart, U, j->hit_astart, j->hit_bstart, j->hit_cb, j->row_off, qs, status, ticket, max_count));
+  QueryStats h;
+  CU(cudaMemcpyAsync(&h, qs, sizeof h, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  j->H = h.H; j->M = h.M;
   prof_bytes("probe_lookup_rec", 8.0 * U + 128.0 * U + 8.0 * U);
   prof_bytes("join_compact", 12.0 * U + 20.0 * j->H);
-  *out = j;
   if (M) *M = j->M;
+  *out = j.release();
   return KMG_OK;
 }
 
@@ -1690,30 +1648,25 @@ static int dotplot_run(const Rows &rows, const uint64_t *row_off, uint64_t H, ui
                        double *out) {
   cudaStream_t s = g_ctx.stream();
   const uint64_t cells = (uint64_t)ax.n * ay.n;
-  unsigned long long *img = nullptr;
-  uint64_t *blk = nullptr;
-  TRY(dalloc(&img, cells, s));
-  auto body = [&]() -> int {
-    CU(cudaMemsetAsync(img, 0, cells * sizeof(unsigned long long), s));
-    if (M) TRY(dalloc(&blk, (size_t)ceil_div<uint64_t>(std::min(M, DOT_SLICE_ROWS), EMIT_TILE), s));
-    for (uint64_t first = 0; first < M; first += DOT_SLICE_ROWS) {
-      const uint64_t n = std::min(DOT_SLICE_ROWS, M - first);
-      TRY(block_starts(row_off, H, first, n, s, blk));
-      LAUNCH("dotplot_bin", s, dotplot_bin_kernel<EMIT_THREADS, Rows><<<(unsigned)ceil_div<uint64_t>(n, EMIT_TILE), EMIT_THREADS, 0, s>>>(
-                                   rows, row_off, H, first, n, blk, ax, ay, img));
-    }
-    const int sms = g_ctx.sms;
-    const unsigned long long *im = img;
-    return stream_rows(cells, 8, out, CHUNK_BYTES / 8, [=](uint64_t f, uint64_t n, void *dst, uint64_t *, cudaStream_t st) -> int {
-      const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(n, 256), (uint64_t)sms * 16);
-      LAUNCH("dotplot_finish", st, dotplot_finish_kernel<<<grid, 256, 0, st>>>(im + f, n, (double *)dst));
-      return KMG_OK;
-    });
-  };
-  const int rc = body();
+  DevBuf<unsigned long long> img(s);
+  DevBuf<uint64_t> blk(s);
+  TRY(img.alloc(cells));
+  CU(cudaMemsetAsync(img, 0, cells * sizeof(unsigned long long), s));
+  if (M) TRY(blk.alloc((size_t)ceil_div<uint64_t>(std::min(M, DOT_SLICE_ROWS), EMIT_TILE)));
+  for (uint64_t first = 0; first < M; first += DOT_SLICE_ROWS) {
+    const uint64_t n = std::min(DOT_SLICE_ROWS, M - first);
+    TRY(block_starts(row_off, H, first, n, s, blk));
+    LAUNCH("dotplot_bin", s, dotplot_bin_kernel<EMIT_THREADS, Rows><<<(unsigned)ceil_div<uint64_t>(n, EMIT_TILE), EMIT_THREADS, 0, s>>>(
+                                 rows, row_off, H, first, n, blk, ax, ay, img));
+  }
+  const int sms = g_ctx.sms;
+  const unsigned long long *im = img;
+  TRY(stream_rows(cells, 8, out, CHUNK_BYTES / 8, [=](uint64_t f, uint64_t n, void *dst, uint64_t *, cudaStream_t st) -> int {
+    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(n, 256), (uint64_t)sms * 16);
+    LAUNCH("dotplot_finish", st, dotplot_finish_kernel<<<grid, 256, 0, st>>>(im + f, n, (double *)dst));
+    return KMG_OK;
+  }));
   cudaStreamSynchronize(s);
-  dfree(blk, s); dfree(img, s);
-  if (rc != KMG_OK) return rc;
   prof_bytes("dotplot_bin", row_bytes * (double)M + 8.0 * (double)cells);
   prof_bytes("dotplot_finish", 16.0 * (double)cells);
   return KMG_OK;
@@ -1727,10 +1680,9 @@ extern "C" int kmg_query_dotplot(const kmg_index *ix, const char *q, int64_t qle
   kmg_query *st = nullptr;
   uint64_t M = 0;
   TRY(query_seq(ix, q, qlen, k, rc == 1, max_count ? max_count : UINT32_MAX, &st, &M));
+  const QueryPtr probe(st);
   const ProbeRows rows{st->hit_i, st->hit_start, ix->pos};
-  const int rv = dotplot_run(rows, st->row_off, st->H, M, 4.0, dot_axis(x0, x1, nx), dot_axis(y0, y1, ny), out);
-  kmg_query_free(st);
-  return rv;
+  return dotplot_run(rows, st->row_off, st->H, M, 4.0, dot_axis(x0, x1, nx), dot_axis(y0, y1, ny), out);
 }
 
 extern "C" int kmg_join_dotplot(const kmg_index *a, const kmg_index *b, int64_t x0, int64_t x1, int nx, int64_t y0, int64_t y1, int ny,
@@ -1740,10 +1692,9 @@ extern "C" int kmg_join_dotplot(const kmg_index *a, const kmg_index *b, int64_t 
   kmg_join *j = nullptr;
   uint64_t M = 0;
   TRY(join_begin(a, b, max_count ? max_count : UINT32_MAX, &j, &M));
+  const JoinPtr join(j);
   const JoinRows rows{j->hit_astart, j->hit_bstart, j->hit_cb, a->pos, b->pos};
-  const int rv = dotplot_run(rows, j->row_off, j->H, M, 8.0, dot_axis(x0, x1, nx), dot_axis(y0, y1, ny), out);
-  kmg_join_free(j);
-  return rv;
+  return dotplot_run(rows, j->row_off, j->H, M, 8.0, dot_axis(x0, x1, nx), dot_axis(y0, y1, ny), out);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1761,69 +1712,64 @@ constexpr int SEG_PAIR_ITEMS = 8, SEG_PAIR_TILE = 256 * SEG_PAIR_ITEMS;
 
 // p[0, keep) moved into a fresh array of cap elements
 template <typename T>
-static int seg_grow(T *&p, uint64_t keep, uint64_t cap, cudaStream_t s) {
-  T *q = nullptr;
-  TRY(dalloc(&q, (size_t)cap, s));
+static int seg_grow(DevBuf<T> &p, uint64_t keep, uint64_t cap, cudaStream_t s) {
+  DevBuf<T> q(s);
+  TRY(q.alloc((size_t)cap));
   if (keep) CU(cudaMemcpyAsync(q, p, keep * sizeof(T), cudaMemcpyDeviceToDevice, s));
-  dfree(p, s);
-  p = q;
+  p.reset(q.release());
   return KMG_OK;
 }
 
 // Run starts (i, j) and run ends (diagonal key, i) of the probe st, each in row order, into arrays of at least R0 entries.
 template <bool ANTI>
-static int segments_mark(const kmg_query *st, const uint32_t *pos, int2 *&starts, uint64_t *&ekey, uint32_t *&ei, uint64_t *R0) {
+static int segments_mark(const kmg_query *st, const uint32_t *pos, DevBuf<int2> &starts, DevBuf<uint64_t> &ekey, DevBuf<uint32_t> &ei,
+                         uint64_t *R0) {
   cudaStream_t s = g_ctx.stream();
   const uint64_t M = st->M;
   const uint64_t slice_tiles = ceil_div<uint64_t>(std::min(M, SEG_SLICE_ROWS), EMIT_TILE);
   uint64_t cap = std::min(M, SEG_CAP0), bs = 0, be = 0;
-  uint64_t *blk = nullptr, *tot = nullptr;
-  Pair64 *status = nullptr;
-  uint32_t *ticket = nullptr;
-  auto body = [&]() -> int {
-    TRY(dalloc(&starts, (size_t)cap, s));
-    TRY(dalloc(&ekey, (size_t)cap, s));
-    TRY(dalloc(&ei, (size_t)cap, s));
-    TRY(dalloc(&blk, (size_t)slice_tiles, s));
-    TRY(dalloc(&status, (size_t)slice_tiles, s));
-    TRY(dalloc(&ticket, 1, s));
-    TRY(dalloc(&tot, 2, s));
-    for (uint64_t first = 0; first < M;) {
-      const uint64_t n = std::min(SEG_SLICE_ROWS, M - first);
-      const uint64_t tiles = ceil_div<uint64_t>(n, EMIT_TILE);
-      CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
-      CU(cudaMemsetAsync(ticket, 0, 4, s));
-      TRY(block_starts(st->row_off, st->H, first, n, s, blk));
-      LAUNCH("segments_mark", s, segments_mark_kernel<EMIT_THREADS, ANTI><<<(unsigned)tiles, EMIT_THREADS, 0, s>>>(
-                                     st->hit_i, st->hit_start, st->row_off, st->H, M, pos, first, n, blk, status, ticket, bs, be,
-                                     cap, starts, ekey, ei, tot));
-      uint64_t h[2];
-      CU(cudaMemcpyAsync(h, tot, sizeof h, cudaMemcpyDeviceToHost, s));
-      CU(cudaStreamSynchronize(s));
-      const uint64_t need = std::max(bs + h[0], be + h[1]);
-      if (need > (uint64_t)INT32_MAX)
-        return fail(KMG_ERR_RANGE, "more than 2^31 - 1 runs (%llu so far) to pair", (unsigned long long)need);
-      if (need > cap) {                                   // the slice did not fit: keep what is done, make room, run it again
-        const uint64_t ncap = std::min<uint64_t>(std::min(M, (uint64_t)INT32_MAX), need + need / 4);
-        TRY(seg_grow(starts, bs, ncap, s));
-        TRY(seg_grow(ekey, be, ncap, s));
-        TRY(seg_grow(ei, be, ncap, s));
-        cap = ncap;
-        continue;
-      }
-      bs += h[0]; be += h[1];
-      first += n;
+  DevBuf<uint64_t> blk(s), tot(s);
+  DevBuf<Pair64> status(s);
+  DevBuf<uint32_t> ticket(s);
+  TRY(starts.alloc((size_t)cap));
+  TRY(ekey.alloc((size_t)cap));
+  TRY(ei.alloc((size_t)cap));
+  TRY(blk.alloc((size_t)slice_tiles));
+  TRY(status.alloc((size_t)slice_tiles));
+  TRY(ticket.alloc(1));
+  TRY(tot.alloc(2));
+  for (uint64_t first = 0; first < M;) {
+    const uint64_t n = std::min(SEG_SLICE_ROWS, M - first);
+    const uint64_t tiles = ceil_div<uint64_t>(n, EMIT_TILE);
+    CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
+    CU(cudaMemsetAsync(ticket, 0, 4, s));
+    TRY(block_starts(st->row_off, st->H, first, n, s, blk));
+    LAUNCH("segments_mark", s, segments_mark_kernel<EMIT_THREADS, ANTI><<<(unsigned)tiles, EMIT_THREADS, 0, s>>>(
+                                   st->hit_i, st->hit_start, st->row_off, st->H, M, pos, first, n, blk, status, ticket, bs, be,
+                                   cap, starts, ekey, ei, tot));
+    uint64_t h[2];
+    CU(cudaMemcpyAsync(h, tot, sizeof h, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    const uint64_t need = std::max(bs + h[0], be + h[1]);
+    if (need > (uint64_t)INT32_MAX)
+      return fail(KMG_ERR_RANGE, "more than 2^31 - 1 runs (%llu so far) to pair", (unsigned long long)need);
+    if (need > cap) {                                   // the slice did not fit: keep what is done, make room, run it again
+      const uint64_t ncap = std::min<uint64_t>(std::min(M, (uint64_t)INT32_MAX), need + need / 4);
+      TRY(seg_grow(starts, bs, ncap, s));
+      TRY(seg_grow(ekey, be, ncap, s));
+      TRY(seg_grow(ei, be, ncap, s));
+      cap = ncap;
+      continue;
     }
-    if (bs != be)
-      return fail(KMG_ERR_CUDA, "internal error: %llu run starts but %llu run ends", (unsigned long long)bs, (unsigned long long)be);
-    return KMG_OK;
-  };
-  const int rc = body();
-  dfree(blk, s); dfree(status, s); dfree(ticket, s); dfree(tot, s);
+    bs += h[0]; be += h[1];
+    first += n;
+  }
+  if (bs != be)
+    return fail(KMG_ERR_CUDA, "internal error: %llu run starts but %llu run ends", (unsigned long long)bs, (unsigned long long)be);
   // rows (4 B) and one neighbouring position on either side; hits (16 B); the starts (8 B) and ends (12 B) written
-  if (rc == KMG_OK) prof_bytes("segments_mark", 12.0 * M + 16.0 * st->H + 20.0 * bs);
+  prof_bytes("segments_mark", 12.0 * M + 16.0 * st->H + 20.0 * bs);
   *R0 = bs;
-  return rc;
+  return KMG_OK;
 }
 
 // The runs of the probe st (freed here, on every path) with at least min_rows rows, as (i, j, n) triples in the order of
@@ -1832,55 +1778,50 @@ template <bool ANTI>
 static int segments_of(kmg_query *st, uint32_t min_rows, int32_t **rows, uint64_t *R) {
   *rows = nullptr;
   *R = 0;
+  QueryPtr probe(st);
   const uint64_t M = st->M;
-  if (M == 0) { kmg_query_free(st); return KMG_OK; }
+  if (M == 0) return KMG_OK;
   cudaStream_t s = g_ctx.stream();
-  int2 *starts = nullptr;
-  uint64_t *ekey = nullptr, *tot = nullptr;
-  uint32_t *ei = nullptr, *ticket = nullptr;
-  Pair64 *status = nullptr;
-  int32_t *tmp = nullptr, *out = nullptr;
-  kmg_index *ends = nullptr;
+  DevBuf<int2> starts(s);
+  DevBuf<uint64_t> ekey(s);
+  DevBuf<uint32_t> ei(s);
   uint64_t R0 = 0;
-  auto body = [&]() -> int {
-    const int m = segments_mark<ANTI>(st, st->idx->pos, starts, ekey, ei, &R0);
-    kmg_query_free(st);                                   // the probe is done with: only the runs stay
-    st = nullptr;
-    TRY(m);
-    // the ends sorted by diagonal, i ascending inside one: keys below 2^32 (segment_key) are the 32 bits of a 16-mer
-    TRY(kmg_build_records(ekey, ei, (int64_t)R0, 16, &ends));
-    dfree(ekey, s); dfree(ei, s);
-    const uint64_t tiles = ceil_div<uint64_t>(R0, SEG_PAIR_TILE);
-    TRY(dalloc(&tmp, (size_t)(3 * R0), s));
-    TRY(dalloc(&status, (size_t)tiles, s));
-    TRY(dalloc(&ticket, 1, s));
-    TRY(dalloc(&tot, 2, s));
-    CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
-    CU(cudaMemsetAsync(ticket, 0, 4, s));
-    LAUNCH("segments_pair", s, segments_pair_kernel<256, SEG_PAIR_ITEMS, ANTI><<<(unsigned)tiles, 256, 0, s>>>(
-                                   starts, R0, ends->ukeys, ends->U, ends->ustart, ends->pos, min_rows, status, ticket, tmp, tot));
-    uint64_t h[2];
-    CU(cudaMemcpyAsync(h, tot, sizeof h, cudaMemcpyDeviceToHost, s));
+  TRY(segments_mark<ANTI>(st, st->idx->pos, starts, ekey, ei, &R0));
+  probe.reset();                                          // the probe is done with: only the runs stay
+  // the ends sorted by diagonal, i ascending inside one: keys below 2^32 (segment_key) are the 32 bits of a 16-mer
+  kmg_index *e = nullptr;
+  TRY(kmg_build_records(ekey, ei, (int64_t)R0, 16, &e));
+  const IndexPtr ends(e);
+  ekey.reset(); ei.reset();
+  const uint64_t tiles = ceil_div<uint64_t>(R0, SEG_PAIR_TILE);
+  DevBuf<int32_t> tmp(s);
+  DevBuf<Pair64> status(s);
+  DevBuf<uint32_t> ticket(s);
+  DevBuf<uint64_t> tot(s);
+  TRY(tmp.alloc((size_t)(3 * R0)));
+  TRY(status.alloc((size_t)tiles));
+  TRY(ticket.alloc(1));
+  TRY(tot.alloc(2));
+  CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
+  CU(cudaMemsetAsync(ticket, 0, 4, s));
+  LAUNCH("segments_pair", s, segments_pair_kernel<256, SEG_PAIR_ITEMS, ANTI><<<(unsigned)tiles, 256, 0, s>>>(
+                                 starts, R0, ends->ukeys, ends->U, ends->ustart, ends->pos, min_rows, status, ticket, tmp, tot));
+  uint64_t h[2];
+  CU(cudaMemcpyAsync(h, tot, sizeof h, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  if (h[1] != M)
+    return fail(KMG_ERR_CUDA, "internal error: the runs hold %llu rows, the probe %llu", (unsigned long long)h[1], (unsigned long long)M);
+  prof_bytes("segments_pair", 8.0 * R0 + 12.0 * R0 + 12.0 * h[0]);   // starts; the diagonal's key and end; the triples
+  DevBuf<int32_t> out(s);
+  if (h[0] == R0) out.reset(tmp.release());
+  else if (h[0]) {                                        // keep exactly the runs that passed min_rows
+    TRY(out.alloc((size_t)(3 * h[0])));
+    CU(cudaMemcpyAsync(out, tmp, 12 * h[0], cudaMemcpyDeviceToDevice, s));
     CU(cudaStreamSynchronize(s));
-    if (h[1] != M)
-      return fail(KMG_ERR_CUDA, "internal error: the runs hold %llu rows, the probe %llu", (unsigned long long)h[1], (unsigned long long)M);
-    prof_bytes("segments_pair", 8.0 * R0 + 12.0 * R0 + 12.0 * h[0]);   // starts; the diagonal's key and end; the triples
-    if (h[0] == R0) { out = tmp; tmp = nullptr; }
-    else if (h[0]) {                                      // keep exactly the runs that passed min_rows
-      TRY(dalloc(&out, (size_t)(3 * h[0]), s));
-      CU(cudaMemcpyAsync(out, tmp, 12 * h[0], cudaMemcpyDeviceToDevice, s));
-      CU(cudaStreamSynchronize(s));
-    }
-    *R = h[0];
-    return KMG_OK;
-  };
-  const int rv = body();
-  if (st) kmg_query_free(st);
+  }
   cudaStreamSynchronize(s);
-  dfree(starts, s); dfree(ekey, s); dfree(ei, s); dfree(tot, s); dfree(ticket, s); dfree(status, s); dfree(tmp, s);
-  if (ends) kmg_free(ends);
-  if (rv != KMG_OK) { dfree(out, s); *R = 0; return rv; }
-  *rows = out;
+  *rows = out.release();
+  *R = h[0];
   return KMG_OK;
 }
 
@@ -1902,71 +1843,66 @@ static int join_probe(const kmg_index *a, const kmg_index *cb, bool rc, uint32_t
   *out = nullptr;
   kmg_index *b = const_cast<kmg_index *>(cb);
   cudaStream_t s = g_ctx.stream();
-  kmg_query *q = new (std::nothrow) kmg_query();
+  QueryPtr q(new (std::nothrow) kmg_query());
   if (!q) return fail(KMG_ERR_NOMEM, "host allocation failed");
   q->idx = b;
-  if (a->U == 0 || b->U == 0) { *out = q; return KMG_OK; }
-  int rv = ensure_hash(b);
-  if (rv != KMG_OK) { delete q; return rv; }
+  if (a->U == 0 || b->U == 0) { *out = q.release(); return KMG_OK; }
+  TRY(ensure_hash(b));
   const uint64_t U = a->U, N = a->N;
-  uint64_t *rkeys = nullptr, *blk = nullptr;
-  uint2 *found = nullptr, *found_pos = nullptr;
-  uint32_t *d_last = nullptr, *ticket = nullptr;
-  QueryStats *qs = nullptr;
-  Pair64 *status = nullptr;
+  const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(U, 256), (uint64_t)g_ctx.sms * 16);
   uint32_t X = 0;                                         // a's largest position: found_pos has one entry per x in [1, X]
-  auto body = [&]() -> int {
-    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(U, 256), (uint64_t)g_ctx.sms * 16);
-    TRY(dalloc(&d_last, 1, s));
-    CU(cudaMemsetAsync(d_last, 0, 4, s));
-    LAUNCH("last_pos", s, last_pos_kernel<<<grid, 256, 0, s>>>(a->ustart, a->pos, U, d_last));
-    CU(cudaMemcpyAsync(&X, d_last, 4, cudaMemcpyDeviceToHost, s));
-    const uint64_t *keys = a->ukeys;
-    if (rc) {
-      TRY(dalloc(&rkeys, (size_t)U, s));
-      LAUNCH("revcomp_keys", s, revcomp_keys_kernel<<<grid, 256, 0, s>>>(a->ukeys, U, a->k, rkeys));
-      keys = rkeys;
-    }
-    TRY(dalloc(&found, (size_t)U, s));
-    const KeyHash kt{b->hash, b->hash_nb, b->hash_hbits};
-    const SeqView sv{};
-    LAUNCH("probe_lookup_rec", s, probe_lookup_kernel<PROBE_THREADS, PROBE_ITEMS, false><<<(unsigned)ceil_div<uint64_t>(U, PROBE_TILE), PROBE_THREADS, 0, s>>>(
-                                      sv, keys, (int64_t)U, nullptr, kt, found));
-    CU(cudaStreamSynchronize(s));
-    dfree(rkeys, s);
-    TRY(dalloc(&found_pos, (size_t)X, s));
-    CU(cudaMemsetAsync(found_pos, 0, (size_t)X * sizeof(uint2), s));
-    TRY(dalloc(&blk, (size_t)ceil_div<uint64_t>(std::min(N, SEG_SLICE_ROWS), EMIT_TILE), s));
-    for (uint64_t first = 0; first < N; first += SEG_SLICE_ROWS) {
-      const uint64_t n = std::min(SEG_SLICE_ROWS, N - first);
-      TRY(block_starts(a->ustart, U, first, n, s, blk));
-      LAUNCH("join_scatter", s, join_scatter_kernel<EMIT_THREADS><<<(unsigned)ceil_div<uint64_t>(n, EMIT_TILE), EMIT_THREADS, 0, s>>>(
-                                    a->ustart, U, a->pos, found, max_count, first, n, blk, found_pos));
-    }
-    const uint64_t tiles = ceil_div<uint64_t>(X, COMPACT_TILE);
-    TRY(dalloc(&q->hit_i, (size_t)X, s));
-    TRY(dalloc(&q->hit_start, (size_t)X, s));
-    TRY(dalloc(&q->row_off, (size_t)X, s));
-    TRY(dalloc(&qs, 1, s));
-    TRY(dalloc(&status, (size_t)tiles, s));
-    TRY(dalloc(&ticket, 1, s));
-    CU(cudaMemsetAsync(qs, 0, sizeof(QueryStats), s));
-    CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
-    CU(cudaMemsetAsync(ticket, 0, 4, s));
-    LAUNCH("probe_compact", s, probe_compact_kernel<PROBE_THREADS, COMPACT_ITEMS, true><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
-                                   found_pos, 1, nullptr, (int64_t)X, nullptr, q->hit_i, q->hit_start, q->row_off, qs, status, ticket,
-                                   max_count));
-    QueryStats h;
-    CU(cudaMemcpyAsync(&h, qs, sizeof h, cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    q->H = h.H; q->M = h.M;
-    return KMG_OK;
-  };
-  rv = body();
+  DevBuf<uint32_t> d_last(s);
+  TRY(d_last.alloc(1));
+  CU(cudaMemsetAsync(d_last, 0, 4, s));
+  LAUNCH("last_pos", s, last_pos_kernel<<<grid, 256, 0, s>>>(a->ustart, a->pos, U, d_last));
+  CU(cudaMemcpyAsync(&X, d_last, 4, cudaMemcpyDeviceToHost, s));
+  const uint64_t *keys = a->ukeys;
+  DevBuf<uint64_t> rkeys(s);
+  if (rc) {
+    TRY(rkeys.alloc((size_t)U));
+    LAUNCH("revcomp_keys", s, revcomp_keys_kernel<<<grid, 256, 0, s>>>(a->ukeys, U, a->k, rkeys));
+    keys = rkeys;
+  }
+  DevBuf<uint2> found(s);
+  TRY(found.alloc((size_t)U));
+  const KeyHash kt{b->hash, b->hash_nb, b->hash_hbits};
+  const SeqView sv{};
+  LAUNCH("probe_lookup_rec", s, probe_lookup_kernel<PROBE_THREADS, PROBE_ITEMS, false><<<(unsigned)ceil_div<uint64_t>(U, PROBE_TILE), PROBE_THREADS, 0, s>>>(
+                                    sv, keys, (int64_t)U, nullptr, kt, found));
+  CU(cudaStreamSynchronize(s));
+  rkeys.reset();
+  DevBuf<uint2> found_pos(s);
+  TRY(found_pos.alloc((size_t)X));
+  CU(cudaMemsetAsync(found_pos, 0, (size_t)X * sizeof(uint2), s));
+  DevBuf<uint64_t> blk(s);
+  TRY(blk.alloc((size_t)ceil_div<uint64_t>(std::min(N, SEG_SLICE_ROWS), EMIT_TILE)));
+  for (uint64_t first = 0; first < N; first += SEG_SLICE_ROWS) {
+    const uint64_t n = std::min(SEG_SLICE_ROWS, N - first);
+    TRY(block_starts(a->ustart, U, first, n, s, blk));
+    LAUNCH("join_scatter", s, join_scatter_kernel<EMIT_THREADS><<<(unsigned)ceil_div<uint64_t>(n, EMIT_TILE), EMIT_THREADS, 0, s>>>(
+                                  a->ustart, U, a->pos, found, max_count, first, n, blk, found_pos));
+  }
+  const uint64_t tiles = ceil_div<uint64_t>(X, COMPACT_TILE);
+  DevBuf<QueryStats> qs(s);
+  DevBuf<Pair64> status(s);
+  DevBuf<uint32_t> ticket(s);
+  TRY(dalloc(&q->hit_i, (size_t)X, s));
+  TRY(dalloc(&q->hit_start, (size_t)X, s));
+  TRY(dalloc(&q->row_off, (size_t)X, s));
+  TRY(qs.alloc(1));
+  TRY(status.alloc((size_t)tiles));
+  TRY(ticket.alloc(1));
+  CU(cudaMemsetAsync(qs, 0, sizeof(QueryStats), s));
+  CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
+  CU(cudaMemsetAsync(ticket, 0, 4, s));
+  LAUNCH("probe_compact", s, probe_compact_kernel<PROBE_THREADS, COMPACT_ITEMS, true><<<(unsigned)tiles, PROBE_THREADS, 0, s>>>(
+                                 found_pos, 1, nullptr, (int64_t)X, nullptr, q->hit_i, q->hit_start, q->row_off, qs, status, ticket,
+                                 max_count));
+  QueryStats h;
+  CU(cudaMemcpyAsync(&h, qs, sizeof h, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  q->H = h.H; q->M = h.M;
   cudaStreamSynchronize(s);
-  dfree(d_last, s); dfree(rkeys, s); dfree(found, s); dfree(blk, s); dfree(found_pos, s);
-  dfree(qs, s); dfree(status, s); dfree(ticket, s);
-  if (rv != KMG_OK) { kmg_query_free(q); return rv; }
   prof_bytes("last_pos", 8.0 * U);
   if (rc) prof_bytes("revcomp_keys", 16.0 * U);
   prof_bytes("probe_lookup_rec", 8.0 * U + 128.0 * U + 8.0 * U);
@@ -1974,7 +1910,7 @@ static int join_probe(const kmg_index *a, const kmg_index *cb, bool rc, uint32_t
   // 32-byte sector of DRAM when it scatters) for a shared k-mer; the memset of found_pos
   prof_bytes("join_scatter", 16.0 * U + 4.0 * N + 32.0 * (double)q->H + 8.0 * X);
   prof_bytes("probe_compact", 8.0 * X + 16.0 * q->H);
-  *out = q;
+  *out = q.release();
   return KMG_OK;
 }
 
@@ -1994,14 +1930,14 @@ extern "C" int kmg_segments_begin(const kmg_index *ix, const char *q, int64_t ql
   *st = nullptr;
   if (!ix) return fail(KMG_ERR_ARG, "index is NULL");
   if (rc != 0 && rc != 1) return fail(KMG_ERR_ARG, "rc must be 0 or 1");
-  kmg_segments *g = new (std::nothrow) kmg_segments();
+  SegmentsPtr g(new (std::nothrow) kmg_segments());
   if (!g) return fail(KMG_ERR_NOMEM, "host allocation failed");
   g->device = ix->device;
   int rv = segments_run(ix, q, qlen, k, rc, max_count, min_rows, &g->rows, &g->R);
   if (rv == KMG_ERR_UNSTABLE) rv = segments_run(ix, q, qlen, k, rc, max_count, min_rows, &g->rows, &g->R);   // the sort now ranks by bitmap
-  if (rv != KMG_OK) { delete g; return rv; }
-  *st = g;
+  TRY(rv);
   if (R) *R = g->R;
+  *st = g.release();
   return KMG_OK;
 }
 
@@ -2014,35 +1950,38 @@ extern "C" int kmg_join_segments_begin(const kmg_index *a, const kmg_index *b, i
   if (a->device != b->device) return fail(KMG_ERR_ARG, "the two indexes live on different devices (%d, %d)", a->device, b->device);
   if (rc && a->k != b->k) return fail(KMG_ERR_K, "the reverse complement needs indexes of one k (here %d and %d)", a->k, b->k);
   TRY(use_index(a));
-  kmg_segments *g = new (std::nothrow) kmg_segments();
+  SegmentsPtr g(new (std::nothrow) kmg_segments());
   if (!g) return fail(KMG_ERR_NOMEM, "host allocation failed");
   g->device = a->device;
   g->anti = rc == 1;
   int rv = join_segments_run(a, b, rc, max_count, min_rows, &g->rows, &g->R);
   if (rv == KMG_ERR_UNSTABLE) rv = join_segments_run(a, b, rc, max_count, min_rows, &g->rows, &g->R);   // the sort now ranks by bitmap
-  if (rv != KMG_OK) { delete g; return rv; }
-  *st = g;
+  TRY(rv);
   if (R) *R = g->R;
+  *st = g.release();
   return KMG_OK;
+}
+
+// Rows [first, first + n) of a finished int32 result of `width` words per row (segments: 3, chains: 6) to out.
+static int emit_int32_rows(const int32_t *rows, int width, uint64_t first, uint64_t n, int32_t *out, const char *name) {
+  if (n == 0) return KMG_OK;
+  if (!out) return fail(KMG_ERR_ARG, "out is NULL");
+  const size_t row_bytes = 4 * (size_t)width;
+  const int sms = g_ctx.sms;
+  int rc = stream_rows(n, row_bytes, out, CHUNK_BYTES / row_bytes, [=](uint64_t f, uint64_t cnt, void *dst, uint64_t *, cudaStream_t s) -> int {
+    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(width * cnt, 256), (uint64_t)sms * 16);
+    LAUNCH(name, s, segments_emit_kernel<<<grid, 256, 0, s>>>(rows + width * (first + f), width * cnt, (int32_t *)dst));
+    return KMG_OK;
+  });
+  prof_bytes(name, 2.0 * row_bytes * n);
+  return rc;
 }
 
 extern "C" int kmg_segments_emit_chunk(kmg_segments *g, uint64_t first, uint64_t n, int32_t *out) {
   if (!g) return fail(KMG_ERR_ARG, "segments handle is NULL");
-  TRY(ctx_init());
-  if (g->device != g_ctx.device)
-    return fail(KMG_ERR_ARG, "the segments live on device %d but this thread works on device %d", g->device, g_ctx.device);
+  TRY(use_device(g->device, "the segments live"));
   if (first > g->R || n > g->R - first) return fail(KMG_ERR_ARG, "runs outside the result");
-  if (n == 0) return KMG_OK;
-  if (!out) return fail(KMG_ERR_ARG, "out is NULL");
-  const int32_t *rows = g->rows;
-  const int sms = g_ctx.sms;
-  int rc = stream_rows(n, 12, out, CHUNK_BYTES / 12, [=](uint64_t f, uint64_t cnt, void *dst, uint64_t *, cudaStream_t s) -> int {
-    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(3 * cnt, 256), (uint64_t)sms * 16);
-    LAUNCH("segments_emit", s, segments_emit_kernel<<<grid, 256, 0, s>>>(rows + 3 * (first + f), 3 * cnt, (int32_t *)dst));
-    return KMG_OK;
-  });
-  prof_bytes("segments_emit", 24.0 * n);
-  return rc;
+  return emit_int32_rows(g->rows, 3, first, n, out, "segments_emit");
 }
 
 extern "C" int kmg_segments_emit(kmg_segments *g, int32_t *out) {
@@ -2052,14 +1991,7 @@ extern "C" int kmg_segments_emit(kmg_segments *g, int32_t *out) {
 
 extern "C" int kmg_segments_free(kmg_segments *g) {
   if (!g) return KMG_OK;
-  int prev = -1;
-  cudaGetDevice(&prev);
-  cudaSetDevice(g->device);
-  const bool mine = g_ctx.ready && g_ctx.device == g->device;
-  if (mine) cudaStreamSynchronize(g_ctx.stream()); else cudaDeviceSynchronize();
-  if (g->rows) g_arena[g->device & 63].put(g->rows, nullptr, true);
-  cudaGetLastError();
-  if (prev >= 0) cudaSetDevice(prev);
+  release_on_device(g->device, {g->rows});
   delete g;
   return KMG_OK;
 }
@@ -2083,93 +2015,92 @@ static int chains_of(const int32_t *runs, uint64_t R, uint32_t G, uint32_t W, ui
   *C = 0;
   if (R == 0) return KMG_OK;
   cudaStream_t s = g_ctx.stream();
-  uint64_t *key = nullptr, *tot = nullptr;
-  uint32_t *run = nullptr, *si = nullptr, *sI = nullptr, *flag = nullptr, *ticket = nullptr;
-  int32_t *succ = nullptr, *pred = nullptr, *head = nullptr, *tmp = nullptr, *out = nullptr;
-  unsigned long long *nsum = nullptr, *nm = nullptr, *last = nullptr;
-  Pair64 *status = nullptr;
-  kmg_index *diag = nullptr;
+  const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(R, 256), (uint64_t)g_ctx.sms * 16);
+  DevBuf<uint64_t> key(s);
+  DevBuf<uint32_t> run(s);
+  TRY(key.alloc((size_t)R));
+  TRY(run.alloc((size_t)R));
+  LAUNCH("chains_keys", s, chains_keys_kernel<ANTI><<<grid, 256, 0, s>>>(runs, R, key, run));
+  // the runs by diagonal, i ascending inside one (stable): keys below 2^32 (segment_key) are the 32 bits of a 16-mer
+  kmg_index *d = nullptr;
+  TRY(kmg_build_records(key, run, (int64_t)R, 16, &d));
+  IndexPtr diag(d);
+  key.reset(); run.reset();
+  DevBuf<uint32_t> si(s), sI(s);
+  TRY(si.alloc((size_t)R));
+  TRY(sI.alloc((size_t)R));
+  LAUNCH("chains_gather", s, chains_gather_kernel<<<grid, 256, 0, s>>>(runs, diag->pos, R, si, sI));
+  DevBuf<int32_t> succ(s), pred(s);
+  DevBuf<unsigned long long> nsum(s);
+  TRY(succ.alloc((size_t)R));
+  TRY(pred.alloc((size_t)R));
+  TRY(nsum.alloc(1));
+  CU(cudaMemsetAsync(nsum, 0, 8, s));
+  LAUNCH("chains_link", s, chains_link_kernel<ANTI><<<(unsigned)ceil_div<uint64_t>(R, 256), 256, 0, s>>>(
+                               runs, R, diag->ukeys, diag->U, diag->ustart, diag->pos, si, sI, G, W, succ, pred, nsum));
+  const uint64_t U = diag->U;
+  diag.reset();
+  si.reset(); sI.reset();
+  DevBuf<int32_t> head(s);
+  TRY(head.alloc((size_t)R));
+  LAUNCH("chains_heads", s, chains_heads_kernel<<<grid, 256, 0, s>>>(succ, pred, R, head));
+  succ.reset(); pred.reset();
+  // the first run of every chain by pointer jumping: a round that moves no pointer ends it
+  DevBuf<uint32_t> flag(s);
+  TRY(flag.alloc(1));
   int rounds = 0;
-  auto body = [&]() -> int {
-    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(R, 256), (uint64_t)g_ctx.sms * 16);
-    TRY(dalloc(&key, (size_t)R, s));
-    TRY(dalloc(&run, (size_t)R, s));
-    LAUNCH("chains_keys", s, chains_keys_kernel<ANTI><<<grid, 256, 0, s>>>(runs, R, key, run));
-    // the runs by diagonal, i ascending inside one (stable): keys below 2^32 (segment_key) are the 32 bits of a 16-mer
-    TRY(kmg_build_records(key, run, (int64_t)R, 16, &diag));
-    dfree(key, s); dfree(run, s);
-    TRY(dalloc(&si, (size_t)R, s));
-    TRY(dalloc(&sI, (size_t)R, s));
-    LAUNCH("chains_gather", s, chains_gather_kernel<<<grid, 256, 0, s>>>(runs, diag->pos, R, si, sI));
-    TRY(dalloc(&succ, (size_t)R, s));
-    TRY(dalloc(&pred, (size_t)R, s));
-    TRY(dalloc(&nsum, 1, s));
-    CU(cudaMemsetAsync(nsum, 0, 8, s));
-    LAUNCH("chains_link", s, chains_link_kernel<ANTI><<<(unsigned)ceil_div<uint64_t>(R, 256), 256, 0, s>>>(
-                                 runs, R, diag->ukeys, diag->U, diag->ustart, diag->pos, si, sI, G, W, succ, pred, nsum));
-    const uint64_t U = diag->U;
-    kmg_free(diag);
-    diag = nullptr;
-    dfree(si, s); dfree(sI, s);
-    TRY(dalloc(&head, (size_t)R, s));
-    LAUNCH("chains_heads", s, chains_heads_kernel<<<grid, 256, 0, s>>>(succ, pred, R, head));
-    dfree(succ, s); dfree(pred, s);
-    // the first run of every chain by pointer jumping: a round that moves no pointer ends it
-    TRY(dalloc(&flag, 1, s));
-    for (uint32_t moved = 1; moved;) {
-      if (++rounds > CHAIN_MAX_ROUNDS) return fail(KMG_ERR_CUDA, "internal error: pointer jumping did not settle in %d rounds", CHAIN_MAX_ROUNDS);
-      CU(cudaMemsetAsync(flag, 0, 4, s));
-      LAUNCH("chains_jump", s, chains_jump_kernel<<<grid, 256, 0, s>>>(head, R, flag));
-      CU(cudaMemcpyAsync(&moved, flag, 4, cudaMemcpyDeviceToHost, s));
-      CU(cudaStreamSynchronize(s));
-    }
-    TRY(dalloc(&nm, (size_t)R, s));
-    TRY(dalloc(&last, (size_t)R, s));
-    CU(cudaMemsetAsync(nm, 0, R * 8, s));
-    CU(cudaMemsetAsync(last, 0, R * 8, s));
-    LAUNCH("chains_aggregate", s, chains_aggregate_kernel<ANTI><<<grid, 256, 0, s>>>(runs, head, R, nm, last));
-    const uint64_t tiles = ceil_div<uint64_t>(R, CHAIN_COMPACT_TILE);
-    TRY(dalloc(&tmp, (size_t)(6 * R), s));
-    TRY(dalloc(&status, (size_t)tiles, s));
-    TRY(dalloc(&ticket, 1, s));
-    TRY(dalloc(&tot, 3, s));
-    CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
-    CU(cudaMemsetAsync(ticket, 0, 4, s));
-    LAUNCH("chains_compact", s, chains_compact_kernel<256, CHAIN_COMPACT_ITEMS, ANTI><<<(unsigned)tiles, 256, 0, s>>>(
-                                    runs, head, nm, last, R, min_rows, status, ticket, tmp, tot));
-    uint64_t h[3], n_runs = 0;
-    CU(cudaMemcpyAsync(h, tot, sizeof h, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(&n_runs, nsum, 8, cudaMemcpyDeviceToHost, s));
+  for (uint32_t moved = 1; moved;) {
+    if (++rounds > CHAIN_MAX_ROUNDS) return fail(KMG_ERR_CUDA, "internal error: pointer jumping did not settle in %d rounds", CHAIN_MAX_ROUNDS);
+    CU(cudaMemsetAsync(flag, 0, 4, s));
+    LAUNCH("chains_jump", s, chains_jump_kernel<<<grid, 256, 0, s>>>(head, R, flag));
+    CU(cudaMemcpyAsync(&moved, flag, 4, cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
-    if (h[1] != R || h[2] != n_runs)
-      return fail(KMG_ERR_CUDA, "internal error: the chains hold %llu runs of %llu rows, the handle %llu runs of %llu rows",
-                  (unsigned long long)h[1], (unsigned long long)h[2], (unsigned long long)R, (unsigned long long)n_runs);
-    // runs (12 B) and their keys (8 B); the gathered i and I; the link search (the runs, one lower bound over the U
-    // diagonal keys and the candidates' i / I, counted as 64 B per run); head, aggregates, the rows written
-    prof_bytes("chains_keys", 24.0 * R);
-    prof_bytes("chains_gather", 24.0 * R);
-    prof_bytes("chains_link", 12.0 * R + 8.0 * U + 64.0 * R + 8.0 * R);
-    prof_bytes("chains_heads", 16.0 * R);
-    prof_bytes("chains_jump", 8.0 * R * rounds);
-    prof_bytes("chains_aggregate", 16.0 * R + 16.0 * (R - h[0]));
-    prof_bytes("chains_compact", 16.0 * R + 24.0 * h[0]);
-    if (h[0] == R) { out = tmp; tmp = nullptr; }
-    else if (h[0]) {                                      // keep exactly the chains that passed min_rows
-      TRY(dalloc(&out, (size_t)(6 * h[0]), s));
-      CU(cudaMemcpyAsync(out, tmp, 24 * h[0], cudaMemcpyDeviceToDevice, s));
-      CU(cudaStreamSynchronize(s));
-    }
-    *C = h[0];
-    return KMG_OK;
-  };
-  const int rv = body();
+  }
+  DevBuf<unsigned long long> nm(s), last(s);
+  TRY(nm.alloc((size_t)R));
+  TRY(last.alloc((size_t)R));
+  CU(cudaMemsetAsync(nm, 0, R * 8, s));
+  CU(cudaMemsetAsync(last, 0, R * 8, s));
+  LAUNCH("chains_aggregate", s, chains_aggregate_kernel<ANTI><<<grid, 256, 0, s>>>(runs, head, R, nm, last));
+  const uint64_t tiles = ceil_div<uint64_t>(R, CHAIN_COMPACT_TILE);
+  DevBuf<int32_t> tmp(s);
+  DevBuf<Pair64> status(s);
+  DevBuf<uint32_t> ticket(s);
+  DevBuf<uint64_t> tot(s);
+  TRY(tmp.alloc((size_t)(6 * R)));
+  TRY(status.alloc((size_t)tiles));
+  TRY(ticket.alloc(1));
+  TRY(tot.alloc(3));
+  CU(cudaMemsetAsync(status, 0, tiles * sizeof(Pair64), s));
+  CU(cudaMemsetAsync(ticket, 0, 4, s));
+  LAUNCH("chains_compact", s, chains_compact_kernel<256, CHAIN_COMPACT_ITEMS, ANTI><<<(unsigned)tiles, 256, 0, s>>>(
+                                  runs, head, nm, last, R, min_rows, status, ticket, tmp, tot));
+  uint64_t h[3], n_runs = 0;
+  CU(cudaMemcpyAsync(h, tot, sizeof h, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(&n_runs, nsum, 8, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  if (h[1] != R || h[2] != n_runs)
+    return fail(KMG_ERR_CUDA, "internal error: the chains hold %llu runs of %llu rows, the handle %llu runs of %llu rows",
+                (unsigned long long)h[1], (unsigned long long)h[2], (unsigned long long)R, (unsigned long long)n_runs);
+  // runs (12 B) and their keys (8 B); the gathered i and I; the link search (the runs, one lower bound over the U
+  // diagonal keys and the candidates' i / I, counted as 64 B per run); head, aggregates, the rows written
+  prof_bytes("chains_keys", 24.0 * R);
+  prof_bytes("chains_gather", 24.0 * R);
+  prof_bytes("chains_link", 12.0 * R + 8.0 * U + 64.0 * R + 8.0 * R);
+  prof_bytes("chains_heads", 16.0 * R);
+  prof_bytes("chains_jump", 8.0 * R * rounds);
+  prof_bytes("chains_aggregate", 16.0 * R + 16.0 * (R - h[0]));
+  prof_bytes("chains_compact", 16.0 * R + 24.0 * h[0]);
+  DevBuf<int32_t> out(s);
+  if (h[0] == R) out.reset(tmp.release());
+  else if (h[0]) {                                        // keep exactly the chains that passed min_rows
+    TRY(out.alloc((size_t)(6 * h[0])));
+    CU(cudaMemcpyAsync(out, tmp, 24 * h[0], cudaMemcpyDeviceToDevice, s));
+    CU(cudaStreamSynchronize(s));
+  }
   cudaStreamSynchronize(s);
-  dfree(key, s); dfree(run, s); dfree(si, s); dfree(sI, s); dfree(succ, s); dfree(pred, s); dfree(head, s);
-  dfree(nsum, s); dfree(flag, s); dfree(nm, s); dfree(last, s); dfree(tmp, s); dfree(status, s); dfree(ticket, s);
-  dfree(tot, s);
-  if (diag) kmg_free(diag);
-  if (rv != KMG_OK) { dfree(out, s); *C = 0; return rv; }
-  *rows = out;
+  *rows = out.release();
+  *C = h[0];
   return KMG_OK;
 }
 
@@ -2181,10 +2112,8 @@ extern "C" int kmg_chains_begin(const kmg_segments *seg, uint32_t max_gap, uint3
   if (max_gap > (uint32_t)INT32_MAX) return fail(KMG_ERR_ARG, "max_gap must be below 2^31");
   if (max_shift > max_gap) return fail(KMG_ERR_ARG, "max_shift (%u) must not exceed max_gap (%u)", max_shift, max_gap);
   if (max_shift > 1024) return fail(KMG_ERR_ARG, "max_shift must be at most 1024");
-  TRY(ctx_init());
-  if (seg->device != g_ctx.device)
-    return fail(KMG_ERR_ARG, "the segments live on device %d but this thread works on device %d", seg->device, g_ctx.device);
-  kmg_chains *g = new (std::nothrow) kmg_chains();
+  TRY(use_device(seg->device, "the segments live"));
+  ChainsPtr g(new (std::nothrow) kmg_chains());
   if (!g) return fail(KMG_ERR_NOMEM, "host allocation failed");
   g->device = seg->device;
   auto run = [&]() {
@@ -2193,29 +2122,17 @@ extern "C" int kmg_chains_begin(const kmg_segments *seg, uint32_t max_gap, uint3
   };
   int rv = run();
   if (rv == KMG_ERR_UNSTABLE) rv = run();                 // the sort now ranks by bitmap
-  if (rv != KMG_OK) { delete g; return rv; }
-  *st = g;
+  TRY(rv);
   if (C) *C = g->C;
+  *st = g.release();
   return KMG_OK;
 }
 
 extern "C" int kmg_chains_emit_chunk(kmg_chains *g, uint64_t first, uint64_t n, int32_t *out) {
   if (!g) return fail(KMG_ERR_ARG, "chains handle is NULL");
-  TRY(ctx_init());
-  if (g->device != g_ctx.device)
-    return fail(KMG_ERR_ARG, "the chains live on device %d but this thread works on device %d", g->device, g_ctx.device);
+  TRY(use_device(g->device, "the chains live"));
   if (first > g->C || n > g->C - first) return fail(KMG_ERR_ARG, "chains outside the result");
-  if (n == 0) return KMG_OK;
-  if (!out) return fail(KMG_ERR_ARG, "out is NULL");
-  const int32_t *rows = g->rows;
-  const int sms = g_ctx.sms;
-  int rc = stream_rows(n, 24, out, CHUNK_BYTES / 24, [=](uint64_t f, uint64_t cnt, void *dst, uint64_t *, cudaStream_t s) -> int {
-    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(6 * cnt, 256), (uint64_t)sms * 16);
-    LAUNCH("chains_emit", s, segments_emit_kernel<<<grid, 256, 0, s>>>(rows + 6 * (first + f), 6 * cnt, (int32_t *)dst));
-    return KMG_OK;
-  });
-  prof_bytes("chains_emit", 48.0 * n);
-  return rc;
+  return emit_int32_rows(g->rows, 6, first, n, out, "chains_emit");
 }
 
 extern "C" int kmg_chains_emit(kmg_chains *g, int32_t *out) {
@@ -2225,14 +2142,7 @@ extern "C" int kmg_chains_emit(kmg_chains *g, int32_t *out) {
 
 extern "C" int kmg_chains_free(kmg_chains *g) {
   if (!g) return KMG_OK;
-  int prev = -1;
-  cudaGetDevice(&prev);
-  cudaSetDevice(g->device);
-  const bool mine = g_ctx.ready && g_ctx.device == g->device;
-  if (mine) cudaStreamSynchronize(g_ctx.stream()); else cudaDeviceSynchronize();
-  if (g->rows) g_arena[g->device & 63].put(g->rows, nullptr, true);
-  cudaGetLastError();
-  if (prev >= 0) cudaSetDevice(prev);
+  release_on_device(g->device, {g->rows});
   delete g;
   return KMG_OK;
 }
@@ -2242,23 +2152,20 @@ extern "C" int kmg_chains_free(kmg_chains *g) {
 // ------------------------------------------------------------------------------------------------
 // The caller's shard [g0,g1) is copied into an aligned, padded buffer whose byte 16 is window start s0.
 static int shard_view(const void *d_seq, int64_t g0, int64_t g1, int64_t L, int64_t s0, int64_t s1, int k,
-                      cudaStream_t s, DevSeq *ds, SeqView *sv) {
+                      cudaStream_t s, DevBuf<uint8_t> &buf, SeqView *sv) {
   if (k < 1 || k > KMG_MAX_K) return fail(KMG_ERR_K, "k must be in [1,32]");
   if (!(0 <= g0 && g0 <= g1 && g1 <= L && 0 <= s0 && s0 <= s1)) return fail(KMG_ERR_ARG, "inconsistent shard bounds");
   const int64_t need_lo = s0 > 0 ? s0 - 1 : 0, need_hi = std::min<int64_t>(L, s1 + k - 1);
   if (s1 > s0 && (g0 > need_lo || g1 < need_hi)) return fail(KMG_ERR_ARG, "shard bytes [%lld,%lld) do not cover [%lld,%lld)", (long long)g0, (long long)g1, (long long)need_lo, (long long)need_hi);
   const int64_t avail = std::max<int64_t>(0, need_hi - s0);
-  size_t cap = 16 + (size_t)((avail + 15) / 16) * 16 + 16;
-  TRY(dalloc(&ds->buf, cap, s));
-  ds->base = ds->buf + 16;
-  CU(cudaMemsetAsync(ds->buf, 0, 16, s));
-  CU(cudaMemsetAsync(ds->buf + cap - 32, 0, 32, s));
+  TRY(seq_alloc(buf, avail, s));
+  uint8_t *base = buf + 16;
   if (avail > 0) {
     const int64_t lead = s0 > 0 ? 1 : 0;        // one byte of left context for rule (iii)
-    CU(cudaMemcpyAsync(ds->base - lead, (const uint8_t *)d_seq + (s0 - lead - g0), (size_t)(avail + lead), cudaMemcpyDefault, s));
+    CU(cudaMemcpyAsync(base - lead, (const uint8_t *)d_seq + (s0 - lead - g0), (size_t)(avail + lead), cudaMemcpyDefault, s));
   }
   int64_t nstarts = std::min<int64_t>(s1, L - k + 1) - s0;
-  sv->base = ds->base; sv->nstarts = nstarts > 0 ? nstarts : 0; sv->avail = avail; sv->s0 = s0; sv->L = L; sv->k = k;
+  sv->base = base; sv->nstarts = nstarts > 0 ? nstarts : 0; sv->avail = avail; sv->s0 = s0; sv->L = L; sv->k = k;
   return KMG_OK;
 }
 
@@ -2280,11 +2187,40 @@ extern "C" int kmg_shard_sample(const void *d_seq, int64_t g0, int64_t g1, int64
   if (n <= 0 || !d_samples) return fail(KMG_ERR_ARG, "bad sample request");
   TRY(ctx_init());
   cudaStream_t s = g_ctx.stream();
-  DevSeq ds; SeqView sv;
-  TRY(shard_view(d_seq, g0, g1, L, s0, s1, k, s, &ds, &sv));
+  DevBuf<uint8_t> buf(s);
+  SeqView sv;
+  TRY(shard_view(d_seq, g0, g1, L, s0, s1, k, s, buf, &sv));
   LAUNCH("sample", s, sample_kernel<<<ceil_div(n, 256), 256, 0, s>>>(sv, n, d_samples));
   CU(cudaStreamSynchronize(s));
-  dfree(ds.buf, s);
+  return KMG_OK;
+}
+
+// The records of the shard sv, grouped by owner (nparts - 1 splitters), into (d_keys, d_pos); counts[i]: owner i's records
+static int partition_records(const SeqView &sv, const uint64_t *splitters, int nparts, uint64_t *d_keys, uint32_t *d_pos, uint64_t *counts,
+                             cudaStream_t s) {
+  SortScratch sc(s);
+  DevBuf<uint64_t> d_spl(s);
+  TRY(scratch_alloc(sc, sv.nstarts, s));
+  TRY(d_spl.alloc((size_t)RADIX));
+  if (nparts > 1) CU(cudaMemcpyAsync(d_spl, splitters, (size_t)(nparts - 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+  OwnerBin ob{d_spl, nparts};
+  const int64_t tiles = ceil_div<int64_t>(sv.nstarts, HIST_TILE);
+  const unsigned hgrid = (unsigned)std::min<int64_t>(tiles, (int64_t)g_ctx.sms * 2);
+  LAUNCH("hist_seq_owner", s, hist_seq_kernel<HIST_THREADS, HIST_ITEMS, OwnerBin><<<hgrid, HIST_THREADS, 0, s>>>(sv, sc.hist(0), ob));
+  TRY(launch_scan_hist(RADIX_BITS, s, sc.hist(0), sc.gbase(0), (uint64_t *)nullptr));
+  PassParams<OwnerBin, NoBin> P{};
+  P.sv = sv; P.keys_out = d_keys; P.pos_out = d_pos;
+  P.gbase = sc.gbase(0); P.hist_next = nullptr;
+  P.status = sc.status; P.ticket = sc.ticket(0); P.epoch = 1;
+  P.bin = ob;
+  TRY((launch_pass<true, OwnerBin, NoBin, false>("partition", P, sv.nstarts, s)));
+  std::vector<uint32_t> h(RADIX);
+  CU(cudaMemcpyAsync(h.data(), sc.hist(0), RADIX * 4, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  double tot = 0;
+  for (int i = 0; i < nparts; ++i) { counts[i] = h[i]; tot += h[i]; }
+  prof_bytes("hist_seq_owner", (double)sv.avail);
+  prof_bytes("partition", (double)sv.avail + 12.0 * tot);
   return KMG_OK;
 }
 
@@ -2294,42 +2230,15 @@ extern "C" int kmg_shard_partition(const void *d_seq, int64_t g0, int64_t g1, in
   if (nparts > 1 && !splitters) return fail(KMG_ERR_ARG, "splitters is NULL");
   TRY(ctx_init());
   cudaStream_t s = g_ctx.stream();
-  DevSeq ds; SeqView sv;
-  TRY(shard_view(d_seq, g0, g1, L, s0, s1, k, s, &ds, &sv));
+  DevBuf<uint8_t> buf(s);
+  SeqView sv;
+  TRY(shard_view(d_seq, g0, g1, L, s0, s1, k, s, buf, &sv));
   for (int i = 0; i < nparts; ++i) counts[i] = 0;
-  if (sv.nstarts == 0) { dfree(ds.buf, s); return KMG_OK; }
-  if (!d_keys || !d_pos) { dfree(ds.buf, s); return fail(KMG_ERR_ARG, "record arrays are NULL"); }
-  if (s0 + sv.nstarts > (int64_t)INT32_MAX) { dfree(ds.buf, s); return fail(KMG_ERR_RANGE, "positions exceed int"); }
-  SortScratch sc;
-  uint64_t *d_spl = nullptr;
-  auto body = [&]() -> int {
-    TRY(scratch_alloc(sc, sv.nstarts, s));
-    TRY(dalloc(&d_spl, (size_t)RADIX, s));
-    if (nparts > 1) CU(cudaMemcpyAsync(d_spl, splitters, (size_t)(nparts - 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    OwnerBin ob{d_spl, nparts};
-    const int64_t tiles = ceil_div<int64_t>(sv.nstarts, HIST_TILE);
-    const unsigned hgrid = (unsigned)std::min<int64_t>(tiles, (int64_t)g_ctx.sms * 2);
-    LAUNCH("hist_seq_owner", s, hist_seq_kernel<HIST_THREADS, HIST_ITEMS, OwnerBin><<<hgrid, HIST_THREADS, 0, s>>>(sv, sc.hist(0), ob));
-    TRY(launch_scan_hist(RADIX_BITS, s, sc.hist(0), sc.gbase(0), (uint64_t *)nullptr));
-    PassParams<OwnerBin, NoBin> P{};
-    P.sv = sv; P.keys_out = d_keys; P.pos_out = d_pos;
-    P.gbase = sc.gbase(0); P.hist_next = nullptr;
-    P.status = sc.status; P.ticket = sc.ticket(0); P.epoch = 1;
-    P.bin = ob;
-    TRY((launch_pass<true, OwnerBin, NoBin, false>("partition", P, sv.nstarts, s)));
-    std::vector<uint32_t> h(RADIX);
-    CU(cudaMemcpyAsync(h.data(), sc.hist(0), RADIX * 4, cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    double tot = 0;
-    for (int i = 0; i < nparts; ++i) { counts[i] = h[i]; tot += h[i]; }
-    prof_bytes("hist_seq_owner", (double)sv.avail);
-    prof_bytes("partition", (double)sv.avail + 12.0 * tot);
-    return KMG_OK;
-  };
-  int rc = body();
-  dfree(d_spl, s); dfree(ds.buf, s);
-  scratch_free(sc, s);
-  if (rc != KMG_OK) cudaStreamSynchronize(s);
+  if (sv.nstarts == 0) return KMG_OK;
+  if (!d_keys || !d_pos) return fail(KMG_ERR_ARG, "record arrays are NULL");
+  if (s0 + sv.nstarts > (int64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "positions exceed int");
+  const int rc = partition_records(sv, splitters, nparts, d_keys, d_pos, counts, s);
+  if (rc != KMG_OK) cudaStreamSynchronize(s);             // nothing may still write the caller's arrays
   return rc;
 }
 
@@ -2341,49 +2250,38 @@ extern "C" int kmg_build_records(uint64_t *d_keys, uint32_t *d_pos, int64_t n, i
   if (n > (int64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "too many records");
   TRY(ctx_init());
   cudaStream_t s = g_ctx.stream();
-  kmg_index *ix = new (std::nothrow) kmg_index();
+  IndexPtr ix(new (std::nothrow) kmg_index());
   if (!ix) return fail(KMG_ERR_NOMEM, "host allocation failed");
   ix->device = g_ctx.device;
   ix->k = k;
   if (n == 0) {
-    int rc = dalloc(&ix->ustart, 1, s);
-    if (rc == KMG_OK) cudaMemsetAsync(ix->ustart, 0, 4, s);
+    TRY(dalloc(&ix->ustart, 1, s));
+    cudaMemsetAsync(ix->ustart, 0, 4, s);
     cudaStreamSynchronize(s);
-    if (rc != KMG_OK) { delete ix; return rc; }
-    *out = ix;
+    *out = ix.release();
     return KMG_OK;
   }
-  SortScratch sc;
-  uint64_t *ka = d_keys, *kb = nullptr;
-  uint32_t *pa = d_pos, *pb = nullptr, *pfinal = nullptr;
-  auto body = [&]() -> int {
-    TRY(scratch_alloc(sc, n, s));
-    TRY(dalloc(&kb, (size_t)n, s));
-    TRY(dalloc(&pb, (size_t)n, s));
-    const unsigned hgrid = (unsigned)std::min<int64_t>(ceil_div<int64_t>(n, 256 * 16), (int64_t)g_ctx.sms * 8);
-    LAUNCH("hist_rec", s, hist_rec_kernel<256, DigitBin><<<hgrid, 256, 0, s>>>(d_keys, n, nullptr, sc.hist(0), DigitBin{0}));
-    TRY(launch_scan_hist(RADIX_BITS, s, sc.hist(0), sc.gbase(0), &sc.stats()->n));
-    TRY(dalloc(&pfinal, (size_t)n, s));                    // the index must own its positions
-    TRY(sort_tail(sc, SortPlan{RADIX_BITS, num_passes(k)}, 0, true, ka, pa, kb, pb, n, s, pfinal));      // keys end in ka (may be the caller's array)
-    TRY(finish_index(ix, sc, ka, pfinal, n, s));
-    pfinal = nullptr;
-    if (ix->unstable) { demote_rank_variant(); return fail(KMG_ERR_UNSTABLE, "position lists not ascending after the one-atomic sort pass; rebuild (the bitmap variant is now selected)"); }
-    const int R = num_passes(k);
-    prof_bytes("hist_rec", 8.0 * n);
-    if (R > 1) prof_bytes("sort_pass_hist", 24.0 * n * (R - 1));
-    prof_bytes("sort_pass", 24.0 * n);
-    return KMG_OK;
-  };
-  int rc = body();
-  // free whichever of the ping-pong buffers are ours
-  if (ka != d_keys) dfree(ka, s);
-  if (kb != d_keys) dfree(kb, s);
-  if (pa != d_pos) dfree(pa, s);
-  if (pb != d_pos) dfree(pb, s);
-  dfree(pfinal, s);
-  scratch_free(sc, s);
-  if (rc != KMG_OK) { cudaStreamSynchronize(s); kmg_free(ix); return rc; }
-  *out = ix;
+  SortScratch sc(s);
+  DevBuf<uint64_t> kbuf(s);
+  DevBuf<uint32_t> pbuf(s), pfinal(s);
+  TRY(scratch_alloc(sc, n, s));
+  TRY(kbuf.alloc((size_t)n));
+  TRY(pbuf.alloc((size_t)n));
+  uint64_t *ka = d_keys, *kb = kbuf;                       // the passes ping-pong between the caller's arrays and ours
+  uint32_t *pa = d_pos, *pb = pbuf;
+  const unsigned hgrid = (unsigned)std::min<int64_t>(ceil_div<int64_t>(n, 256 * 16), (int64_t)g_ctx.sms * 8);
+  LAUNCH("hist_rec", s, hist_rec_kernel<256, DigitBin><<<hgrid, 256, 0, s>>>(d_keys, n, nullptr, sc.hist(0), DigitBin{0}));
+  TRY(launch_scan_hist(RADIX_BITS, s, sc.hist(0), sc.gbase(0), &sc.stats()->n));
+  TRY(pfinal.alloc((size_t)n));                            // the index must own its positions
+  TRY(sort_tail(sc, SortPlan{RADIX_BITS, num_passes(k)}, 0, true, ka, pa, kb, pb, n, s, pfinal));      // keys end in ka (may be the caller's array)
+  TRY(finish_index(ix.get(), sc, ka, pfinal, n, s));
+  pfinal.release();
+  if (ix->unstable) { demote_rank_variant(); return fail(KMG_ERR_UNSTABLE, "position lists not ascending after the one-atomic sort pass; rebuild (the bitmap variant is now selected)"); }
+  const int R = num_passes(k);
+  prof_bytes("hist_rec", 8.0 * n);
+  if (R > 1) prof_bytes("sort_pass_hist", 24.0 * n * (R - 1));
+  prof_bytes("sort_pass", 24.0 * n);
+  *out = ix.release();
   return KMG_OK;
 }
 
@@ -2394,27 +2292,33 @@ extern "C" int kmg_build_records(uint64_t *d_keys, uint32_t *d_pos, int64_t n, i
 struct kmg_shard {
   int device = 0;
   bool hashed = false;     // grouped sharded build: records and owner ranges are those of mix64(key)
-  DevSeq ds;
+  uint8_t *buf = nullptr;  // the shard's bytes (seq_alloc): sv.base = buf + 16
   SeqView sv;
 };
+static kmg_shard *new_shard(DevBuf<uint8_t> &buf, const SeqView &sv, bool hashed) {
+  kmg_shard *sh = new (std::nothrow) kmg_shard();
+  if (!sh) return nullptr;
+  sh->device = g_ctx.device; sh->hashed = hashed; sh->sv = sv; sh->buf = buf.release();
+  return sh;
+}
 
 extern "C" int kmg_shard_open(const void *d_seq, int64_t g0, int64_t g1, int64_t L, int64_t s0, int64_t s1, int k, kmg_shard **out) {
   if (!out) return fail(KMG_ERR_ARG, "out is NULL");
   *out = nullptr;
   TRY(ctx_init());
-  kmg_shard *sh = new (std::nothrow) kmg_shard();
-  if (!sh) return fail(KMG_ERR_NOMEM, "host allocation failed");
-  sh->device = g_ctx.device;
-  int rc = shard_view(d_seq, g0, g1, L, s0, s1, k, g_ctx.stream(), &sh->ds, &sh->sv);
-  if (rc != KMG_OK) { delete sh; return rc; }
-  if (s0 + sh->sv.nstarts > (int64_t)INT32_MAX) { kmg_shard_close(sh); return fail(KMG_ERR_RANGE, "positions exceed int"); }
-  *out = sh;
+  DevBuf<uint8_t> buf(g_ctx.stream());
+  SeqView sv;
+  TRY(shard_view(d_seq, g0, g1, L, s0, s1, k, g_ctx.stream(), buf, &sv));
+  if (s0 + sv.nstarts > (int64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "positions exceed int");
+  if (!(*out = new_shard(buf, sv, false))) return fail(KMG_ERR_NOMEM, "host allocation failed");
   return KMG_OK;
 }
 extern "C" int kmg_shard_close(kmg_shard *sh) {
   if (!sh) return KMG_OK;
-  if (g_ctx.ready && g_ctx.device == sh->device) dfree(sh->ds.buf, g_ctx.stream());
-  else { cudaSetDevice(sh->device); g_arena[sh->device & 63].put(sh->ds.buf, nullptr, false); }
+  // no synchronisation: the sharded calls never wait for the device
+  const bool mine = g_ctx.ready && g_ctx.device == sh->device;
+  if (!mine) cudaSetDevice(sh->device);
+  g_arena[sh->device & 63].put(sh->buf, mine ? g_ctx.stream() : nullptr, false);
   delete sh;
   return KMG_OK;
 }
@@ -2447,8 +2351,8 @@ extern "C" int kmg_shard_count(const kmg_shard *sh, const uint64_t *d_splitters,
   if (nparts > 1 && !d_splitters) return fail(KMG_ERR_ARG, "splitters is NULL");
   TRY(ctx_init());
   cudaStream_t s = g_ctx.stream();
-  uint32_t *hist = nullptr;
-  TRY(dalloc(&hist, (size_t)RADIX, s));
+  DevBuf<uint32_t> hist(s);
+  TRY(hist.alloc((size_t)RADIX));
   CU(cudaMemsetAsync(hist, 0, RADIX * 4, s));
   if (sh->sv.nstarts > 0) {
     OwnerBin ob{d_splitters, nparts};
@@ -2461,7 +2365,6 @@ extern "C" int kmg_shard_count(const kmg_shard *sh, const uint64_t *d_splitters,
     prof_bytes("hist_seq_owner", (double)sh->sv.avail);
   }
   LAUNCH("widen_counts", s, widen_counts_kernel<<<1, MAX_PEERS, 0, s>>>(hist, nparts, d_counts));
-  dfree(hist, s);
   return KMG_OK;
 }
 
@@ -2474,33 +2377,27 @@ extern "C" int kmg_shard_scatter(const kmg_shard *sh, const uint64_t *d_splitter
   if (capacity > (uint64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "capacity exceeds int coordinates");
   TRY(ctx_init());
   cudaStream_t s = g_ctx.stream();
-  SortScratch sc;
-  PeerTable *tab = nullptr;
-  auto body = [&]() -> int {
-    TRY(scratch_alloc(sc, sh->sv.nstarts, s));
-    TRY(dalloc(&tab, 1, s));
-    PeerPtrs pp{};
-    for (int i = 0; i < nparts; ++i) { pp.keys[i] = (uint64_t *)peer_keys[i]; pp.pos[i] = (uint32_t *)peer_pos[i]; }
-    LAUNCH("owner_offsets", s, owner_offsets_kernel<<<1, RADIX, 0, s>>>(d_matrix, nparts, rank, capacity, pp, sc.gbase(0), tab, d_info));
-    if (sh->sv.nstarts == 0) return KMG_OK;
-    OwnerBin ob{d_splitters, nparts};
-    PassParams<OwnerBin, NoBin> P{};
-    P.sv = sh->sv;
-    P.gbase = sc.gbase(0); P.hist_next = nullptr;
-    P.status = sc.status; P.ticket = sc.ticket(0); P.epoch = 1;
-    P.pos_add = (uint32_t)pos_add;
-    P.hashed = sh->hashed ? 1u : 0u;                    // the owner is then looked up for mix64(key), which is what is written
-    P.peer = tab;
-    P.bin = ob;
-    // few bins, many lanes per bin: the bitmap variant measured best here (0.51 ms at N=2; ballots 0.54 ms)
-    TRY((launch_pass_cfg<PassCfg<256, 24, 2, 0, 8, 8>, true, OwnerBin, NoBin, false, true>("scatter_peer", P, sh->sv.nstarts, s)));
-    prof_bytes("scatter_peer", (double)sh->sv.avail + 12.0 * (double)sh->sv.nstarts);
-    return KMG_OK;
-  };
-  int rc = body();
-  dfree(tab, s);
-  scratch_free(sc, s);
-  return rc;
+  SortScratch sc(s);
+  DevBuf<PeerTable> tab(s);
+  TRY(scratch_alloc(sc, sh->sv.nstarts, s));
+  TRY(tab.alloc(1));
+  PeerPtrs pp{};
+  for (int i = 0; i < nparts; ++i) { pp.keys[i] = (uint64_t *)peer_keys[i]; pp.pos[i] = (uint32_t *)peer_pos[i]; }
+  LAUNCH("owner_offsets", s, owner_offsets_kernel<<<1, RADIX, 0, s>>>(d_matrix, nparts, rank, capacity, pp, sc.gbase(0), tab, d_info));
+  if (sh->sv.nstarts == 0) return KMG_OK;
+  OwnerBin ob{d_splitters, nparts};
+  PassParams<OwnerBin, NoBin> P{};
+  P.sv = sh->sv;
+  P.gbase = sc.gbase(0); P.hist_next = nullptr;
+  P.status = sc.status; P.ticket = sc.ticket(0); P.epoch = 1;
+  P.pos_add = (uint32_t)pos_add;
+  P.hashed = sh->hashed ? 1u : 0u;                    // the owner is then looked up for mix64(key), which is what is written
+  P.peer = tab;
+  P.bin = ob;
+  // few bins, many lanes per bin: the bitmap variant measured best here (0.51 ms at N=2; ballots 0.54 ms)
+  TRY((launch_pass_cfg<PassCfg<256, 24, 2, 0, 8, 8>, true, OwnerBin, NoBin, false, true>("scatter_peer", P, sh->sv.nstarts, s)));
+  prof_bytes("scatter_peer", (double)sh->sv.avail + 12.0 * (double)sh->sv.nstarts);
+  return KMG_OK;
 }
 
 __global__ void set_n_kernel(const uint64_t *info, uint64_t cap, uint64_t *n) { *n = info[0] < cap ? info[0] : cap; }
@@ -2515,87 +2412,68 @@ static int owner_build(uint64_t *d_keys, uint32_t *d_pos, uint64_t capacity, con
                        const uint64_t *d_counts, int k, int order, kmg_index **out) {
   TRY(ctx_init());
   cudaStream_t s = g_ctx.stream();
-  kmg_index *ix = new (std::nothrow) kmg_index();
+  IndexPtr ix(new (std::nothrow) kmg_index());
   if (!ix) return fail(KMG_ERR_NOMEM, "host allocation failed");
   ix->device = g_ctx.device;
   ix->k = k;
   const int64_t n = (int64_t)capacity;
-  SortScratch sc;
-  uint64_t *ka = d_keys, *kb = nullptr;
-  uint32_t *pa = d_pos, *pb = nullptr, *pfinal = nullptr;
-  TileSegs *seg = nullptr;
+  SortScratch sc(s);
+  DevBuf<uint64_t> kbuf(s);
+  DevBuf<uint32_t> pbuf(s), pfinal(s);
+  DevBuf<TileSegs> seg(s);
   uint64_t h_info[2] = {0, 0};
   uint32_t h_seg_overflow = 0;
   const bool grouped = grouped_for(k, order, n);
   // the arrays are sized with slack (1.25-1.3x what an owner expects); the digit plan follows the expected record count
   const SortPlan gp = grouped_plan(d_counts ? n * 10 / 13 : n * 4 / 5);
-  auto body = [&]() -> int {
-    TRY(scratch_alloc(sc, n, s, grouped ? gp.rb : RADIX_BITS));
-    TRY(dalloc(&kb, (size_t)n, s));
-    TRY(dalloc(&pb, (size_t)n, s));
-    const unsigned hgrid = (unsigned)std::min<int64_t>(ceil_div<int64_t>(n, 256 * 16), (int64_t)g_ctx.sms * 8);
-    const int rb0 = grouped ? gp.rb : RADIX_BITS;
-    if (d_counts) {
-      TRY(dalloc(&seg, 1, s));
-      LAUNCH("tile_segs", s, tile_segs_kernel<<<1, MAX_SEGS, 0, s>>>(d_counts, nsegs, region_cap, record_tile(rb0), seg, &sc.stats()->n));
-      LAUNCH("hist_rec", s, hist_seg_kernel<256, DigitBin><<<hgrid, 256, 0, s>>>(d_keys, seg, sc.hist(0), DigitBin{0, (1u << rb0) - 1}));
-      CU(cudaMemcpyAsync(&h_seg_overflow, &seg->overflow, 4, cudaMemcpyDeviceToHost, s));
-    } else {
-      LAUNCH("set_n", s, set_n_kernel<<<1, 1, 0, s>>>(d_info, capacity, &sc.stats()->n));
-      LAUNCH("hist_rec", s, hist_rec_kernel<256, DigitBin><<<hgrid, 256, 0, s>>>(d_keys, n, &sc.stats()->n, sc.hist(0), DigitBin{0, (1u << rb0) - 1}));
-      CU(cudaMemcpyAsync(h_info, d_info, sizeof h_info, cudaMemcpyDeviceToHost, s));
-    }
-    TRY(launch_scan_hist(rb0, s, sc.hist(0), sc.gbase(0), (uint64_t *)nullptr));
-    TRY(dalloc(&pfinal, (size_t)n, s));
-    if (grouped) {
-      // records carry mix64(key): sort on its low bits, then partition the groups in which k-mers share them.
-      // The passes ping-pong (caller's arrays <-> ours); the fix-up needs the result and a scratch pair, so the
-      // last pass may not divert into pfinal: copy the positions at the end instead.
-      TRY(sort_tail(sc, gp, 0, true, ka, pa, kb, pb, n, s, nullptr, seg, nsegs));
-      uint32_t h_cnt[4] = {0, 0, 0, 0};
-      uint32_t *fixmem = nullptr;
-      int rc = fix_groups(sc, gp.bits(), ka, pa, kb, pb, n, s, h_cnt, &fixmem);
-      if (rc == KMG_OK && pa != d_pos) {                     // the sorted positions are in an array of ours: the index keeps it
-        dfree(pfinal, s);
-        pfinal = pa;
-        pa = nullptr;
-      } else if (rc == KMG_OK && cudaMemcpyAsync(pfinal, pa, (size_t)n * 4, cudaMemcpyDeviceToDevice, s) != cudaSuccess) {
-        rc = fail(KMG_ERR_CUDA, "copy failed");
-      }
-      if (rc == KMG_OK) {
-        rc = finish_index(ix, sc, ka, pfinal, n, s, true);   // synchronises
-        if (rc == KMG_OK) pfinal = nullptr;                  // the index owns it now (it is freed with the index)
-      }
-      dfree(fixmem, s);
-      TRY(rc);
-      if (h_cnt[2]) return fail(KMG_ERR_RANGE, "more colliding groups than the task lists hold");
-      ix->grouped = true;
-      ix->hbits = gp.bits();
-    } else {
-      TRY(sort_tail(sc, SortPlan{RADIX_BITS, num_passes(k)}, 0, true, ka, pa, kb, pb, n, s, pfinal, seg, nsegs));
-      TRY(finish_index(ix, sc, ka, pfinal, n, s));            // synchronises
-    }
-    pfinal = nullptr;
-    if (ix->unstable) { demote_rank_variant(); return fail(KMG_ERR_UNSTABLE, "position lists not ascending after the one-atomic sort pass; rebuild (the bitmap variant is now selected)"); }
-    const int R = grouped ? gp.passes : num_passes(k);
-    prof_bytes("hist_rec", 8.0 * (double)ix->N);
-    if (R > 1) prof_bytes("sort_pass_hist", 24.0 * (double)ix->N * (R - 1));
-    prof_bytes("sort_pass", 24.0 * (double)ix->N);
-    if (grouped) prof_bytes("group_detect", 8.0 * (double)ix->N);
-    return KMG_OK;
-  };
-  int rc = body();
-  if (ka != d_keys) dfree(ka, s);
-  if (kb != d_keys) dfree(kb, s);
-  if (pa && pa != d_pos) dfree(pa, s);
-  if (pb != d_pos) dfree(pb, s);
-  dfree(pfinal, s);
-  dfree(seg, s);
-  scratch_free(sc, s);
-  if (rc == KMG_OK && (h_info[1] || h_seg_overflow))
-    rc = fail(KMG_ERR_RANGE, "an owner received more than the exchange capacity of %llu records", (unsigned long long)(d_counts ? region_cap : capacity));
-  if (rc != KMG_OK) { cudaStreamSynchronize(s); kmg_free(ix); return rc; }
-  *out = ix;
+  TRY(scratch_alloc(sc, n, s, grouped ? gp.rb : RADIX_BITS));
+  TRY(kbuf.alloc((size_t)n));
+  TRY(pbuf.alloc((size_t)n));
+  uint64_t *ka = d_keys, *kb = kbuf;                       // the passes ping-pong between the caller's arrays and ours
+  uint32_t *pa = d_pos, *pb = pbuf;
+  const unsigned hgrid = (unsigned)std::min<int64_t>(ceil_div<int64_t>(n, 256 * 16), (int64_t)g_ctx.sms * 8);
+  const int rb0 = grouped ? gp.rb : RADIX_BITS;
+  if (d_counts) {
+    TRY(seg.alloc(1));
+    LAUNCH("tile_segs", s, tile_segs_kernel<<<1, MAX_SEGS, 0, s>>>(d_counts, nsegs, region_cap, record_tile(rb0), seg, &sc.stats()->n));
+    LAUNCH("hist_rec", s, hist_seg_kernel<256, DigitBin><<<hgrid, 256, 0, s>>>(d_keys, seg, sc.hist(0), DigitBin{0, (1u << rb0) - 1}));
+    CU(cudaMemcpyAsync(&h_seg_overflow, &seg.get()->overflow, 4, cudaMemcpyDeviceToHost, s));
+  } else {
+    LAUNCH("set_n", s, set_n_kernel<<<1, 1, 0, s>>>(d_info, capacity, &sc.stats()->n));
+    LAUNCH("hist_rec", s, hist_rec_kernel<256, DigitBin><<<hgrid, 256, 0, s>>>(d_keys, n, &sc.stats()->n, sc.hist(0), DigitBin{0, (1u << rb0) - 1}));
+    CU(cudaMemcpyAsync(h_info, d_info, sizeof h_info, cudaMemcpyDeviceToHost, s));
+  }
+  TRY(launch_scan_hist(rb0, s, sc.hist(0), sc.gbase(0), (uint64_t *)nullptr));
+  TRY(pfinal.alloc((size_t)n));
+  if (grouped) {
+    // records carry mix64(key): sort on its low bits, then partition the groups in which k-mers share them.
+    // The passes ping-pong (caller's arrays <-> ours); the fix-up needs the result and a scratch pair, so the
+    // last pass may not divert into pfinal: copy the positions at the end instead.
+    TRY(sort_tail(sc, gp, 0, true, ka, pa, kb, pb, n, s, nullptr, seg, nsegs));
+    uint32_t h_cnt[4] = {0, 0, 0, 0};
+    DevBuf<uint32_t> fixmem(s);
+    TRY(fix_groups(sc, gp.bits(), ka, pa, kb, pb, n, s, h_cnt, fixmem));
+    if (pa != d_pos) pfinal.reset(pbuf.release());          // the sorted positions are in our array: the index keeps it
+    else if (cudaMemcpyAsync(pfinal, pa, (size_t)n * 4, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return fail(KMG_ERR_CUDA, "copy failed");
+    TRY(finish_index(ix.get(), sc, ka, pfinal, n, s, true));   // synchronises
+    pfinal.release();                                        // the index owns it now (it is freed with the index)
+    if (h_cnt[2]) return fail(KMG_ERR_RANGE, "more colliding groups than the task lists hold");
+    ix->grouped = true;
+    ix->hbits = gp.bits();
+  } else {
+    TRY(sort_tail(sc, SortPlan{RADIX_BITS, num_passes(k)}, 0, true, ka, pa, kb, pb, n, s, pfinal, seg, nsegs));
+    TRY(finish_index(ix.get(), sc, ka, pfinal, n, s));            // synchronises
+    pfinal.release();
+  }
+  if (ix->unstable) { demote_rank_variant(); return fail(KMG_ERR_UNSTABLE, "position lists not ascending after the one-atomic sort pass; rebuild (the bitmap variant is now selected)"); }
+  const int R = grouped ? gp.passes : num_passes(k);
+  prof_bytes("hist_rec", 8.0 * (double)ix->N);
+  if (R > 1) prof_bytes("sort_pass_hist", 24.0 * (double)ix->N * (R - 1));
+  prof_bytes("sort_pass", 24.0 * (double)ix->N);
+  if (grouped) prof_bytes("group_detect", 8.0 * (double)ix->N);
+  if (h_info[1] || h_seg_overflow)
+    return fail(KMG_ERR_RANGE, "an owner received more than the exchange capacity of %llu records", (unsigned long long)(d_counts ? region_cap : capacity));
+  *out = ix.release();
   return KMG_OK;
 }
 
@@ -2646,38 +2524,32 @@ extern "C" int kmg_shard_scatter_ranges(const kmg_shard *sh, int nparts, int ran
   if (!sh->hashed) return fail(KMG_ERR_ARG, "region exchange needs a shard of mixed keys (grouped order, k large enough)");
   TRY(ctx_init());
   cudaStream_t s = g_ctx.stream();
-  SortScratch sc;
-  PeerTable *tab = nullptr;
-  auto body = [&]() -> int {
-    TRY(scratch_alloc(sc, sh->sv.nstarts, s, 4));
-    TRY(dalloc(&tab, 1, s));
-    PeerPtrs pp{}, pc{};
-    for (int i = 0; i < nparts; ++i) { pp.keys[i] = (uint64_t *)peer_keys[i]; pp.pos[i] = (uint32_t *)peer_pos[i]; pc.keys[i] = (uint64_t *)peer_counts[i]; }
-    LAUNCH("region_table", s, region_table_kernel<<<1, 256, 0, s>>>(pp, pc, nparts, rank, region_cap, tab, sc.gbase(0), sh->sv.nstarts == 0));
-    if (sh->sv.nstarts == 0) return KMG_OK;
-    PassParams<RangeBin, NoBin> P{};
-    P.sv = sh->sv;
-    P.gbase = sc.gbase(0); P.hist_next = nullptr;
-    P.status = sc.status; P.ticket = sc.ticket(0); P.epoch = 1;
-    P.pos_add = (uint32_t)pos_add;
-    P.hashed = 1;
-    P.peer = tab;
-    P.dbg = g_sort_dbg;
-    P.bin = RangeBin{(uint32_t)nparts};
-    // kmg_tune "scatter_shape" (tuning runs): more resident tiles per SM = more remote stores in flight on the NVLink
-    if (rank_variant() >= 3 && !g_scatter_bitmap) {
-      if (g_scatter_shape == 1) TRY((launch_pass_cfg<PassCfg<256, 24, 3, 3, 4, 4>, true, RangeBin, NoBin, false, true>("scatter_peer", P, sh->sv.nstarts, s)));
-      else if (g_scatter_shape == 2) TRY((launch_pass_cfg<PassCfg<256, 16, 4, 3, 4, 4>, true, RangeBin, NoBin, false, true>("scatter_peer", P, sh->sv.nstarts, s)));
-      else TRY((launch_pass_cfg<PassCfg<256, 24, 2, 3, 4, 4>, true, RangeBin, NoBin, false, true>("scatter_peer", P, sh->sv.nstarts, s)));
-    } else
-      TRY((launch_pass_cfg<PassCfg<256, 24, 2, 0, 8, 4>, true, RangeBin, NoBin, false, true>("scatter_peer", P, sh->sv.nstarts, s)));
-    prof_bytes("scatter_peer", (double)sh->sv.avail + 12.0 * (double)sh->sv.nstarts);
-    return KMG_OK;
-  };
-  int rc = body();
-  dfree(tab, s);
-  scratch_free(sc, s);
-  return rc;
+  SortScratch sc(s);
+  DevBuf<PeerTable> tab(s);
+  TRY(scratch_alloc(sc, sh->sv.nstarts, s, 4));
+  TRY(tab.alloc(1));
+  PeerPtrs pp{}, pc{};
+  for (int i = 0; i < nparts; ++i) { pp.keys[i] = (uint64_t *)peer_keys[i]; pp.pos[i] = (uint32_t *)peer_pos[i]; pc.keys[i] = (uint64_t *)peer_counts[i]; }
+  LAUNCH("region_table", s, region_table_kernel<<<1, 256, 0, s>>>(pp, pc, nparts, rank, region_cap, tab, sc.gbase(0), sh->sv.nstarts == 0));
+  if (sh->sv.nstarts == 0) return KMG_OK;
+  PassParams<RangeBin, NoBin> P{};
+  P.sv = sh->sv;
+  P.gbase = sc.gbase(0); P.hist_next = nullptr;
+  P.status = sc.status; P.ticket = sc.ticket(0); P.epoch = 1;
+  P.pos_add = (uint32_t)pos_add;
+  P.hashed = 1;
+  P.peer = tab;
+  P.dbg = g_sort_dbg;
+  P.bin = RangeBin{(uint32_t)nparts};
+  // kmg_tune "scatter_shape" (tuning runs): more resident tiles per SM = more remote stores in flight on the NVLink
+  if (rank_variant() >= 3 && !g_scatter_bitmap) {
+    if (g_scatter_shape == 1) TRY((launch_pass_cfg<PassCfg<256, 24, 3, 3, 4, 4>, true, RangeBin, NoBin, false, true>("scatter_peer", P, sh->sv.nstarts, s)));
+    else if (g_scatter_shape == 2) TRY((launch_pass_cfg<PassCfg<256, 16, 4, 3, 4, 4>, true, RangeBin, NoBin, false, true>("scatter_peer", P, sh->sv.nstarts, s)));
+    else TRY((launch_pass_cfg<PassCfg<256, 24, 2, 3, 4, 4>, true, RangeBin, NoBin, false, true>("scatter_peer", P, sh->sv.nstarts, s)));
+  } else
+    TRY((launch_pass_cfg<PassCfg<256, 24, 2, 0, 8, 4>, true, RangeBin, NoBin, false, true>("scatter_peer", P, sh->sv.nstarts, s)));
+  prof_bytes("scatter_peer", (double)sh->sv.avail + 12.0 * (double)sh->sv.nstarts);
+  return KMG_OK;
 }
 
 // match the (mixed key, i) records of a region-mode scatter: compacted into dense arrays, then as kmg_query_received
@@ -2690,30 +2562,26 @@ extern "C" int kmg_query_regions(const kmg_index *ix, const uint64_t *d_keys, co
   TRY(use_index(ix));
   cudaStream_t s = g_ctx.stream();
   const uint64_t capacity = region_cap * (uint64_t)nparts;
-  TileSegs *seg = nullptr;
-  uint64_t *dk = nullptr, *dn = nullptr;
-  uint32_t *di = nullptr;
+  DevBuf<TileSegs> seg(s);
+  DevBuf<uint64_t> dn(s), dk(s);
+  DevBuf<uint32_t> di(s);
   uint32_t h_seg_overflow = 0;
-  auto body = [&]() -> int {
-    TRY(dalloc(&seg, 1, s));
-    TRY(dalloc(&dn, 1, s));
-    TRY(dalloc(&dk, (size_t)capacity, s));
-    TRY(dalloc(&di, (size_t)capacity, s));
-    LAUNCH("tile_segs", s, tile_segs_kernel<<<1, MAX_SEGS, 0, s>>>(d_counts, nparts, region_cap, (uint32_t)PROBE_TILE, seg, dn));
-    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(region_cap, 256), (uint64_t)g_ctx.sms * 8);
-    LAUNCH("seg_compact", s, seg_compact_kernel<<<grid, 256, 0, s>>>(d_keys, (const uint32_t *)d_i, seg, dk, di));
-    CU(cudaMemcpyAsync(&h_seg_overflow, &seg->overflow, 4, cudaMemcpyDeviceToHost, s));
-    SeqView sv{};
-    return query_common(ix, false, sv, dk, (const int32_t *)di, (int64_t)capacity, st, M, dn, true);   // synchronises
-  };
-  int rc = body();
-  dfree(seg, s); dfree(dn, s); dfree(dk, s); dfree(di, s);
-  if (rc == KMG_OK && h_seg_overflow) {
+  TRY(seg.alloc(1));
+  TRY(dn.alloc(1));
+  TRY(dk.alloc((size_t)capacity));
+  TRY(di.alloc((size_t)capacity));
+  LAUNCH("tile_segs", s, tile_segs_kernel<<<1, MAX_SEGS, 0, s>>>(d_counts, nparts, region_cap, (uint32_t)PROBE_TILE, seg, dn));
+  const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(region_cap, 256), (uint64_t)g_ctx.sms * 8);
+  LAUNCH("seg_compact", s, seg_compact_kernel<<<grid, 256, 0, s>>>(d_keys, (const uint32_t *)d_i, seg, dk, di));
+  CU(cudaMemcpyAsync(&h_seg_overflow, &seg.get()->overflow, 4, cudaMemcpyDeviceToHost, s));
+  SeqView sv{};
+  TRY(query_common(ix, false, sv, dk, (const int32_t *)di.get(), (int64_t)capacity, st, M, dn, true));   // synchronises
+  if (h_seg_overflow) {
     kmg_query_free(*st);
     *st = nullptr;
     return fail(KMG_ERR_RANGE, "an owner received more than the exchange capacity of %llu records", (unsigned long long)region_cap);
   }
-  return rc;
+  return KMG_OK;
 }
 
 // ---- exchange buffers that other processes on the node can map (CUDA IPC over NVLink) ---------------------
@@ -2877,35 +2745,25 @@ extern "C" int kmg_shard_open_packed(const void *d_own, int64_t n_own, int64_t L
   if (n_own != s1 - s0 || (n_own > 0 && !d_own)) return fail(KMG_ERR_ARG, "rank %d must hold bytes [%lld,%lld) of the sequence", rank, (long long)s0, (long long)s1);
   TRY(ctx_init());
   cudaStream_t s = g_ctx.stream();
-  kmg_shard *sh = new (std::nothrow) kmg_shard();
-  if (!sh) return fail(KMG_ERR_NOMEM, "host allocation failed");
-  sh->device = g_ctx.device;
-  sh->hashed = grouped_for(k, order, 0);
   const int pack_bytes = PACK_HDR + 8 * n_samples;
-  auto body = [&]() -> int {
-    const int64_t need_hi = std::min<int64_t>(L, s1 + k - 1);
-    const int64_t avail = std::max<int64_t>(0, need_hi - s0);
-    const size_t cap = 16 + (size_t)((avail + 15) / 16) * 16 + 16;
-    TRY(dalloc(&sh->ds.buf, cap, s));
-    sh->ds.base = sh->ds.buf + 16;
-    CU(cudaMemsetAsync(sh->ds.buf, 0, 16, s));
-    CU(cudaMemsetAsync(sh->ds.buf + cap - 32, 0, 32, s));
-    if (n_own > 0) CU(cudaMemcpyAsync(sh->ds.base, d_own, (size_t)n_own, cudaMemcpyDefault, s));
-    const int need_right = (int)(need_hi - s1);
-    if (need_right > 0 || s0 > 0)
-      LAUNCH("halo_fill", s, halo_fill_kernel<<<1, 32, 0, s>>>(sh->ds.base, n_own, need_right, s0 > 0 && n_own > 0, rank, world, per, L, k,
-                                                               (const uint8_t *)d_allpack, pack_bytes));
-    int64_t nstarts = std::min<int64_t>(s1, L - k + 1) - s0;
-    sh->sv.base = sh->ds.base; sh->sv.nstarts = nstarts > 0 ? nstarts : 0; sh->sv.avail = avail; sh->sv.s0 = s0; sh->sv.L = L; sh->sv.k = k;
-    if (s0 + sh->sv.nstarts > (int64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "positions exceed int");
-    if (world > 1 && d_splitters)
-      LAUNCH("select_splitters", s, select_splitters_kernel<<<ceil_div(n_samples * world, 256), 256, 0, s>>>(
-                                        (const uint8_t *)d_allpack, pack_bytes, n_samples, world, d_splitters));
-    return KMG_OK;
-  };
-  int rc = body();
-  if (rc != KMG_OK) { kmg_shard_close(sh); return rc; }
-  *out = sh;
+  const int64_t need_hi = std::min<int64_t>(L, s1 + k - 1);
+  const int64_t avail = std::max<int64_t>(0, need_hi - s0);
+  DevBuf<uint8_t> buf(s);
+  TRY(seq_alloc(buf, avail, s));
+  uint8_t *base = buf + 16;
+  if (n_own > 0) CU(cudaMemcpyAsync(base, d_own, (size_t)n_own, cudaMemcpyDefault, s));
+  const int need_right = (int)(need_hi - s1);
+  if (need_right > 0 || s0 > 0)
+    LAUNCH("halo_fill", s, halo_fill_kernel<<<1, 32, 0, s>>>(base, n_own, need_right, s0 > 0 && n_own > 0, rank, world, per, L, k,
+                                                             (const uint8_t *)d_allpack, pack_bytes));
+  int64_t nstarts = std::min<int64_t>(s1, L - k + 1) - s0;
+  SeqView sv;
+  sv.base = base; sv.nstarts = nstarts > 0 ? nstarts : 0; sv.avail = avail; sv.s0 = s0; sv.L = L; sv.k = k;
+  if (s0 + sv.nstarts > (int64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "positions exceed int");
+  if (world > 1 && d_splitters)
+    LAUNCH("select_splitters", s, select_splitters_kernel<<<ceil_div(n_samples * world, 256), 256, 0, s>>>(
+                                      (const uint8_t *)d_allpack, pack_bytes, n_samples, world, d_splitters));
+  if (!(*out = new_shard(buf, sv, grouped_for(k, order, 0)))) return fail(KMG_ERR_NOMEM, "host allocation failed");
   return KMG_OK;
 }
 
@@ -2991,81 +2849,65 @@ extern "C" int kmg_count_new(int k, int source_n, kmg_counter **out) {
 }
 extern "C" int kmg_count_free(kmg_counter *c) {
   if (!c) return KMG_OK;
-  int prev = -1;
-  cudaGetDevice(&prev);
-  cudaSetDevice(c->device);
-  const bool mine = g_ctx.ready && g_ctx.device == c->device;
-  if (mine) cudaStreamSynchronize(g_ctx.stream()); else cudaDeviceSynchronize();
-  g_arena[c->device & 63].put(c->keys, nullptr, true);
-  g_arena[c->device & 63].put(c->counts, nullptr, true);
-  g_arena[c->device & 63].put(c->hash, nullptr, true);
-  cudaGetLastError();
-  if (prev >= 0) cudaSetDevice(prev);
+  release_on_device(c->device, {c->keys, c->counts, c->hash});
   delete c;
   return KMG_OK;
 }
-static int use_counter(const kmg_counter *c) {
-  if (!c) return fail(KMG_ERR_ARG, "counter is NULL");
-  TRY(ctx_init());
-  if (c->device != g_ctx.device) return fail(KMG_ERR_ARG, "the count table lives on device %d but this thread works on device %d", c->device, g_ctx.device);
-  return KMG_OK;
-}
+static int use_counter(const kmg_counter *c) { return c ? use_device(c->device, "the count table lives") : fail(KMG_ERR_ARG, "counter is NULL"); }
 
 // seq_to_counts(seq, k, hash, source, source_n) for one sequence (src/kmer_hash.c:220-252)
 extern "C" int kmg_count_add(kmg_counter *c, const char *seq, int64_t len, int source) {
   TRY(use_counter(c));
   if (source < 0 || source >= c->source_n) return fail(KMG_ERR_ARG, "source_n must be larger than 1 and larger than source");
   if (len < 0 || (len > 0 && !seq)) return fail(KMG_ERR_ARG, "bad sequence pointer/length");
-  kmg_index *b = nullptr;
-  TRY(kmg_build_ordered(seq, len, c->k, KMG_ORDER_SORTED, &b));
-  if (b->U == 0) { kmg_free(b); return KMG_OK; }
+  kmg_index *bi = nullptr;
+  TRY(kmg_build_ordered(seq, len, c->k, KMG_ORDER_SORTED, &bi));
+  const IndexPtr b(bi);
+  if (b->U == 0) return KMG_OK;
   cudaStream_t s = g_ctx.stream();
   {                                                          // the key table describes the arrays about to be replaced
     std::lock_guard<std::mutex> g(c->mu);
-    dfree(c->hash, s);
+    DevBuf<uint4> table(s, c->hash);
+    c->hash = nullptr;
     c->hash_nb = 0;
   }
   const int sn = c->source_n;
   const unsigned grid_of_b = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(b->U, 256), (uint64_t)g_ctx.sms * 16);
-  uint64_t *cat_keys = nullptr;
-  uint32_t *cat_pay = nullptr;
-  int32_t *ncounts = nullptr;
-  kmg_index *m = nullptr;
-  auto body = [&]() -> int {
-    if (c->U == 0) {                                         // first batch: the table is the batch
-      TRY(dalloc(&ncounts, (size_t)b->U * sn, s));
-      CU(cudaMemsetAsync(ncounts, 0, (size_t)b->U * sn * sizeof(int32_t), s));
-      LAUNCH("count_first", s, count_first_kernel<<<grid_of_b, 256, 0, s>>>(b->ustart, b->U, sn, source, ncounts));
-      CU(cudaStreamSynchronize(s));
-      c->keys = b->ukeys; b->ukeys = nullptr;                // the batch's key array becomes the table's
-      c->counts = ncounts; ncounts = nullptr;
-      c->U = b->U; c->new_total += b->U;
-      return KMG_OK;
-    }
-    const uint64_t Ut = c->U, n = Ut + b->U;
-    if (n > (uint64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "count table would exceed 2^31-1 k-mers");
-    TRY(dalloc(&cat_keys, (size_t)n, s));
-    TRY(dalloc(&cat_pay, (size_t)n, s));
-    CU(cudaMemcpyAsync(cat_keys, c->keys, Ut * 8, cudaMemcpyDeviceToDevice, s));
-    CU(cudaMemcpyAsync(cat_keys + Ut, b->ukeys, b->U * 8, cudaMemcpyDeviceToDevice, s));
-    LAUNCH("iota", s, iota_kernel<<<(unsigned)std::min<uint64_t>(ceil_div<uint64_t>(n, 256), (uint64_t)g_ctx.sms * 16), 256, 0, s>>>(cat_pay, n));
-    TRY(kmg_build_records(cat_keys, cat_pay, (int64_t)n, c->k, &m));      // stable: a key's table entry precedes its batch entry
-    TRY(dalloc(&ncounts, (size_t)m->U * sn, s));
-    LAUNCH("count_merge", s, count_merge_kernel<<<(unsigned)std::min<uint64_t>(ceil_div<uint64_t>(m->U, 256), (uint64_t)g_ctx.sms * 16), 256, 0, s>>>(
-                                 m->ustart, m->pos, m->U, Ut, c->counts, b->ustart, sn, source, ncounts));
+  if (c->U == 0) {                                           // first batch: the table is the batch
+    DevBuf<int32_t> ncounts(s);
+    TRY(ncounts.alloc((size_t)b->U * sn));
+    CU(cudaMemsetAsync(ncounts, 0, (size_t)b->U * sn * sizeof(int32_t), s));
+    LAUNCH("count_first", s, count_first_kernel<<<grid_of_b, 256, 0, s>>>(b->ustart, b->U, sn, source, ncounts));
     CU(cudaStreamSynchronize(s));
-    dfree(c->keys, s); dfree(c->counts, s);
-    c->keys = m->ukeys; m->ukeys = nullptr;
-    c->counts = ncounts; ncounts = nullptr;
-    c->new_total += m->U - Ut;
-    c->U = m->U;
+    c->keys = b->ukeys; b->ukeys = nullptr;                // the batch's key array becomes the table's
+    c->counts = ncounts.release();
+    c->U = b->U; c->new_total += b->U;
     return KMG_OK;
-  };
-  const int rc = body();
-  dfree(cat_keys, s); dfree(cat_pay, s); dfree(ncounts, s);
-  if (m) kmg_free(m);
-  kmg_free(b);
-  return rc;
+  }
+  const uint64_t Ut = c->U, n = Ut + b->U;
+  if (n > (uint64_t)INT32_MAX) return fail(KMG_ERR_RANGE, "count table would exceed 2^31-1 k-mers");
+  DevBuf<uint64_t> cat_keys(s);
+  DevBuf<uint32_t> cat_pay(s);
+  TRY(cat_keys.alloc((size_t)n));
+  TRY(cat_pay.alloc((size_t)n));
+  CU(cudaMemcpyAsync(cat_keys, c->keys, Ut * 8, cudaMemcpyDeviceToDevice, s));
+  CU(cudaMemcpyAsync(cat_keys + Ut, b->ukeys, b->U * 8, cudaMemcpyDeviceToDevice, s));
+  LAUNCH("iota", s, iota_kernel<<<(unsigned)std::min<uint64_t>(ceil_div<uint64_t>(n, 256), (uint64_t)g_ctx.sms * 16), 256, 0, s>>>(cat_pay, n));
+  kmg_index *mi = nullptr;
+  TRY(kmg_build_records(cat_keys, cat_pay, (int64_t)n, c->k, &mi));      // stable: a key's table entry precedes its batch entry
+  const IndexPtr m(mi);
+  DevBuf<int32_t> ncounts(s);
+  TRY(ncounts.alloc((size_t)m->U * sn));
+  LAUNCH("count_merge", s, count_merge_kernel<<<(unsigned)std::min<uint64_t>(ceil_div<uint64_t>(m->U, 256), (uint64_t)g_ctx.sms * 16), 256, 0, s>>>(
+                               m->ustart, m->pos, m->U, Ut, c->counts, b->ustart, sn, source, ncounts));
+  CU(cudaStreamSynchronize(s));
+  DevBuf<uint64_t> old_keys(s, c->keys);                     // the table's arrays before this batch: freed on return
+  DevBuf<int32_t> old_counts(s, c->counts);
+  c->keys = m->ukeys; m->ukeys = nullptr;
+  c->counts = ncounts.release();
+  c->new_total += m->U - Ut;
+  c->U = m->U;
+  return KMG_OK;
 }
 
 extern "C" int kmg_count_sizes(const kmg_counter *c, uint64_t *U, int *source_n, int *k, uint64_t *new_total) {
@@ -3136,17 +2978,14 @@ extern "C" int kmg_count_spectrum(const kmg_counter *c, int source, uint32_t max
   if (max_count < 1 || max_count > (1u << 30)) return fail(KMG_ERR_ARG, "Unsuitable value of max_count");
   if (source >= c->source_n) return fail(KMG_ERR_ARG, "source out of range");
   cudaStream_t s = g_ctx.stream();
-  unsigned long long *d = nullptr;
-  TRY(dalloc(&d, (size_t)max_count + 1, s));
-  int rc = KMG_OK;
-  if (cudaMemsetAsync(d, 0, ((size_t)max_count + 1) * 8, s) != cudaSuccess) rc = fail(KMG_ERR_CUDA, "memset failed");
-  if (rc == KMG_OK && c->U) {
+  DevBuf<unsigned long long> d(s);
+  TRY(d.alloc((size_t)max_count + 1));
+  if (cudaMemsetAsync(d, 0, ((size_t)max_count + 1) * 8, s) != cudaSuccess) return fail(KMG_ERR_CUDA, "memset failed");
+  if (c->U) {
     const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(c->U, 256), (uint64_t)g_ctx.sms * 16);
     spectrum_counts_kernel<<<grid, 256, 0, s>>>(c->counts, c->U, c->source_n, source, max_count, d);
   }
-  if (rc == KMG_OK) rc = spectrum_out(d, max_count, spec, s);
-  dfree(d, s);
-  return rc;
+  return spectrum_out(d, max_count, spec, s);
 }
 // the same for a position index: the count of a k-mer is the length of its position list
 extern "C" int kmg_index_spectrum(const kmg_index *ix, uint32_t max_count, double *spec) {
@@ -3154,17 +2993,14 @@ extern "C" int kmg_index_spectrum(const kmg_index *ix, uint32_t max_count, doubl
   if (!spec) return fail(KMG_ERR_ARG, "spec is NULL");
   if (max_count < 1 || max_count > (1u << 30)) return fail(KMG_ERR_ARG, "Unsuitable value of max_count");
   cudaStream_t s = g_ctx.stream();
-  unsigned long long *d = nullptr;
-  TRY(dalloc(&d, (size_t)max_count + 1, s));
-  int rc = KMG_OK;
-  if (cudaMemsetAsync(d, 0, ((size_t)max_count + 1) * 8, s) != cudaSuccess) rc = fail(KMG_ERR_CUDA, "memset failed");
-  if (rc == KMG_OK && ix->U) {
+  DevBuf<unsigned long long> d(s);
+  TRY(d.alloc((size_t)max_count + 1));
+  if (cudaMemsetAsync(d, 0, ((size_t)max_count + 1) * 8, s) != cudaSuccess) return fail(KMG_ERR_CUDA, "memset failed");
+  if (ix->U) {
     const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(ix->U, 256), (uint64_t)g_ctx.sms * 16);
     spectrum_index_kernel<<<grid, 256, 0, s>>>(ix->ustart, ix->U, max_count, d);
   }
-  if (rc == KMG_OK) rc = spectrum_out(d, max_count, spec, s);
-  dfree(d, s);
-  return rc;
+  return spectrum_out(d, max_count, spec, s);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -3178,19 +3014,14 @@ static int ensure_count_hash(kmg_counter *c) {
   cudaStream_t s = g_ctx.stream();
   uint64_t cap = 4 * BUCKET_SLOTS;
   while (cap < 2 * c->U) cap <<= 1;
-  uint4 *slots = nullptr;
-  TRY(dalloc(&slots, cap, s));
-  auto body = [&]() -> int {
-    CU(cudaMemsetAsync(slots, 0, cap * sizeof(uint4), s));
-    const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(c->U, 256), (uint64_t)g_ctx.sms * 32);
-    LAUNCH("count_hash_insert", s, hash_insert_kernel<<<grid, 256, 0, s>>>(c->keys, CountPayload{c->counts, c->source_n}, c->U,
-                                                                         KeyHash{slots, cap / BUCKET_SLOTS, 0}, false));
-    CU(cudaStreamSynchronize(s));
-    return KMG_OK;
-  };
-  const int rc = body();
-  if (rc != KMG_OK) { dfree(slots, s); return rc; }
-  c->hash = slots; c->hash_nb = cap / BUCKET_SLOTS;
+  DevBuf<uint4> slots(s);
+  TRY(slots.alloc(cap));
+  CU(cudaMemsetAsync(slots, 0, cap * sizeof(uint4), s));
+  const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(c->U, 256), (uint64_t)g_ctx.sms * 32);
+  LAUNCH("count_hash_insert", s, hash_insert_kernel<<<grid, 256, 0, s>>>(c->keys, CountPayload{c->counts, c->source_n}, c->U,
+                                                                       KeyHash{slots, cap / BUCKET_SLOTS, 0}, false));
+  CU(cudaStreamSynchronize(s));
+  c->hash = slots.release(); c->hash_nb = cap / BUCKET_SLOTS;
   prof_bytes("count_hash_insert", 12.0 * c->U + 16.0 * c->U);
   return KMG_OK;
 }
@@ -3211,10 +3042,10 @@ static int depth_args(const char *q, int64_t qlen, int k, int strands, const int
 static int depth_run(const char *qseq, int64_t qlen, int64_t nwin, int k, bool both, KeyHash kt, const int32_t *counts, int cols,
                      int32_t *out) {
   cudaStream_t s = g_ctx.stream();
-  DevSeq ds;
-  TRY(upload_seq(qseq, qlen, s, &ds));
+  DevBuf<uint8_t> dseq(s);
+  TRY(upload_seq(qseq, qlen, s, dseq));
   SeqView sv;
-  sv.base = ds.base; sv.nstarts = nwin; sv.avail = qlen; sv.s0 = 0; sv.L = qlen; sv.k = k;
+  sv.base = dseq + 16; sv.nstarts = nwin; sv.avail = qlen; sv.s0 = 0; sv.L = qlen; sv.k = k;
   const size_t row_bytes = 4 * (size_t)cols;
   const bool multi = cols > 1;                           // not counts != nullptr: an empty table has no matrix
   const int rc = stream_rows((uint64_t)nwin, row_bytes, out, CHUNK_BYTES / row_bytes, [=](uint64_t first, uint64_t rows, void *dst, uint64_t *, cudaStream_t st) -> int {
@@ -3227,7 +3058,6 @@ static int depth_run(const char *qseq, int64_t qlen, int64_t nwin, int k, bool b
 #undef KMG_DEPTH
     return KMG_OK;
   });
-  dfree(ds.buf, s);
   // one 128-byte line of HBM per table request (tools/micro/gups.cu); with several columns one more per request for the
   // row gather; counted for every window, so a query whose windows miss or are invalid is charged the same
   const double lines = (both ? 2.0 : 1.0) * (multi ? 2.0 : 1.0) * (double)nwin;
@@ -3274,15 +3104,7 @@ struct kmg_reads {
 
 extern "C" int kmg_reads_free(kmg_reads *r) {
   if (!r) return KMG_OK;
-  int prev = -1;
-  cudaGetDevice(&prev);
-  cudaSetDevice(r->device);
-  const bool mine = g_ctx.ready && g_ctx.device == r->device;
-  if (mine) cudaStreamSynchronize(g_ctx.stream()); else cudaDeviceSynchronize();
-  g_arena[r->device & 63].put(r->seq, nullptr, true);
-  g_arena[r->device & 63].put(r->d_rec_off, nullptr, true);
-  cudaGetLastError();
-  if (prev >= 0) cudaSetDevice(prev);
+  release_on_device(r->device, {r->seq, r->d_rec_off});
   delete r;
   return KMG_OK;
 }
@@ -3294,102 +3116,98 @@ extern "C" int kmg_reads_from_memory(const void *text, int64_t len, kmg_reads **
   if (len < 0 || (len > 0 && !text)) return fail(KMG_ERR_ARG, "bad text pointer/length");
   TRY(ctx_init());
   cudaStream_t s = g_ctx.stream();
-  kmg_reads *r = new (std::nothrow) kmg_reads();
+  ReadsPtr r(new (std::nothrow) kmg_reads());
   if (!r) return fail(KMG_ERR_NOMEM, "host allocation failed");
   r->device = g_ctx.device;
   r->rec_off.assign(1, 0);
-  if (len == 0) { *out = r; return KMG_OK; }
+  if (len == 0) { *out = r.release(); return KMG_OK; }
   const uint64_t n = (uint64_t)len, nblocks = (n + 15) / 16;
-  uint8_t *d_text = nullptr, *kind = nullptr;
-  uint64_t *nl = nullptr, *seq_len = nullptr, *seq_before = nullptr, *hdr_before = nullptr, *name_pos = nullptr;
-  uint32_t *blk_nl = nullptr, *tickets = nullptr, *name_len = nullptr;
-  Pair64 *status = nullptr;
-  ReadsInfo *info = nullptr;
+  const size_t cap = (size_t)nblocks * 16 + 64;
+  DevBuf<uint8_t> d_text(s);
+  TRY(d_text.alloc(cap));
+  CU(cudaMemsetAsync(d_text + (cap - 80), 0, 80, s));
+  if (n > (uint64_t)(8 << 20) && staged_transfers() && ptr_kind(text) == PK_HOST_PAGEABLE) TRY(staged_upload(d_text, text, n, s));
+  else CU(cudaMemcpyAsync(d_text, text, n, cudaMemcpyDefault, s));
+  DevBuf<ReadsInfo> info(s);
+  DevBuf<uint32_t> tickets(s);
+  TRY(info.alloc(1));
+  TRY(tickets.alloc(4));
+  CU(cudaMemsetAsync(info, 0, sizeof(ReadsInfo), s));
+  CU(cudaMemsetAsync(tickets, 0, 16, s));
+  // 1. newlines (a line-start byte decides FASTA / FASTQ: the first byte of the file)
+  uint8_t first = 0;
+  CU(cudaMemcpyAsync(&first, d_text, 1, cudaMemcpyDeviceToHost, s));
+  const uint64_t tiles1 = ceil_div<uint64_t>(nblocks, 256 * 4);
+  DevBuf<Pair64> status(s);
+  TRY(status.alloc((size_t)std::max<uint64_t>(tiles1, 1)));
+  CU(cudaMemsetAsync(status, 0, (size_t)tiles1 * sizeof(Pair64), s));
+  unsigned long long *d_cnt = reinterpret_cast<unsigned long long *>(&info.get()->total_bases), h_cnt = 0;    // borrowed until line_scan sets it
+  LAUNCH("nl_count", s, nl_count_kernel<<<(unsigned)std::min<uint64_t>(ceil_div<uint64_t>(nblocks, 256), (uint64_t)g_ctx.sms * 16), 256, 0, s>>>(d_text, n, d_cnt));
+  CU(cudaMemcpyAsync(&h_cnt, d_cnt, 8, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  DevBuf<uint64_t> nl(s);
+  DevBuf<uint32_t> blk_nl(s);
+  TRY(nl.alloc((size_t)h_cnt + 2));
+  TRY(blk_nl.alloc((size_t)nblocks));
   ReadsInfo h{};
-  std::vector<uint64_t> h_name_pos;
+  LAUNCH("nl_scan", s, nl_scan_kernel<256><<<(unsigned)tiles1, 256, 0, s>>>(d_text, n, nl, blk_nl, status, tickets + 0, info));
+  CU(cudaMemcpyAsync(&h, info, sizeof h, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  if (first != '>' && first != '@') return fail(KMG_ERR_ARG, "not a FASTA/FASTQ file: it starts with byte 0x%02x", first);
+  const bool fastq = first == '@';
+  const uint64_t nlines = h.n_lines;
+  DevBuf<uint64_t> seq_len(s), seq_before(s), hdr_before(s);
+  DevBuf<uint8_t> kind(s);
+  TRY(seq_len.alloc((size_t)nlines + 1));
+  TRY(kind.alloc((size_t)nlines + 1));
+  TRY(seq_before.alloc((size_t)nlines + 1));
+  TRY(hdr_before.alloc((size_t)nlines + 1));
+  const unsigned lgrid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(std::max<uint64_t>(nlines, 1), 256), (uint64_t)g_ctx.sms * 16);
+  LAUNCH("line_info", s, line_info_kernel<<<lgrid, 256, 0, s>>>(d_text, n, nl, info, fastq, seq_len, kind, info));
+  const uint64_t tiles2 = ceil_div<uint64_t>(std::max<uint64_t>(nlines, 1), 256 * 8);
+  TRY(status.alloc((size_t)tiles2));                        // the newline scan's status goes back first
+  CU(cudaMemsetAsync(status, 0, (size_t)tiles2 * sizeof(Pair64), s));
+  LAUNCH("line_scan", s, line_scan_kernel<256, 8><<<(unsigned)tiles2, 256, 0, s>>>(seq_len, kind, info, seq_before, hdr_before, status, tickets + 1));
+  CU(cudaMemcpyAsync(&h, info, sizeof h, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  if (h.bad) return fail(KMG_ERR_ARG, "malformed FASTQ: only the four-line form (@name / sequence / + / qualities of the same length) is read");
+  r->n_records = h.n_records; r->total_bases = h.total_bases;
+  const uint64_t packed = h.total_bases + h.n_records;
+  TRY(dalloc(&r->seq, (size_t)packed + 16, s));
+  TRY(dalloc(&r->d_rec_off, (size_t)h.n_records + 1, s));
+  DevBuf<uint64_t> name_pos(s);
+  DevBuf<uint32_t> name_len(s);
+  TRY(name_pos.alloc((size_t)h.n_records + 1));
+  TRY(name_len.alloc((size_t)h.n_records + 1));
+  LAUNCH("records", s, record_kernel<<<lgrid, 256, 0, s>>>(d_text, n, nl, info, kind, seq_before, hdr_before, r->d_rec_off, name_pos, name_len));
+  const unsigned pgrid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(nblocks, 256), (uint64_t)g_ctx.sms * 16);
+  LAUNCH("pack_reads", s, pack_kernel<<<pgrid, 256, 0, s>>>(d_text, n, nl, blk_nl, info, kind, seq_before, hdr_before, r->seq, info));
+  if (h.n_records)
+    LAUNCH("record_finish", s, record_finish_kernel<<<(unsigned)std::min<uint64_t>(ceil_div<uint64_t>(h.n_records, 256), (uint64_t)g_ctx.sms * 16), 256, 0, s>>>(info, r->d_rec_off, r->seq));
+  std::unique_ptr<uint64_t[]> h_name_pos(new uint64_t[h.n_records + 1]);
   std::vector<uint32_t> h_name_len;
-  auto body = [&]() -> int {
-    const size_t cap = (size_t)nblocks * 16 + 64;
-    TRY(dalloc(&d_text, cap, s));
-    CU(cudaMemsetAsync(d_text + (cap - 80), 0, 80, s));
-    if (n > (uint64_t)(8 << 20) && staged_transfers() && ptr_kind(text) == PK_HOST_PAGEABLE) TRY(staged_upload(d_text, text, n, s));
-    else CU(cudaMemcpyAsync(d_text, text, n, cudaMemcpyDefault, s));
-    TRY(dalloc(&info, 1, s));
-    TRY(dalloc(&tickets, 4, s));
-    CU(cudaMemsetAsync(info, 0, sizeof(ReadsInfo), s));
-    CU(cudaMemsetAsync(tickets, 0, 16, s));
-    // 1. newlines (a line-start byte decides FASTA / FASTQ: the first byte of the file)
-    uint8_t first = 0;
-    CU(cudaMemcpyAsync(&first, d_text, 1, cudaMemcpyDeviceToHost, s));
-    const uint64_t tiles1 = ceil_div<uint64_t>(nblocks, 256 * 4);
-    TRY(dalloc(&status, (size_t)std::max<uint64_t>(tiles1, 1), s));
-    CU(cudaMemsetAsync(status, 0, (size_t)tiles1 * sizeof(Pair64), s));
-    unsigned long long *d_cnt = reinterpret_cast<unsigned long long *>(&info->total_bases), h_cnt = 0;    // borrowed until line_scan sets it
-    LAUNCH("nl_count", s, nl_count_kernel<<<(unsigned)std::min<uint64_t>(ceil_div<uint64_t>(nblocks, 256), (uint64_t)g_ctx.sms * 16), 256, 0, s>>>(d_text, n, d_cnt));
-    CU(cudaMemcpyAsync(&h_cnt, d_cnt, 8, cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    TRY(dalloc(&nl, (size_t)h_cnt + 2, s));
-    TRY(dalloc(&blk_nl, (size_t)nblocks, s));
-    LAUNCH("nl_scan", s, nl_scan_kernel<256><<<(unsigned)tiles1, 256, 0, s>>>(d_text, n, nl, blk_nl, status, tickets + 0, info));
-    CU(cudaMemcpyAsync(&h, info, sizeof h, cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    if (first != '>' && first != '@') return fail(KMG_ERR_ARG, "not a FASTA/FASTQ file: it starts with byte 0x%02x", first);
-    const bool fastq = first == '@';
-    const uint64_t nlines = h.n_lines;
-    TRY(dalloc(&seq_len, (size_t)nlines + 1, s));
-    TRY(dalloc(&kind, (size_t)nlines + 1, s));
-    TRY(dalloc(&seq_before, (size_t)nlines + 1, s));
-    TRY(dalloc(&hdr_before, (size_t)nlines + 1, s));
-    const unsigned lgrid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(std::max<uint64_t>(nlines, 1), 256), (uint64_t)g_ctx.sms * 16);
-    LAUNCH("line_info", s, line_info_kernel<<<lgrid, 256, 0, s>>>(d_text, n, nl, info, fastq, seq_len, kind, info));
-    const uint64_t tiles2 = ceil_div<uint64_t>(std::max<uint64_t>(nlines, 1), 256 * 8);
-    dfree(status, s);
-    TRY(dalloc(&status, (size_t)tiles2, s));
-    CU(cudaMemsetAsync(status, 0, (size_t)tiles2 * sizeof(Pair64), s));
-    LAUNCH("line_scan", s, line_scan_kernel<256, 8><<<(unsigned)tiles2, 256, 0, s>>>(seq_len, kind, info, seq_before, hdr_before, status, tickets + 1));
-    CU(cudaMemcpyAsync(&h, info, sizeof h, cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    if (h.bad) return fail(KMG_ERR_ARG, "malformed FASTQ: only the four-line form (@name / sequence / + / qualities of the same length) is read");
-    r->n_records = h.n_records; r->total_bases = h.total_bases;
-    const uint64_t packed = h.total_bases + h.n_records;
-    TRY(dalloc(&r->seq, (size_t)packed + 16, s));
-    TRY(dalloc(&r->d_rec_off, (size_t)h.n_records + 1, s));
-    TRY(dalloc(&name_pos, (size_t)h.n_records + 1, s));
-    TRY(dalloc(&name_len, (size_t)h.n_records + 1, s));
-    LAUNCH("records", s, record_kernel<<<lgrid, 256, 0, s>>>(d_text, n, nl, info, kind, seq_before, hdr_before, r->d_rec_off, name_pos, name_len));
-    const unsigned pgrid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(nblocks, 256), (uint64_t)g_ctx.sms * 16);
-    LAUNCH("pack_reads", s, pack_kernel<<<pgrid, 256, 0, s>>>(d_text, n, nl, blk_nl, info, kind, seq_before, hdr_before, r->seq, info));
-    if (h.n_records)
-      LAUNCH("record_finish", s, record_finish_kernel<<<(unsigned)std::min<uint64_t>(ceil_div<uint64_t>(h.n_records, 256), (uint64_t)g_ctx.sms * 16), 256, 0, s>>>(info, r->d_rec_off, r->seq));
-    r->rec_off.resize((size_t)h.n_records + 1);
-    h_name_pos.resize((size_t)h.n_records + 1);
-    h_name_len.resize((size_t)h.n_records + 1);
-    CU(cudaMemcpyAsync(r->rec_off.data(), r->d_rec_off, (h.n_records + 1) * 8, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(h_name_pos.data(), name_pos, (h.n_records + 1) * 8, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(h_name_len.data(), name_len, (h.n_records + 1) * 4, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(&h, info, sizeof h, cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    if (h.bad) return fail(KMG_ERR_ARG, "sequence data before the first header line");
-    // names: short strings, fetched from the text where it lives
-    r->names.resize((size_t)h.n_records);
-    const bool text_on_host = ptr_kind(text) != PK_DEVICE;
-    std::vector<char> tmp;
-    for (uint64_t i = 0; i < h.n_records; ++i) {
-      if (text_on_host) r->names[i].assign((const char *)text + h_name_pos[i], h_name_len[i]);
-      else {
-        tmp.resize(h_name_len[i]);
-        if (h_name_len[i]) CU(cudaMemcpy(tmp.data(), d_text + h_name_pos[i], h_name_len[i], cudaMemcpyDeviceToHost));
-        r->names[i].assign(tmp.data(), h_name_len[i]);
-      }
+  r->rec_off.resize((size_t)h.n_records + 1);
+  h_name_len.resize((size_t)h.n_records + 1);
+  CU(cudaMemcpyAsync(r->rec_off.data(), r->d_rec_off, (h.n_records + 1) * 8, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(h_name_pos.get(), name_pos, (h.n_records + 1) * 8, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(h_name_len.data(), name_len, (h.n_records + 1) * 4, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(&h, info, sizeof h, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  if (h.bad) return fail(KMG_ERR_ARG, "sequence data before the first header line");
+  // names: short strings, fetched from the text where it lives
+  r->names.resize((size_t)h.n_records);
+  const bool text_on_host = ptr_kind(text) != PK_DEVICE;
+  std::vector<char> tmp;
+  for (uint64_t i = 0; i < h.n_records; ++i) {
+    if (text_on_host) r->names[i].assign((const char *)text + h_name_pos[i], h_name_len[i]);
+    else {
+      tmp.resize(h_name_len[i]);
+      if (h_name_len[i]) CU(cudaMemcpy(tmp.data(), d_text + h_name_pos[i], h_name_len[i], cudaMemcpyDeviceToHost));
+      r->names[i].assign(tmp.data(), h_name_len[i]);
     }
-    prof_bytes("nl_scan", (double)n); prof_bytes("pack_reads", (double)n + (double)packed);
-    return KMG_OK;
-  };
-  const int rc = body();
-  dfree(d_text, s); dfree(kind, s); dfree(nl, s); dfree(seq_len, s); dfree(seq_before, s); dfree(hdr_before, s);
-  dfree(name_pos, s); dfree(blk_nl, s); dfree(tickets, s); dfree(name_len, s); dfree(status, s); dfree(info, s);
-  if (rc != KMG_OK) { cudaStreamSynchronize(s); kmg_reads_free(r); return rc; }
-  *out = r;
+  }
+  prof_bytes("nl_scan", (double)n); prof_bytes("pack_reads", (double)n + (double)packed);
+  *out = r.release();
   return KMG_OK;
 }
 
@@ -3414,12 +3232,7 @@ extern "C" int kmg_reads_open(const char *path, kmg_reads **out) {
   return kmg_reads_from_memory(text.data(), (int64_t)used, out);
 }
 
-static int use_reads(const kmg_reads *r) {
-  if (!r) return fail(KMG_ERR_ARG, "reads is NULL");
-  TRY(ctx_init());
-  if (r->device != g_ctx.device) return fail(KMG_ERR_ARG, "the reads live on device %d but this thread works on device %d", r->device, g_ctx.device);
-  return KMG_OK;
-}
+static int use_reads(const kmg_reads *r) { return r ? use_device(r->device, "the reads live") : fail(KMG_ERR_ARG, "reads is NULL"); }
 extern "C" int kmg_reads_count(const kmg_reads *r, uint64_t *n_records, uint64_t *total_bases) {
   if (!r) return fail(KMG_ERR_ARG, "reads is NULL");
   if (n_records) *n_records = r->n_records;
@@ -3459,23 +3272,17 @@ extern "C" int kmg_count_add_reads(kmg_counter *c, const kmg_reads *r, int sourc
   if (r->n_records == 0) return KMG_OK;
   cudaStream_t s = g_ctx.stream();
   const uint64_t packed = r->total_bases + r->n_records;
-  uint8_t *tmp = nullptr;
-  ReadsInfo *info = nullptr;
-  TRY(dalloc(&tmp, (size_t)packed + 16, s));
-  int rc = dalloc(&info, 1, s);
-  if (rc == KMG_OK) {
-    ReadsInfo h{};
-    h.n_records = r->n_records; h.total_bases = r->total_bases;
-    if (cudaMemcpyAsync(info, &h, sizeof h, cudaMemcpyHostToDevice, s) != cudaSuccess ||
-        cudaMemcpyAsync(tmp, r->seq, (size_t)packed, cudaMemcpyDeviceToDevice, s) != cudaSuccess) rc = fail(KMG_ERR_CUDA, "copy failed");
-    if (rc == KMG_OK) {
-      const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(r->n_records, 256), (uint64_t)g_ctx.sms * 16);
-      mask_for_counting_kernel<<<grid, 256, 0, s>>>(info, r->d_rec_off, c->k, tmp);
-      if (cudaStreamSynchronize(s) != cudaSuccess) rc = fail(KMG_ERR_CUDA, "masking failed: %s", cudaGetErrorString(cudaGetLastError()));
-    }
-    // the last record's separator is the final byte: drop it so that the end-of-string rule sees the record's own end... it is an 'N' either way
-    if (rc == KMG_OK) rc = kmg_count_add(c, (const char *)tmp, (int64_t)packed, source);
-  }
-  dfree(tmp, s); dfree(info, s);
-  return rc;
+  DevBuf<uint8_t> tmp(s);
+  DevBuf<ReadsInfo> info(s);
+  TRY(tmp.alloc((size_t)packed + 16));
+  TRY(info.alloc(1));
+  ReadsInfo h{};
+  h.n_records = r->n_records; h.total_bases = r->total_bases;
+  if (cudaMemcpyAsync(info, &h, sizeof h, cudaMemcpyHostToDevice, s) != cudaSuccess ||
+      cudaMemcpyAsync(tmp, r->seq, (size_t)packed, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return fail(KMG_ERR_CUDA, "copy failed");
+  const unsigned grid = (unsigned)std::min<uint64_t>(ceil_div<uint64_t>(r->n_records, 256), (uint64_t)g_ctx.sms * 16);
+  mask_for_counting_kernel<<<grid, 256, 0, s>>>(info, r->d_rec_off, c->k, tmp);
+  if (cudaStreamSynchronize(s) != cudaSuccess) return fail(KMG_ERR_CUDA, "masking failed: %s", cudaGetErrorString(cudaGetLastError()));
+  // the last record's separator is the final byte: drop it so that the end-of-string rule sees the record's own end... it is an 'N' either way
+  return kmg_count_add(c, (const char *)tmp.get(), (int64_t)packed, source);
 }
